@@ -4,6 +4,7 @@ updates/s, HBM GB/s against the roofline, at 1/2/4/8 B200).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--config config3] [--cutoff-km 2000]
     python bench.py --impl reference ...         # the reference's CPU path (numpy oracle) on host cores
+    python bench.py ... --dump-outputs DIR       # also write the last timed step's outputs to DIR/*.npy
 
 One step = one complete analysis (all observations of the workload, in serial order) of a synthetic
 ensemble.  Three measurements share one JSON line:
@@ -54,7 +55,14 @@ def parse():
     ap.add_argument('--no-check', action='store_true', help='skip the sharded-vs-unsharded comparison (N > 1)')
     ap.add_argument('--cpu-seconds', type=float, default=20.0, help='target CPU time of the baseline sample')
     ap.add_argument('--seed', type=int, default=0)
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='after the timed steps, write what the last one computed to DIR/<name>.npy (see dump_outputs); '
+                         'GPU path only: --impl reference times a partial CPU sample of the analysis, so it has no '
+                         'complete output to write')
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != 'ours':
+        ap.error('--dump-outputs writes the outputs of the GPU path (--impl ours)')
+    return args
 
 
 def measured_traffic(args, cfg, world, kernel):
@@ -146,6 +154,40 @@ def obs_arrays(case):
                             halfwidth=case.ob_halfwidth, assimilate=case.ob_assimilate.astype(np.uint8),
                             row0=(case.ob_var * nt + tlo) * (ny * nx), row1=(case.ob_var * nt + thi) * (ny * nx),
                             tw0=wlo, tw1=whi)
+
+
+DUMP_BYTES = 64 * 10 ** 6
+
+
+def _fixed_sample(n, cap):
+    """All of range(n), or `cap` indices of it drawn with a fixed seed, in increasing order: the same ones in every
+    run with the same n."""
+    if n <= cap:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(0).choice(n, cap, replace=False))
+
+
+def dump_outputs(path, X, res):
+    """--dump-outputs: what engine.analysis_device, the timed path, gave back in the last timed step, as
+    path/<name>.npy, at most DUMP_BYTES in all.  Inputs depend only on the command line (seeded synthetic case), so
+    two builds run with the same arguments can be compared file by file.
+      prior_mean, prior_var, post_mean, post_var   per-ob diagnostics, float64 (NaN where an ob was not assimilated)
+      assimilated                                  1.0 / 0.0 per ob
+      analysis                                     the analysis ensemble [rows, nens] in the storage type of the run
+    The diagnostics are kept to a quarter of the budget and the analysis to the rest: past that, a fixed sample of
+    obs / state rows (_fixed_sample) is written instead of all of them.  Not available with --impl reference, whose
+    timed steps run the CPU loop over a sample of the obs and never produce a complete analysis."""
+    os.makedirs(path, exist_ok=True)
+    diag = {'prior_mean': res.prior_mean, 'prior_var': res.prior_var, 'post_mean': res.post_mean,
+            'post_var': res.post_var, 'assimilated': res.assimilated.astype(np.float64)}
+    obs_idx = _fixed_sample(len(res.prior_mean), DUMP_BYTES // 4 // (8 * len(diag)))
+    for name, a in diag.items():
+        np.save(os.path.join(path, name + '.npy'), np.asarray(a, dtype=np.float64)[obs_idx])
+    nrows, nens = X.shape
+    room = DUMP_BYTES - 8 * len(diag) * obs_idx.size - 4096          # 4096: the .npy headers
+    rows = _fixed_sample(nrows, room // (nens * X.element_size()))
+    import torch
+    np.save(os.path.join(path, 'analysis.npy'), X[torch.as_tensor(rows, device=X.device)].cpu().numpy())
 
 
 def workload_name(args, cfg):
@@ -362,6 +404,16 @@ def run_ours(args):
         su_max = su_ms
     ms_step = float(ms_total.item()) / args.steps
     state_pairs = float(pairs.item())                      # sum_k |F_s(k)| over the whole grid
+
+    if args.dump_outputs:
+        # X holds the analysis of the last timed step; at N > 1 its bands are assembled on rank 0 first
+        full = X
+        if world > 1:
+            full = torch.empty((nrows, nens), dtype=tdtype, device=dev) if rank == 0 else None
+            sharding.gather_bands(X, full, bands, nlev, ny, nx, nens, rank)
+        if rank == 0:
+            dump_outputs(args.dump_outputs, full, res)
+        del full
 
     # ---- e2e: host buffers, copies inside the timed region ------------------------------------
     e2e = None

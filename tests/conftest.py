@@ -33,11 +33,15 @@ def decode_inflation(infl):
 
 
 def load_golden(name):
+    """(arrays, parameters) of a golden case.  The file holds the reference's posterior as post - prior (it compresses
+    better), with the prior regenerated from the case's seed; make_golden.py checked when writing it that adding the
+    prior back rebuilds 'post' bit for bit."""
     import json
     import numpy as np
-    g = np.load(os.path.join(GOLDEN, name + '.npz'))
+    g = dict(np.load(os.path.join(GOLDEN, name + '.npz')))
     p = json.loads(str(g['params']))
     p['inflation'] = decode_inflation(p['inflation'])
+    g['post'] = golden_case(p).to_vect() + g.pop('post_minus_prior')
     return g, p
 
 

@@ -101,6 +101,10 @@ def run_case(name, kw, loc, inflation):
     with contextlib.redirect_stdout(io.StringIO()):     # "Unable to find variable ... Skipping"
         post_state, post_obs = EnSRF(state, obs, inflation=decode_inflation(inflation), verbose=False, loc=loc).update()
     post_vect = post_state.to_vect()
+    # stored as post - prior, which keeps the files small (tests/conftest.py:load_golden adds back the prior
+    # regenerated from the seed); the round trip must be exact
+    post_minus_prior = post_vect - prior_vect
+    assert np.array_equal(prior_vect + post_minus_prior, post_vect), name
     f = lambda attr: np.array([np.nan if getattr(o, attr) is None else float(getattr(o, attr))
                                for o in post_obs])
     out = dict(
@@ -109,7 +113,7 @@ def run_case(name, kw, loc, inflation):
         # the caller's state after the call (inflated in place by the float / per-variable forms only)
         prior_after_checksum=np.array([state.to_vect().sum(), np.abs(state.to_vect()).sum()]),
         ye=ye, nearest=near, loc_state0=loc_state0, loc_obs0=loc_obs0,
-        post=post_vect,
+        post_minus_prior=post_minus_prior,
         prior_mean=f('prior_mean'), prior_var=f('prior_var'),
         post_mean=f('post_mean'), post_var=f('post_var'),
         assimilated=np.array([bool(o.assimilated) for o in post_obs]),
