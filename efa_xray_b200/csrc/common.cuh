@@ -223,7 +223,7 @@ __device__ __forceinline__ double loc_weight_fast(double a, double inv_hw, doubl
     return inside ? w : 0.0;
 }
 
-// candidate lists per coarse tile of the state sweeps (state_sweep_pipe.cu)
+// candidate lists per coarse tile of the state sweep (state_sweep_2p.cu)
 #define SP_CT 4                       // coarse tile = SP_CT x SP_CT patches
 struct SweepLists {
     float4 *caps = nullptr;
@@ -237,7 +237,7 @@ struct SweepLists {
 // records of the obs and the candidate lists per coarse tile for the patch shape of the two-phase kernel.
 struct ExbSweepPlan {
     int64_t nlev = 0, ny = 0, nx = 0, nobs = 0, ob_begin = 0, ob_end = 0, y_begin = 0, y_end = 0;
-    int loc_mode = 0, bty = 0, btx = 0;
+    int loc_mode = 0;
     const double *grid_u = nullptr;       // identity of the inputs the plan was built from
     const double *obgeo = nullptr;
     float4 *scan = nullptr;
@@ -247,10 +247,6 @@ struct ExbSweepPlan {
     cudaEvent_t ready = nullptr, used = nullptr;
     bool was_used = false;
 };
-bool sweep_lists_wanted(int loc_mode, int64_t ob_begin, int64_t ob_end);
-int sweep_build_lists(const double *grid_u, int64_t npts, int nx, int y_begin, int y_end, int bty, int btx, const float4 *scan,
-                      int64_t ob_begin, int64_t ob_end, cudaStream_t st, SweepLists *out);
-void sweep_free_lists(SweepLists &l, cudaStream_t st);
 
 template <typename T> struct Vec2;
 template <> struct Vec2<double> { typedef double2 type; };

@@ -1,11 +1,11 @@
 // State sweep, two-phase FP64 tensor-core version (production path for ensembles of up to 103 members).
 //
-// Same mathematics as state_sweep_pipe.cu / state_update_mma.cu (read the header of the latter first: blocked 8-ob
-// form of ensrf.py:95-141 on mma.sync.m8n8k4.f64, the ensemble mean carried as a pseudo-member column).  What changes
-// is who does the scalar FP64 work.  In state_sweep_pipe.cu four producer warps evaluate the Gaspari-Cohn weights
-// (observation.py:117-130, ~60 scalar FP64 instructions per (grid point, ob) pair) WHILE twelve consumer warps issue
-// DMMAs; scalar FP64 and DMMA share one issue port per SM sub-partition, so the producers had to be given a
-// sub-partition of their own, whose tensor pipe then sat idle (ceiling 75 % of the FP64 tensor peak, measured 58 %).
+// Same mathematics as state_update_mma.cu (read its header first: blocked 8-ob form of ensrf.py:95-141 on
+// mma.sync.m8n8k4.f64, the ensemble mean carried as a pseudo-member column).  What changes is who does the scalar FP64
+// work.  The Gaspari-Cohn weights (observation.py:117-130, ~60 scalar FP64 instructions per (grid point, ob) pair) and
+// the DMMAs share one issue port per SM sub-partition.  Producer warps that evaluate the weights WHILE consumer warps
+// issue DMMAs must be given a sub-partition of their own, whose tensor pipe then sits idle: round 1's kernel did this
+// with four producers and twelve consumers (ceiling 75 % of the FP64 tensor peak, measured 58 %; removed since).
 // Here the two kinds of work never run at the same time:
 //   phase A  all 16 warps of the CTA: scan the patch's candidate obs (fp32 cap test over the coarse tile's list),
 //            evaluate omega[ob][grid point] = beta c1 GC(d) for batches of 8 obs and the batch's 8x8 Gram matrix, and
@@ -34,14 +34,12 @@
 #include <cstdlib>
 #include <cstring>
 
-// Warps per CTA (template parameter NW of the kernel, 128 registers per thread either way):
-//   16  one CTA per SM, four warps per sub-partition, 128 state rows per patch (a 17th warp would put five warps on one
-//       sub-partition's 16 K registers: 96 per thread);
-//    8  two CTAs per SM, 64 rows per patch each: while one CTA is in phase A (scalar FP64) the other can be in phase B
-//       (DMMA).  Measured slower (config 3: 146.9 against 137.4 ms, profiles/r02_sweep.md): the two kinds of work
-//       share the FP64 issue port, so overlapping them gains nothing, and the per-patch work (weights, Gram matrices,
-//       scan) is spread over half as many rows.  EXB_S2_WARPS=8 selects it (kept as a tested variant).
+// Warps per CTA: one CTA per SM, four warps per sub-partition, 128 registers per thread, 128 state rows per patch (a
+// 17th warp would put five warps on one sub-partition's 16 K registers: 96 per thread).  Two CTAs of 8 warps per SM,
+// so that one CTA's phase A overlaps the other's phase B, measured slower (DESIGN.md 4.3): the two kinds of work share
+// the FP64 issue port, and the per-patch work is spread over half as many rows.
 // Every warp is a consumer in phase B and takes turns issuing the copies.
+#define S2_NW 16
 #define S2_CAND 2048                   // candidate capacity of a chunk (256 batches)
 #define S2_MAXSTAGES 16
 
@@ -61,8 +59,6 @@ struct S2Params {
     double *scratch;                  // per CTA: S2_CAND/8 blocks of blk_doubles, then the parked rows
     const int *abort_flag;            // watchdog word of the obs-space solve that produced the records (may be null)
     unsigned long long *prof;         // EXB_S2_PROF=1: clocks of warp 0 per phase, summed over CTAs (null: off)
-    int dbg;                          // EXB_S2_DEBUG bit mask, timing experiments only (2 and 4: results are wrong): 1 ye rows of the Gram matrix staged with cp.async,
-                                      // 2 no weights, 4 no Gram
     int64_t npts, nobs, ob_begin, ob_end, scratch_stride;
     int nlev, ny, nx, nens;
     int y_begin, y_end;               // grid rows [y_begin, y_end) of the shard are swept by this launch
@@ -140,8 +136,9 @@ template <int NT3> __host__ __device__ constexpr int s2_yst() { return ((8 * NT3
 template <int NT3> __host__ __device__ constexpr int s2_ydoubles() { return 8 * s2_yst<NT3>() + 16; }
 
 // Stage layout (doubles): y rows [s2_ydoubles] | block = om[8][G] (ob-major) | Gram[64]
-template <int NT3, typename TS, int NW>
-__global__ void __launch_bounds__(NW * 32, 16 / NW) state_sweep_2p_kernel(const S2Params p) {
+template <int NT3, typename TS>
+__global__ void __launch_bounds__(S2_NW * 32, 1) state_sweep_2p_kernel(const S2Params p) {
+    constexpr int NW = S2_NW;
     constexpr int NTH = NW * 32;             // threads per CTA
     constexpr int ROWS = NW * 8;             // state rows per CTA
     constexpr int SCAN = 2 * NTH;            // list entries per scan step (2 per thread)
@@ -341,12 +338,6 @@ __global__ void __launch_bounds__(NW * 32, 16 / NW) state_sweep_2p_kernel(const 
             // Block of batch b (doubles): om[8][G] (ob-major: omega of ob q at grid point g) | Gram[64].
             {
                 double *sob = s_sob + warp * 48;
-                // the ring is idle in this phase: every warp stages the 8 ye rows of its current batch in it (cp.async)
-                // while it evaluates the weights, and forms the Gram matrix from there afterwards
-                double *stg = s_ring + (size_t)warp * (8 * YW);
-                // (measured: staging costs 1.7 % of the kernel more than loading the operands straight from L2 after the
-                // weights, EXB_S2_DEBUG=1 switches it on)
-                const bool stage_rows = (size_t)NW * 8 * YW <= (size_t)S * SD && (p.dbg & 1);
                 // scalars of the obs of a batch, held by lanes 0..7; loaded one batch ahead
                 struct ObSc { double ux, uy, uz, ihw, amax, c1, beta; int kk; };      // (no arithmetic on the loaded values
                                                                                      // here: it would wait for them)
@@ -368,23 +359,12 @@ __global__ void __launch_bounds__(NW * 32, 16 / NW) state_sweep_2p_kernel(const 
                 for (int b = warp; b < nb; b += NW) {
                     const int nq = min(8, ncand - 8 * b);
                     load_sc(b + NW, nxt);
-                    __syncwarp();                                    // the previous batch's readers of sob / stg are done
+                    __syncwarp();                                    // the previous batch's readers of sob are done
                     if (lane < 8) {          // per ob: ux uy uz 1/halfwidth a_max beta*c1
                         *reinterpret_cast<double2 *>(sob + 6 * lane) = make_double2(cur.ux, cur.uy);
                         *reinterpret_cast<double2 *>(sob + 6 * lane + 2) = make_double2(cur.uz, cur.ihw);
                         // beta / ((N-1) kdenom)   (ensrf.py:95, :119, :135-136); the localisation weight multiplies it
                         *reinterpret_cast<double2 *>(sob + 6 * lane + 4) = make_double2(cur.amax, cur.c1 * cur.beta);
-                    }
-                    if (stage_rows) {
-                        // 8 rows x YW doubles = 8 * YW / 2 chunks of 16 bytes, dealt to the lanes
-#pragma unroll 1
-                        for (int q = 0; q < 8; ++q) {
-                            const int kq = __shfl_sync(0xffffffffu, cur.kk, q);
-                            const double *src = p.Yw + (size_t)(kq >= 0 ? kq : p.nobs) * YW;
-                            for (int m = 2 * lane; m < YW; m += 64)
-                                asm volatile("cp.async.cg.shared.global [%0], [%1], 16;\n" ::"r"(s2_smem(stg + q * YW + m)), "l"(src + m));
-                        }
-                        asm volatile("cp.async.commit_group;\n" ::);
                     }
                     __syncwarp();
                     S2_TICK(6);
@@ -414,7 +394,7 @@ __global__ void __launch_bounds__(NW * 32, 16 / NW) state_sweep_2p_kernel(const 
                         npb += (w != 0.0) ? 1 : 0;
                         return w * o45.y;
                     };
-                    const int nfull = (p.dbg & 2) ? 0 : (G >> 5), R = (p.dbg & 2) ? 0 : (G & 31);
+                    const int nfull = G >> 5, R = G & 31;
                     for (int sl = 0; sl < nfull; ++sl) {
                         const int gg = lane + 32 * sl;
                         const double gx = s_gu[gg], gy = s_gu[ROWS + gg], gz = s_gu[2 * ROWS + gg];
@@ -438,31 +418,17 @@ __global__ void __launch_bounds__(NW * 32, 16 / NW) state_sweep_2p_kernel(const 
                     if (lc == 0) npairs += (unsigned long long)npb;
                     S2_TICK(7);
                     // Gram matrix of the batch (members only: the pseudo-member column is masked): row n of the batch,
-                    // this lane's two members of every 8-member tile
+                    // this lane's two members of every 8-member tile, operands straight from Yw (L2)
                     {
                         double g0 = 0.0, g1 = 0.0, h0 = 0.0, h1 = 0.0;
-                        if (p.dbg & 4) {
-                        } else if (stage_rows) {
-                            asm volatile("cp.async.wait_group 0;\n" ::: "memory");
-                            __syncwarp();
-                            const double *yrow = stg + n * YW + 2 * c;
+                        const int krow = __shfl_sync(0xffffffffu, cur.kk, n);
+                        const double *yrow = p.Yw + (size_t)(krow >= 0 ? krow : p.nobs) * YW + 2 * c;
 #pragma unroll
-                            for (int t = 0; t < NT3; ++t) {
-                                const double2 v = *reinterpret_cast<const double2 *>(yrow + 8 * t);
-                                const double v1 = (t == NT3 - 1 && c == 3) ? 0.0 : v.y;
-                                s2_dmma(g0, g1, v.x, v.x);
-                                s2_dmma(h0, h1, v1, v1);
-                            }
-                        } else {
-                            const int krow = __shfl_sync(0xffffffffu, cur.kk, n);
-                            const double *yrow = p.Yw + (size_t)(krow >= 0 ? krow : p.nobs) * YW + 2 * c;
-#pragma unroll
-                            for (int t = 0; t < NT3; ++t) {
-                                const double2 v = __ldg(reinterpret_cast<const double2 *>(yrow + 8 * t));
-                                const double v1 = (t == NT3 - 1 && c == 3) ? 0.0 : v.y;
-                                s2_dmma(g0, g1, v.x, v.x);
-                                s2_dmma(h0, h1, v1, v1);
-                            }
+                        for (int t = 0; t < NT3; ++t) {
+                            const double2 v = __ldg(reinterpret_cast<const double2 *>(yrow + 8 * t));
+                            const double v1 = (t == NT3 - 1 && c == 3) ? 0.0 : v.y;
+                            s2_dmma(g0, g1, v.x, v.x);
+                            s2_dmma(h0, h1, v1, v1);
                         }
                         *reinterpret_cast<double2 *>(gblk + 8 * G + n * 8 + 2 * c) = make_double2(g0 + h0, g1 + h1);
                     }
@@ -472,7 +438,7 @@ __global__ void __launch_bounds__(NW * 32, 16 / NW) state_sweep_2p_kernel(const 
                 S2_TICK(9);
             }
             // the blocks were written through the generic proxy and are read by bulk copies (async proxy)
-            // (and the ring, used as a generic-proxy staging area above, is written by them again)
+            // (and the ring, read through the generic proxy in the previous phase B, is written by them again)
             __threadfence();
             asm volatile("fence.proxy.async.global;\n" ::: "memory");
             asm volatile("fence.proxy.async.shared::cta;\n" ::: "memory");
@@ -691,16 +657,191 @@ __global__ void sweep_rows_kernel(const TS *__restrict__ Yp, const double *__res
 }
 
 // ------------------------------------------------------------------------------------------
-// host side
+// candidate lists per coarse tile
 // ------------------------------------------------------------------------------------------
-// (read per call: a sweep plan made for the other patch shape is ignored by s2_launch, which then builds its own lists)
-static int s2_warps() {
-    const char *e = getenv("EXB_S2_WARPS");
-    return (e && atoi(e) == 8) ? 8 : 16;
+// bounding cap (centre, angular radius) of every coarse tile: one warp per tile
+__global__ void sweep_tile_caps_kernel(const double *__restrict__ grid_u, int64_t npts, int nx, int y_begin, int y_end, int pr0,
+                                       int cty, int ctx, int nctx, int ntiles, float4 *__restrict__ caps) {
+    const int t = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
+    if (t >= ntiles) return;
+    const int ya = max((pr0 / SP_CT + t / nctx) * cty, y_begin), yb = min((pr0 / SP_CT + t / nctx + 1) * cty, y_end);
+    const int xa = (t % nctx) * ctx, xb = min(xa + ctx, nx);
+    const int w = xb - xa, npt = max(yb - ya, 0) * w;
+    double cx = 0, cy = 0, cz = 0;
+    for (int i = lane; i < npt; i += 32) {
+        const int64_t pt = (int64_t)(ya + i / w) * nx + xa + i % w;
+        cx += grid_u[pt]; cy += grid_u[npts + pt]; cz += grid_u[2 * npts + pt];
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        cx += __shfl_xor_sync(0xffffffffu, cx, o); cy += __shfl_xor_sync(0xffffffffu, cy, o); cz += __shfl_xor_sync(0xffffffffu, cz, o);
+    }
+    const double nn = sqrt(cx * cx + cy * cy + cz * cz);
+    if (nn > 1e-9) { cx /= nn; cy /= nn; cz /= nn; }
+    double cmin = 1.0;
+    for (int i = lane; i < npt; i += 32) {
+        const int64_t pt = (int64_t)(ya + i / w) * nx + xa + i % w;
+        cmin = fmin(cmin, cx * grid_u[pt] + cy * grid_u[npts + pt] + cz * grid_u[2 * npts + pt]);
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) cmin = fmin(cmin, __shfl_xor_sync(0xffffffffu, cmin, o));
+    if (lane == 0) {
+        // degenerate centre (tile wraps the globe): radius pi -> everything is a candidate
+        const double rho = (nn > 1e-9 && npt > 0) ? acos(fmax(-1.0, fmin(1.0, cmin))) + 1e-4 : 3.2;
+        caps[t] = make_float4((float)cx, (float)cy, (float)cz, (float)rho);
+    }
 }
 
-void s2_patch_shape(int64_t nlev, int64_t ny, int64_t nx, int *Lc_out, int *bty_out, int *btx_out) {
-    const int rows = 8 * s2_warps();
+// FILL = false: cnt[t] = number of obs whose support can touch tile t; FILL = true: their ascending list
+template <bool FILL>
+__global__ void sweep_tile_list_kernel(const float4 *__restrict__ caps, int ntiles, const float4 *__restrict__ scan,
+                                       int64_t ob_begin, int64_t ob_end, int *__restrict__ cnt,
+                                       const int64_t *__restrict__ off, int *__restrict__ list) {
+    const int t = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
+    if (t >= ntiles) return;
+    const float4 cap = caps[t];
+    int64_t pos = FILL ? off[t] : 0;
+    int count = 0;
+    const unsigned lt = (1u << lane) - 1u;
+    // One warp walks all obs for its tile: the loop is bound by the latency of the scan-record loads, so the records of
+    // TL_UNROLL groups of 32 obs are fetched before the first of them is tested (the groups are still taken in order).
+    constexpr int TL_UNROLL = 8;
+    for (int64_t base = ob_begin; base < ob_end; base += 32 * TL_UNROLL) {
+        float4 sc[TL_UNROLL];
+#pragma unroll
+        for (int u = 0; u < TL_UNROLL; ++u) {
+            const int64_t k = base + 32 * u + lane;
+            sc[u] = (k < ob_end) ? __ldg(scan + k) : make_float4(0.f, 0.f, 0.f, -1.f);
+        }
+#pragma unroll
+        for (int u = 0; u < TL_UNROLL; ++u) {
+            const int64_t k = base + 32 * u + lane;
+            bool hit = false;
+            if (sc[u].w >= 0.f) {                  // (past the end of the range: w = -1)
+                const float ang = sc[u].w + cap.w;
+                hit = (ang >= 3.1405f) || (sc[u].x * cap.x + sc[u].y * cap.y + sc[u].z * cap.z >= __cosf(ang) - 4e-6f);
+            }
+            if (FILL) {
+                const unsigned b = __ballot_sync(0xffffffffu, hit);
+                if (hit) list[pos + __popc(b & lt)] = (int)k;
+                pos += __popc(b);
+            } else {
+                count += hit ? 1 : 0;
+            }
+        }
+    }
+    if (!FILL) {
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) count += __shfl_xor_sync(0xffffffffu, count, o);
+        if (lane == 0) cnt[t] = count;
+    }
+}
+
+// grid row of [y_begin, y_end) closest to the equator (|sin lat| of its first column smallest) -> mapped host word
+__global__ void sweep_eq_row_kernel(const double *__restrict__ uz, int nx, int y_begin, int y_end, long long *__restrict__ out) {
+    __shared__ double bv[256];
+    __shared__ int bi[256];
+    double best = 2.0;
+    int besty = y_begin;
+    for (int y = y_begin + threadIdx.x; y < y_end; y += 256) {
+        const double v = fabs(uz[(int64_t)y * nx]);
+        if (v < best) { best = v; besty = y; }
+    }
+    bv[threadIdx.x] = best; bi[threadIdx.x] = besty;
+    __syncthreads();
+    for (int o = 128; o > 0; o >>= 1) {
+        if (threadIdx.x < o && bv[threadIdx.x + o] < bv[threadIdx.x]) { bv[threadIdx.x] = bv[threadIdx.x + o]; bi[threadIdx.x] = bi[threadIdx.x + o]; }
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) *out = bi[0];
+}
+
+// exclusive prefix sum of cnt[n] into off[n+1], n small (one CTA, serial over chunks of 1024)
+__global__ void __launch_bounds__(1024) sweep_scan_kernel(const int *__restrict__ cnt, int n, int64_t *__restrict__ off,
+                                                         long long *__restrict__ total_host) {
+    __shared__ long long part[1024];
+    __shared__ long long carry_s;
+    const int t = threadIdx.x;
+    if (t == 0) carry_s = 0;
+    __syncthreads();
+    for (int b = 0; b < n; b += 1024) {
+        const int i = b + t;
+        const long long v = i < n ? cnt[i] : 0;
+        part[t] = v;
+        __syncthreads();
+        for (int d = 1; d < 1024; d <<= 1) {
+            const long long y = t >= d ? part[t - d] : 0;
+            __syncthreads();
+            part[t] += y;
+            __syncthreads();
+        }
+        const long long carry = carry_s;
+        if (i < n) off[i] = carry + part[t] - v;
+        __syncthreads();
+        if (t == 1023) carry_s = carry + part[1023];
+        __syncthreads();
+    }
+    if (t == 0) {
+        off[n] = carry_s;
+        *total_host = carry_s;        // mapped pinned host word: no D2H copy queued behind band downloads
+    }
+}
+
+// ------------------------------------------------------------------------------------------
+// host side: candidate lists per coarse tile
+// ------------------------------------------------------------------------------------------
+static bool sweep_lists_wanted(int loc_mode, int64_t ob_begin, int64_t ob_end) {
+    const char *nolist = getenv("EXB_SWEEP_NOLIST");
+    return loc_mode == EXB_LOC_GC && !(nolist && atoi(nolist)) && ob_end - ob_begin > 4096;
+}
+
+// Builds, for every coarse tile (SP_CT x SP_CT patches of bty x btx grid points) that intersects grid rows
+// [y_begin, y_end), the ascending list of obs in [ob_begin, ob_end) whose support can touch the tile.  Synchronises the
+// stream once (list sizes).  out->tile_off is indexed by ABSOLUTE coarse-tile number (coarse row * nctx + coarse col).
+static int sweep_build_lists(const double *grid_u, int64_t npts, int nx, int y_begin, int y_end, int bty, int btx,
+                             const float4 *scan, int64_t ob_begin, int64_t ob_end, cudaStream_t st, SweepLists *out) {
+    const int pr0 = y_begin / bty, pr1 = (y_end + bty - 1) / bty;
+    const int cty = bty * SP_CT, ctx = btx * SP_CT;
+    out->nctx = (nx + ctx - 1) / ctx;
+    const int cr0 = pr0 / SP_CT, cr1 = (pr1 + SP_CT - 1) / SP_CT;
+    const int ntiles = (cr1 - cr0) * out->nctx;
+    EXB_CUDA(exb_malloc_async(&out->caps, sizeof(float4) * ntiles, st));
+    EXB_CUDA(exb_malloc_async(&out->cnt, sizeof(int) * ntiles, st));
+    EXB_CUDA(exb_malloc_async(&out->off, sizeof(int64_t) * (ntiles + 1), st));
+    const unsigned gridw = (unsigned)ceil_div64((int64_t)ntiles * 32, 256);
+    sweep_tile_caps_kernel<<<gridw, 256, 0, st>>>(grid_u, npts, nx, y_begin, y_end, pr0, cty, ctx, out->nctx, ntiles, out->caps);
+    sweep_tile_list_kernel<false><<<gridw, 256, 0, st>>>(out->caps, ntiles, scan, ob_begin, ob_end, out->cnt, nullptr, nullptr);
+    ExbHostWords hw;                   // this call's own mapped words: [0] list total, [1] equator row
+    const int rcw = exb_host_words_acquire(&hw);
+    if (rcw != EXB_OK) return rcw;
+    struct WordsGuard { ExbHostWords w; ~WordsGuard() { exb_host_words_release(w); } } wguard{hw};
+    sweep_scan_kernel<<<1, 1024, 0, st>>>(out->cnt, ntiles, out->off, hw.dev);
+    sweep_eq_row_kernel<<<1, 256, 0, st>>>(grid_u + 2 * npts, nx, y_begin, y_end, hw.dev + 1);
+    exb_count_launches(4);
+    EXB_CUDA(cudaStreamSynchronize(st));
+    const long long total = hw.host[0];
+    out->eq_row = (int)hw.host[1];
+    EXB_CUDA(exb_malloc_async(&out->list, sizeof(int) * (size_t)(total > 0 ? total : 1), st));
+    sweep_tile_list_kernel<true><<<gridw, 256, 0, st>>>(out->caps, ntiles, scan, ob_begin, ob_end, nullptr, out->off, out->list);
+    exb_count_launches(1);
+    // the kernels index tiles by absolute coarse row: shift the offsets' base
+    out->tile_off = out->off - (int64_t)cr0 * out->nctx;
+    return exb_check_launch("sweep_tile_list_kernel");
+}
+
+static void sweep_free_lists(SweepLists &l, cudaStream_t st) {
+    if (l.caps) cudaFreeAsync(l.caps, st);
+    if (l.cnt) cudaFreeAsync(l.cnt, st);
+    if (l.off) cudaFreeAsync(l.off, st);
+    if (l.list) cudaFreeAsync(l.list, st);
+    l.caps = nullptr; l.cnt = nullptr; l.off = nullptr; l.list = nullptr;
+}
+
+// ------------------------------------------------------------------------------------------
+// host side
+// ------------------------------------------------------------------------------------------
+static void s2_patch_shape(int64_t nlev, int64_t ny, int64_t nx, int *Lc_out, int *bty_out, int *btx_out) {
+    const int rows = 8 * S2_NW;
     const int Lc = nlev < rows ? (int)nlev : rows;
     const int G = rows / Lc;
     int bty = 1, btx = G;
@@ -713,9 +854,9 @@ void s2_patch_shape(int64_t nlev, int64_t ny, int64_t nx, int *Lc_out, int *bty_
     *Lc_out = Lc; *bty_out = bty; *btx_out = btx;
 }
 
-template <int NT3, typename TS, int NW>
+template <int NT3, typename TS>
 static int s2_launch(S2Params &p, const TS *Yp, cudaStream_t st, const ExbSweepPlan *plan) {
-    constexpr int NTH = NW * 32, ROWS = NW * 8, PER_SM = 16 / NW;
+    constexpr int NTH = S2_NW * 32, ROWS = S2_NW * 8;
     int Lc, bty, btx;
     s2_patch_shape(p.nlev, p.ny, p.nx, &Lc, &bty, &btx);
     p.ty = bty; p.tx = btx; p.G = bty * btx; p.Lc = Lc;
@@ -731,16 +872,15 @@ static int s2_launch(S2Params &p, const TS *Yp, cudaStream_t st, const ExbSweepP
     EXB_CUDA(cudaGetDevice(&dev));
     EXB_CUDA(cudaDeviceGetAttribute(&max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
     EXB_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-    const size_t fixed = sizeof(double) * (3 * ROWS + NW * 48 + NW * 64) + sizeof(unsigned long long) * 2 * S2_MAXSTAGES +
-                         sizeof(int) * (S2_CAND + ROWS + NW + 4) + sizeof(float) * 4 + 128;
-    // shared memory of the SM = the largest opt-in block + 1 KB reserved per resident CTA
-    const size_t budget = PER_SM == 1 ? (size_t)max_smem - 1024 : ((size_t)max_smem + 1024) / PER_SM - 1024 - 256;
-    int S = (int)((budget - fixed) / (sizeof(double) * p.stage_doubles));
+    const size_t fixed = sizeof(double) * (3 * ROWS + S2_NW * 48 + S2_NW * 64) + sizeof(unsigned long long) * 2 * S2_MAXSTAGES +
+                         sizeof(int) * (S2_CAND + ROWS + S2_NW + 4) + sizeof(float) * 4 + 128;
+    // ring stages: whatever is left of the largest opt-in block, less 1 KB of headroom
+    int S = (int)(((size_t)max_smem - 1024 - fixed) / (sizeof(double) * p.stage_doubles));
     if (S > S2_MAXSTAGES) S = S2_MAXSTAGES;
     if (S < 4) return EXB_ERR_UNSUPPORTED;
     p.nstages = S;
     const size_t smem = fixed + sizeof(double) * (size_t)S * p.stage_doubles;
-    EXB_CUDA(cudaFuncSetAttribute(state_sweep_2p_kernel<NT3, TS, NW>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    EXB_CUDA(cudaFuncSetAttribute(state_sweep_2p_kernel<NT3, TS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
 
     const int64_t npatches = (int64_t)p.ntx * p.npr * p.nlc;
     if (npatches >= 0x7fffffff) {
@@ -749,15 +889,15 @@ static int s2_launch(S2Params &p, const TS *Yp, cudaStream_t st, const ExbSweepP
     }
     if (npatches <= 0) return EXB_OK;
     p.npatches = (int)npatches;
-    const int grid = npatches < (int64_t)sms * PER_SM ? (int)npatches : sms * PER_SM;
+    const int grid = npatches < (int64_t)sms ? (int)npatches : sms;
 
     // candidate lists per coarse tile (localised runs only; the kernel walks the ob range otherwise)
     SweepLists lists;
     p.tile_off = nullptr;
     p.tile_list = nullptr;
     p.nctx = 1;
-    if (plan && plan->have_lists && plan->bty == bty && plan->btx == btx && plan->y_begin <= p.y_begin && p.y_end <= plan->y_end &&
-        plan->ob_begin == p.ob_begin && plan->ob_end == p.ob_end) {
+    if (plan && plan->have_lists && plan->y_begin <= p.y_begin && p.y_end <= plan->y_end && plan->ob_begin == p.ob_begin &&
+        plan->ob_end == p.ob_end) {
         // lists built ahead (exb_sweep_plan_create): indexed by absolute coarse tile, so they serve any row sub-range
         p.nctx = plan->lists.nctx;
         p.pr_eq = plan->lists.eq_row / bty;
@@ -794,10 +934,9 @@ static int s2_launch(S2Params &p, const TS *Yp, cudaStream_t st, const ExbSweepP
             else prof = nullptr;
         }
         p.prof = prof;
-        p.dbg = getenv("EXB_S2_DEBUG") ? atoi(getenv("EXB_S2_DEBUG")) : 0;
-        p.cand_cap = S2_CAND / PER_SM;          // (same scratch area per SM)
+        p.cand_cap = S2_CAND;
         if (const char *e = getenv("EXB_S2_CAP")) { const int v = atoi(e); if (v >= 2 * NTH && v <= S2_CAND) p.cand_cap = v; }
-        state_sweep_2p_kernel<NT3, TS, NW><<<(unsigned)grid, NTH, smem, st>>>(p);
+        state_sweep_2p_kernel<NT3, TS><<<(unsigned)grid, NTH, smem, st>>>(p);
         exb_count_launches(2);
         rc = exb_check_launch("state_sweep_2p_kernel");
         if (prof) {
@@ -808,7 +947,7 @@ static int s2_launch(S2Params &p, const TS *Yp, cudaStream_t st, const ExbSweepP
             double tot = 0;
             for (int i = 0; i < 6; ++i) tot += (double)h[i];
             for (int i = 6; i < 10; ++i) tot += (double)h[i];
-            fprintf(stderr, "[s2 prof] grid %d patches %d: setup %.1f%% scan %.1f%% park+fence %.1f%% rows %.1f%% phaseB %.1f%% barriers %.1f%% | blocks: scalars+staging %.1f%% omega %.1f%% gram %.1f%% rest %.1f%%  (%.3e clk per CTA)\n",
+            fprintf(stderr, "[s2 prof] grid %d patches %d: setup %.1f%% scan %.1f%% park+fence %.1f%% rows %.1f%% phaseB %.1f%% barriers %.1f%% | blocks: scalars %.1f%% omega %.1f%% gram %.1f%% rest %.1f%%  (%.3e clk per CTA)\n",
                     grid, p.npatches, 100 * h[0] / tot, 100 * h[1] / tot, 100 * h[2] / tot, 100 * h[3] / tot, 100 * h[4] / tot, 100 * h[5] / tot,
                     100 * h[6] / tot, 100 * h[7] / tot, 100 * h[8] / tot, 100 * h[9] / tot, tot / grid);
         }
@@ -820,10 +959,10 @@ static int s2_launch(S2Params &p, const TS *Yp, cudaStream_t st, const ExbSweepP
     return rc;
 }
 
-// Called from state_sweep_pipe.cu (exb_state_sweep_pipe).  TS is the storage type of state and ye rows (float64, or
-// float32 with float64 arithmetic in registers: every row is read and rounded back exactly once).  xm == nullptr
-// selects the fused split/recombine mode (Xp then holds full ensemble values).  Returns EXB_ERR_UNSUPPORTED if no
-// variant fits (more than 103 members).
+// Called from state_update.cu.  TS is the storage type of state and ye rows (float64, or float32 with float64
+// arithmetic in registers: every row is read and rounded back exactly once).  xm == nullptr selects the fused
+// split/recombine mode (Xp then holds full ensemble values).  Returns EXB_ERR_UNSUPPORTED if no instantiation fits
+// (more than 103 members).
 template <typename TS>
 int exb_state_sweep_2p(TS *xm, TS *Xp, int64_t nlev, int64_t ny, int64_t nx, int nens, const double *grid_u, const TS *Yp,
                        const double *rec, const double *obgeo, const float4 *scan, int64_t nobs, int64_t ob_begin,
@@ -837,17 +976,10 @@ int exb_state_sweep_2p(TS *xm, TS *Xp, int64_t nlev, int64_t ny, int64_t nx, int
     p.y_begin = (int)y_begin; p.y_end = (int)y_end;
     p.kloc = exb_loc_const();
     const int need = (nens + 1 + 7) / 8;            // 8-member tiles incl. the pseudo-member
-    if (s2_warps() == 8) {
-        if (need <= 4) return s2_launch<4, TS, 8>(p, Yp, st, plan);
-        if (need <= 7) return s2_launch<7, TS, 8>(p, Yp, st, plan);
-        if (need <= 10) return s2_launch<10, TS, 8>(p, Yp, st, plan);
-        if (need <= 13) return s2_launch<13, TS, 8>(p, Yp, st, plan);
-        return EXB_ERR_UNSUPPORTED;
-    }
-    if (need <= 4) return s2_launch<4, TS, 16>(p, Yp, st, plan);
-    if (need <= 7) return s2_launch<7, TS, 16>(p, Yp, st, plan);
-    if (need <= 10) return s2_launch<10, TS, 16>(p, Yp, st, plan);
-    if (need <= 13) return s2_launch<13, TS, 16>(p, Yp, st, plan);
+    if (need <= 4) return s2_launch<4, TS>(p, Yp, st, plan);
+    if (need <= 7) return s2_launch<7, TS>(p, Yp, st, plan);
+    if (need <= 10) return s2_launch<10, TS>(p, Yp, st, plan);
+    if (need <= 13) return s2_launch<13, TS>(p, Yp, st, plan);
     return EXB_ERR_UNSUPPORTED;                       // larger ensembles: state_update_mma.cu / state_update.cu
 }
 
@@ -857,3 +989,73 @@ template int exb_state_sweep_2p<double>(double *, double *, int64_t, int64_t, in
 template int exb_state_sweep_2p<float>(float *, float *, int64_t, int64_t, int64_t, int, const double *, const float *,
                                        const double *, const double *, const float4 *, int64_t, int64_t, int64_t, int64_t,
                                        int64_t, int, unsigned long long *, cudaStream_t, const ExbSweepPlan *);
+
+// Row granularity of the patches for a state with nlev levels: sweeping row ranges whose edges are multiples of
+// this value never splits a patch between two calls.
+extern "C" int exb_state_sweep_row_granularity(int64_t nlev, int64_t ny, int64_t nx) {
+    int Lc, bty, btx;
+    s2_patch_shape(nlev, ny, nx, &Lc, &bty, &btx);
+    return bty;
+}
+
+// ------------------------------------------------------------------------------------------
+// sweep plan: the geometry-only part of the sweep, built ahead of the obs-space solve
+// ------------------------------------------------------------------------------------------
+__global__ void sweep_scan_from_flags_kernel(const double *__restrict__ geo, const uint8_t *__restrict__ assim, int64_t nobs,
+                                             float4 *__restrict__ scan) {
+    const int64_t k = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    if (k >= nobs) return;
+    float4 v;
+    v.x = (float)geo[GEO_UX * nobs + k];
+    v.y = (float)geo[GEO_UY * nobs + k];
+    v.z = (float)geo[GEO_UZ * nobs + k];
+    // same record as su_scan_records_kernel (state_update.cu) builds from rec[REC_ASSIM] after the solve
+    v.w = assim[k] ? (float)geo[GEO_THETA * nobs + k] * 1.000001f + 1e-7f : -1.f;
+    scan[k] = v;
+}
+
+static void sweep_plan_free(ExbSweepPlan *pl) {
+    if (!pl) return;
+    if (pl->was_used && pl->used) cudaStreamWaitEvent(pl->st, pl->used, 0);
+    if (pl->scan) cudaFreeAsync(pl->scan, pl->st);
+    sweep_free_lists(pl->lists, pl->st);
+    if (pl->ready) cudaEventDestroy(pl->ready);
+    if (pl->used) cudaEventDestroy(pl->used);
+    delete pl;
+}
+
+extern "C" int exb_sweep_plan_create(const double *grid_u, int64_t nlev, int64_t ny, int64_t nx, const double *obgeo,
+                                     const uint8_t *ob_assimilate, int64_t nobs, int64_t ob_begin, int64_t ob_end,
+                                     int64_t y_begin, int64_t y_end, int loc_mode, void *stream, void **plan) {
+    EXB_REQUIRE(grid_u && obgeo && ob_assimilate && plan, "null pointer");
+    EXB_REQUIRE(nlev > 0 && ny > 0 && nx > 0 && nobs > 0, "bad sizes");
+    EXB_REQUIRE(0 <= ob_begin && ob_begin <= ob_end && ob_end <= nobs && 0 <= y_begin && y_begin < y_end && y_end <= ny, "bad ranges");
+    *plan = nullptr;
+    cudaStream_t st = (cudaStream_t)stream;
+    ExbSweepPlan *pl = new ExbSweepPlan();
+    struct Guard { ExbSweepPlan *p; ~Guard() { if (p) sweep_plan_free(p); } } guard{pl};
+    pl->nlev = nlev; pl->ny = ny; pl->nx = nx; pl->nobs = nobs; pl->ob_begin = ob_begin; pl->ob_end = ob_end;
+    pl->y_begin = y_begin; pl->y_end = y_end; pl->loc_mode = loc_mode; pl->grid_u = grid_u; pl->obgeo = obgeo; pl->st = st;
+    EXB_CUDA(cudaEventCreateWithFlags(&pl->ready, cudaEventDisableTiming));
+    EXB_CUDA(cudaEventCreateWithFlags(&pl->used, cudaEventDisableTiming));
+    EXB_CUDA(exb_malloc_async(&pl->scan, (size_t)nobs * sizeof(float4), st));
+    sweep_scan_from_flags_kernel<<<(unsigned)ceil_div64(nobs, 256), 256, 0, st>>>(obgeo, ob_assimilate, nobs, pl->scan);
+    exb_count_launches(1);
+    if (sweep_lists_wanted(loc_mode, ob_begin, ob_end)) {
+        int Lc, bty, btx;
+        s2_patch_shape(nlev, ny, nx, &Lc, &bty, &btx);
+        const int rc = sweep_build_lists(grid_u, ny * nx, (int)nx, (int)y_begin, (int)y_end, bty, btx, pl->scan, ob_begin,
+                                         ob_end, st, &pl->lists);
+        if (rc != EXB_OK) return rc;
+        pl->have_lists = true;
+    }
+    EXB_CUDA(cudaEventRecord(pl->ready, st));
+    guard.p = nullptr;
+    *plan = pl;
+    return exb_check_launch("sweep_scan_from_flags_kernel");
+}
+
+extern "C" int exb_sweep_plan_destroy(void *plan) {
+    sweep_plan_free(static_cast<ExbSweepPlan *>(plan));
+    return EXB_OK;
+}

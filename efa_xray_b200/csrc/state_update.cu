@@ -25,10 +25,10 @@ int exb_state_update_mma_f64(double *xm, double *Xp, int64_t nlev, int64_t ny, i
                              unsigned long long *counters, cudaStream_t st);
 
 template <typename TS>
-int exb_state_sweep_pipe(TS *xm, TS *Xp, int64_t nlev, int64_t ny, int64_t nx, int nens, const double *grid_u, const TS *Yp,
-                         const double *rec, const double *obgeo, const float4 *scan, int64_t nobs, int64_t ob_begin,
-                         int64_t ob_end, int64_t y_begin, int64_t y_end, int loc_mode, unsigned long long *counters,
-                         cudaStream_t st, const ExbSweepPlan *plan = nullptr);
+int exb_state_sweep_2p(TS *xm, TS *Xp, int64_t nlev, int64_t ny, int64_t nx, int nens, const double *grid_u, const TS *Yp,
+                       const double *rec, const double *obgeo, const float4 *scan, int64_t nobs, int64_t ob_begin,
+                       int64_t ob_end, int64_t y_begin, int64_t y_end, int loc_mode, unsigned long long *counters,
+                       cudaStream_t st, const ExbSweepPlan *plan = nullptr);
 
 #define SU_NT 256
 #define SU_QCAP 16
@@ -353,13 +353,13 @@ static int state_update_impl(T *xm, T *Xp, int64_t nlev, int64_t ny, int64_t nx,
     exb_count_launches(1);
     {
         // FP64 tensor-core sweeps (float32 states: float32 storage, float64 arithmetic in registers).
-        // EXB_SU_IMPL = pipe (default: warp-specialised, state_sweep_pipe.cu) | mma (state_update_mma.cu, float64
-        // only, also the fallback for ensembles > 103 members) | vector (the kernel below, arithmetic in T)
+        // EXB_SU_IMPL = pipe (default: two-phase, state_sweep_2p.cu) | mma (state_update_mma.cu, float64 only, also the
+        // fallback for ensembles > 103 members) | vector (the kernel below, arithmetic in T)
         const char *impl = getenv("EXB_SU_IMPL");
         const bool vec = impl && strcmp(impl, "vector") == 0, mma = impl && strcmp(impl, "mma") == 0;
         if (!vec && !mma) {
-            int rc = exb_state_sweep_pipe<T>(xm, Xp, nlev, ny, nx, nens, grid_u, Yp, rec, obgeo, scan, nobs, ob_begin, ob_end,
-                                             0, ny, loc_mode, counters, st);
+            int rc = exb_state_sweep_2p<T>(xm, Xp, nlev, ny, nx, nens, grid_u, Yp, rec, obgeo, scan, nobs, ob_begin, ob_end,
+                                           0, ny, loc_mode, counters, st);
             if (rc != EXB_ERR_UNSUPPORTED) {
                 cudaFreeAsync(scan, st);
                 return rc;
@@ -423,8 +423,8 @@ static int state_sweep_impl(T *X, int64_t nlev, int64_t ny, int64_t nx, int nens
             return EXB_ERR_ARG;
         }
         EXB_CUDA(cudaStreamWaitEvent(st, plan->ready, 0));
-        const int rc = exb_state_sweep_pipe<T>(nullptr, X, nlev, ny, nx, nens, grid_u, Yp, rec, obgeo, plan->scan, nobs, ob_begin,
-                                               ob_end, y_begin, y_end, loc_mode, counters, st, plan);
+        const int rc = exb_state_sweep_2p<T>(nullptr, X, nlev, ny, nx, nens, grid_u, Yp, rec, obgeo, plan->scan, nobs, ob_begin,
+                                             ob_end, y_begin, y_end, loc_mode, counters, st, plan);
         cudaEventRecord(plan->used, st);
         plan->was_used = true;
         return rc;
@@ -433,8 +433,8 @@ static int state_sweep_impl(T *X, int64_t nlev, int64_t ny, int64_t nx, int nens
     EXB_CUDA(exb_malloc_async(&scan, (size_t)nobs * sizeof(float4), st));
     su_scan_records_kernel<<<(unsigned)ceil_div64(nobs, 256), 256, 0, st>>>(obgeo, rec, nobs, scan);
     exb_count_launches(1);
-    const int rc = exb_state_sweep_pipe<T>(nullptr, X, nlev, ny, nx, nens, grid_u, Yp, rec, obgeo, scan, nobs, ob_begin,
-                                           ob_end, y_begin, y_end, loc_mode, counters, st);
+    const int rc = exb_state_sweep_2p<T>(nullptr, X, nlev, ny, nx, nens, grid_u, Yp, rec, obgeo, scan, nobs, ob_begin,
+                                         ob_end, y_begin, y_end, loc_mode, counters, st);
     cudaFreeAsync(scan, st);
     return rc;
 }

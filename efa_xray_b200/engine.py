@@ -164,14 +164,6 @@ def stencil_search(grid: GridTables, ob_lat, ob_lon, force_general=False, dev_ta
     return idx4, w4, nex
 
 
-def _dist_search_wanted():
-    """EXB_DIST_SEARCH=1: the ranks of a sharded analysis search a slice of the obs each and all-gather the stencils
-    instead of every rank searching all obs.  Verified at N = 2 (identical analysis) but not faster there -- the setup's
-    critical path is the predecessor-list build, not the search -- so it is off by default."""
-    import os
-    return os.environ.get('EXB_DIST_SEARCH', '0') == '1'
-
-
 def pseudo_distance_order(grid: GridTables, lat, lon, npt):
     """Flat indices of the npt grid points with the smallest pseudo-distance to (lat, lon), ordered by (distance,
     flat index): nearest_points for any npt (state/ensemble.py:152-168)."""
@@ -204,31 +196,7 @@ def ob_priors(X, grid: GridTables, obs: ObsArrays, sfx, nlev=None, band=None, gr
                    'row1': torch.as_tensor(np.ascontiguousarray(obs.row1, dtype=np.int64)).to(dev),
                    'tw0': _dev_f64(obs.tw0, dev), 'tw1': _dev_f64(obs.tw1, dev)}
     tables = (obs_dev['lat'], obs_dev['lon'], obs_dev['sinlat'], obs_dev['coslon'])
-    world = 1
-    if band is not None:
-        import torch.distributed as dist
-        if dist.is_initialized():
-            world = dist.get_world_size(group)
-    if world > 1 and obs.nobs >= 64 * world and _dist_search_wanted():
-        # every rank needs the stencils of ALL obs (it gathers the points of its own band), but the search itself is
-        # the same on every rank: each one searches a slice of the obs and the slices are all-gathered (6 MB)
-        import torch.distributed as dist
-        rank = dist.get_rank(group)
-        chunk = -(-obs.nobs // world)
-        a, b = min(rank * chunk, obs.nobs), min((rank + 1) * chunk, obs.nobs)
-        idx4 = torch.zeros((world * chunk, 4), dtype=torch.int64, device=dev)
-        w4 = torch.zeros((world * chunk, 4), dtype=torch.float64, device=dev)
-        i_mine, w_mine, nex = stencil_search(grid, None, None, dev_tables=tuple(t[a:b] for t in tables))
-        i_pad = torch.zeros((chunk, 4), dtype=torch.int64, device=dev)
-        w_pad = torch.zeros((chunk, 4), dtype=torch.float64, device=dev)
-        i_pad[:b - a].copy_(i_mine)
-        w_pad[:b - a].copy_(w_mine)
-        dist.all_gather_into_tensor(idx4, i_pad, group=group)
-        dist.all_gather_into_tensor(w4, w_pad, group=group)
-        dist.all_reduce(nex, group=group)
-        idx4, w4 = idx4[:obs.nobs].contiguous(), w4[:obs.nobs].contiguous()
-    else:
-        idx4, w4, nex = stencil_search(grid, None, None, dev_tables=tables)
+    idx4, w4, nex = stencil_search(grid, None, None, dev_tables=tables)
     # 8-point stencil = 4 space points x 2 time levels, re-based to the band's shard (index/weight bookkeeping only)
     y0, y1 = band if band is not None else (0, grid.ny)
     idx8 = torch.empty((obs.nobs, 8), dtype=torch.int64, device=dev)
@@ -321,15 +289,10 @@ class ObsPlan:
 
 class SweepPlan:
     """The geometry-only part of the fused state sweep (scan records of the obs, candidate lists per coarse tile),
-    built on a side stream while the ob priors and the obs-space solve are computed (exb_sweep_plan_create).
+    built on a side stream while the ob priors and the obs-space solve are computed (exb_sweep_plan_create).  Creating
+    the plan blocks its caller until the counting pass is done (the list is sized on the host)."""
 
-    `after`: an event on the current stream after which grid_u, geo and the ob arrays are valid (default: everything
-    enqueued on the current stream so far).  background=True makes the call from a helper thread: creating the plan
-    blocks its caller until the counting pass is done (the list is sized on the host), and the thread that enqueues
-    the obs-space solve should not wait for that.  wait() joins it; the sweep needs the handle."""
-
-    def __init__(self, grid_u, nlev, ny, nx, obs_dev, geo, nobs, loc_mode, y_begin=0, y_end=None, after=None,
-                 background=False):
+    def __init__(self, grid_u, nlev, ny, nx, obs_dev, geo, nobs, loc_mode, y_begin=0, y_end=None):
         torch = _torch()
         self.handle = C.c_void_p()
         self.grid_u, self.geo = grid_u, geo          # keep the inputs alive and identical to what the sweep is given
@@ -337,47 +300,12 @@ class SweepPlan:
         ready = obs_dev.get('_ready')
         if ready is not None:
             self.stream.wait_event(ready)
-        if after is not None:
-            self.stream.wait_event(after)
-        else:
-            self.stream.wait_stream(torch.cuda.current_stream())
-        self._thread, self._exc = None, None
-        assim = obs_dev['assimilate']
-
-        def create():
-            _lib.call('exb_sweep_plan_create', _lib.ptr(grid_u), nlev, ny, nx, _lib.ptr(geo), _lib.ptr(assim), nobs,
-                      0, nobs, y_begin, ny if y_end is None else y_end, loc_mode, C.c_void_p(self.stream.cuda_stream),
-                      C.byref(self.handle))
-
-        if not background:
-            create()
-            return
-
-        def work():
-            try:
-                with torch.cuda.device(geo.device):       # the current device is a per-thread setting
-                    create()
-            except BaseException as e:                   # re-raised by wait()
-                self._exc = e
-
-        import threading
-        self._thread = threading.Thread(target=work, name='exb-sweep-plan', daemon=True)
-        self._thread.start()
-
-    def wait(self):
-        t, self._thread = self._thread, None
-        if t is not None:
-            t.join()
-        e, self._exc = self._exc, None
-        if e is not None:
-            raise e
-        return self
+        self.stream.wait_stream(torch.cuda.current_stream())
+        _lib.call('exb_sweep_plan_create', _lib.ptr(grid_u), nlev, ny, nx, _lib.ptr(geo), _lib.ptr(obs_dev['assimilate']),
+                  nobs, 0, nobs, y_begin, ny if y_end is None else y_end, loc_mode, C.c_void_p(self.stream.cuda_stream),
+                  C.byref(self.handle))
 
     def destroy(self):
-        try:
-            self.wait()
-        except BaseException:
-            pass
         if self.handle:
             _lib.call('exb_sweep_plan_destroy', self.handle)
             self.handle = C.c_void_p()
@@ -635,14 +563,6 @@ def analysis_device(X, nlev, grid: GridTables, obs: ObsArrays, loc_mode, inflati
                 plan = ObsPlan(obs_dev, geo, obs.nobs, loc_mode)
             fused = fused_sweep_available(X.dtype, nens)
             grid_u = grid.u if band is None else grid.u[:, y0 * nx:y1 * nx].contiguous()
-            # EXB_PLAN_THREAD=1: the sweep plan is made from a helper thread (see SweepPlan).  Measured on config 3: the
-            # 1.3 ms this thread no longer waits are given back by a solve that shares the device with the plan's
-            # kernels (164.9 against 165.3 ms per analysis) -- off by default.
-            plan_thread = os.environ.get('EXB_PLAN_THREAD', '0') == '1'
-            ev_geom = None
-            if plan_thread:
-                ev_geom = torch.cuda.Event()
-                ev_geom.record()             # obs arrays, geo and grid_u are valid from here on
             if Y is None:
                 Yp, nex = ob_priors(X, grid, obs, sfx, nlev=nlev, band=band, group=group, obs_dev=obs_dev)
             elif isinstance(Y, tuple):   # (H.x, n_exact) from ob_priors, owned by this call
@@ -652,21 +572,17 @@ def analysis_device(X, nlev, grid: GridTables, obs: ObsArrays, loc_mode, inflati
             Ym = torch.empty(obs.nobs, dtype=X.dtype, device=dev)
             _lib.call('exb_split_mean_pert_' + sfx, _lib.ptr(Yp), _lib.ptr(Ym), obs.nobs, nens, _lib.stream_ptr())
             tm.mark('setup_ob_priors')
-            lists_first = os.environ.get('EXB_PLAN_ORDER', '1') != '0'
-            if plan is not None and lists_first:
+            if plan is not None:
                 # the solve is next on the critical path: its lists are filled before the sweep's plan is started
                 plan.finish()
             if fused and sweep_plan_wanted():
                 # candidate lists of the sweep: geometry only as well, built on another side stream.  Creating the plan
                 # blocks its caller until the counting pass is done, so it comes after the ob priors have been enqueued
                 # (the device computes them meanwhile)
-                splan = SweepPlan(grid_u, nlev, ny, nx, obs_dev, geo, obs.nobs, loc_mode, after=ev_geom,
-                                  background=plan_thread)
+                splan = SweepPlan(grid_u, nlev, ny, nx, obs_dev, geo, obs.nobs, loc_mode)
             if not fused:
                 xm = torch.empty(nrows, dtype=X.dtype, device=dev)
                 _lib.call('exb_split_mean_pert_' + sfx, _lib.ptr(X), _lib.ptr(xm), nrows, nens, _lib.stream_ptr())
-            if plan is not None and not lists_first:
-                plan.finish()
             tm.mark('setup_plans')
             rec = torch.empty((8, obs.nobs), dtype=torch.float64, device=dev)
             counters = torch.zeros(2, dtype=torch.int64, device=dev)
@@ -684,8 +600,6 @@ def analysis_device(X, nlev, grid: GridTables, obs: ObsArrays, loc_mode, inflati
                 obs_solve(Ym, Yp, obs_dev, geo, nens, loc_mode, rec, counters, sfx, plan=plan)
             tm.mark('obs_solve')
             if fused:
-                if splan is not None:
-                    splan.wait()
                 for ya, yb in (sweep_bands or [(0, ny)]):
                     if before_band is not None:
                         before_band(ya, yb)

@@ -222,7 +222,7 @@ int exb_obs_solve_async_status(void);
  *   Yp, rec, obgeo                           as written by exb_obs_solve_* / exb_obs_prepare
  * counters (device uint64[2], may be NULL): [1] += number of (ob, grid point) pairs with non-zero
  * weight = sum_k |F_s(k)| / nlev of SURVEY.md section 8d.
- * Up to 103 members both types run on the warp-specialised FP64 tensor-core kernel (float32: float32 storage,
+ * Up to 103 members both types run on the two-phase FP64 tensor-core kernel (float32: float32 storage,
  * float64 arithmetic), which synchronises the stream once to size its candidate lists; EXB_SU_IMPL = pipe | mma |
  * vector selects the kernel (DESIGN.md section 4.3). */
 int exb_state_update_f64(double *xm, double *Xp, int64_t nlev, int64_t ny, int64_t nx, int nens,

@@ -380,11 +380,9 @@ def _analysis_with_env(case, env, bands=None):
     dict(ny=31, nx=60, nmem=16, nvars=2, ntimes=1, nobs=7000, cutoff_km=9000.0, seed=45, frac_skip=0.02),
 ])
 def test_sweep_variants_agree(kw):
-    """The two-phase fused sweep (default), the same kernel without candidate lists, its two-CTAs-per-SM
-    instantiation, band-by-band calls, the
-    concurrent producer/consumer kernel of round 1 (EXB_SP_IMPL=v3), and the three-call forms (split / sweep /
-    recombine) on the earlier tensor-core kernel and on the vector kernel all apply the same obs in the same order
-    to every state row."""
+    """The two-phase fused sweep (default), the same kernel without a sweep plan or without candidate lists,
+    band-by-band calls, and the three-call forms (split / sweep / recombine) on the same kernel, on the earlier
+    tensor-core kernel and on the vector kernel all apply the same obs in the same order to every state row."""
     case = make_case(**kw)
     prior = case.to_vect()
     ref, res0 = _analysis_with_env(case, {'EXB_SU_IMPL': 'mma', 'EXB_OBS_IMPL': 'persistent'})
@@ -393,9 +391,6 @@ def test_sweep_variants_agree(kw):
     runs = {
         'pipe_fused': _analysis_with_env(case, {}),
         'pipe_noplan': _analysis_with_env(case, {'EXB_SWEEP_PLAN': '0'}),
-        'pipe_8warps': _analysis_with_env(case, {'EXB_S2_WARPS': '8'}),        # two CTAs of 64 rows per SM
-        'pipe_v3': _analysis_with_env(case, {'EXB_SP_IMPL': 'v3'}),
-        'pipe_v3_split': _analysis_with_env(case, {'EXB_SP_IMPL': 'v3', 'EXB_FUSED': '0'}),
         'pipe_nolist': _analysis_with_env(case, {'EXB_SWEEP_NOLIST': '1'}),
         'pipe_split': _analysis_with_env(case, {'EXB_FUSED': '0'}),
         'vector': _analysis_with_env(case, {'EXB_SU_IMPL': 'vector'}),

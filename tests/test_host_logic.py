@@ -20,17 +20,12 @@ def test_sweep_band_schedule_covers_rows_on_patch_boundaries(lib):
     assert bands[-1][1] - bands[-1][0] <= (bands[0][1] - bands[0][0])
 
 
-def test_patch_shape_of_the_two_kernel_instantiations(lib, monkeypatch):
-    """128 rows per patch with one CTA of 16 warps per SM, 64 with two CTAs of 8 (EXB_S2_WARPS=8): the band schedule
-    follows the patch rows of the instantiation in use."""
+def test_patch_shape_of_the_sweep_kernel(lib):
+    """128 rows per patch with one CTA of 16 warps per SM: the band schedule follows the kernel's patch rows."""
     from efa_xray_b200 import engine
-    monkeypatch.delenv('EXB_S2_WARPS', raising=False)
     assert lib.exb_state_sweep_row_granularity(3, 721, 1440) == 6       # 42 points x 3 levels: 6 x 7 points
-    assert lib.exb_state_sweep_row_granularity(10, 721, 1440) == 3      # 12 points x 10 levels: 3 x 4
-    monkeypatch.setenv('EXB_S2_WARPS', '8')
-    assert lib.exb_state_sweep_row_granularity(3, 721, 1440) == 3       # 21 points: 3 x 7
-    g = lib.exb_state_sweep_row_granularity(10, 721, 1440)              # 6 points: 2 x 3
-    assert g == 2
+    g = lib.exb_state_sweep_row_granularity(10, 721, 1440)              # 12 points x 10 levels: 3 x 4
+    assert g == 3
     for a, b in engine.sweep_band_schedule(10, 721, 1440)[:-1]:
         assert b % g == 0
 

@@ -4,7 +4,7 @@
 * the obs-space solve as a dependency-driven (sparse triangular) solve: a row needs only the published records of the
   EARLIER obs whose support reaches it, applied in index order; rows can then be processed in any order compatible
   with those dependencies, by any number of workers (obs_solve_dag.cu, its distributed variant);
-* the blocked 8-ob form of the state update (Gram recurrence) used on the FP64 tensor cores (state_sweep_pipe.cu);
+* the blocked 8-ob form of the state update (Gram recurrence) used on the FP64 tensor cores (state_sweep_2p.cu);
 * the constants of the branch-free localisation weight (common.cuh) are the series of asin(sqrt a)/sqrt a.
 """
 import os
@@ -109,15 +109,6 @@ def test_blocked_gram_recurrence_equals_sequential_rank1_updates():
     xb = xext - e @ Yext
     np.testing.assert_allclose(xb[:-1], x, rtol=1e-12, atol=1e-13)
     np.testing.assert_allclose(xb[-1], mean, rtol=1e-14)
-    # and the matrix form e = M g of the same recurrence (the EXB_SP_MG variant)
-    M = np.zeros((8, 8))
-    for j in range(8):
-        m = np.zeros(8)
-        for q in range(8):
-            m[q] = omega[q] * ((1.0 if q == j else 0.0) - G[q, :q] @ m[:q])
-        M[:, j] = m
-    np.testing.assert_allclose(M @ g, e, rtol=1e-11, atol=1e-15)
-    assert np.allclose(np.triu(M, 1), 0.0)
 
 
 def test_fast_localisation_weight_constants_and_accuracy():
