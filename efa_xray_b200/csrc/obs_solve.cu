@@ -1,19 +1,14 @@
-// Obs-space serial solve (piece 2 + the obs-row half of piece 4 of the north star).
+// Obs-space serial solve (piece 2 + the obs-row half of piece 4 of the north star): the entry points and the choice
+// between the two solvers, each the only one that runs on its inputs.
 //
-// The Nobs obs-space rows of the reference's augmented state (assimilation.py:149-150) only ever read
-// other obs-space rows (ensrf.py:61-64, :95, :141), so they are evolved here on their own, in the
-// reference's serial order, and leave behind one record per ob (ye_k and a few scalars) from which
-// the state sweep (state_update.cu) can update every state row independently.
+//   obs_solve_dag.cu         dependency-driven solve: the serial chain shrinks to the longest dependency path.  Used
+//                            with localisation; it declines (EXB_ERR_UNSUPPORTED) a dependency graph more than half
+//                            dense, where walking predecessor lists costs more than the panels save.
+//   obs_solve_persistent.cu  one cooperative kernel walking panels of 64 obs.  Used without localisation, where every
+//                            ob depends on every earlier one, and for the graphs the dependency-driven solve declines.
 //
-// Blocked right-looking form of the serial loop, panel width PB:
-//   panel kernel   (1 CTA)   : obs k = b0..b0+PB-1 strictly in order; the panel's rows live in
-//                              registers, ye_k is broadcast through shared memory.  This is the only
-//                              truly serial part of the whole analysis.
-//   trailing kernel (many CTAs): every later row j >= b0+PB applies the PB panel obs in order.
-// Rows j < k are never read again by the reference (ensrf.py:61-64 reads row k at step k only), so they
-// are not updated; row k is frozen at step k and therefore ends up holding ye_k.
-//
-// Thread mapping: a row is owned by a group of 8 lanes, lane s holds members s, s+8, ... (MC per lane).
+// EXB_OBS_IMPL = dag | persistent picks one regardless of the inputs (tests compare the two); dag then also runs on a
+// dense graph.
 #include "common.cuh"
 #include <cstring>
 #include <cstdlib>
@@ -27,285 +22,6 @@ int exb_obs_solve_persistent(T *Ym, T *Yp, const double *ob_value, const double 
                              const double *geo, int64_t nobs, int nens, int loc_mode, double *rec,
                              unsigned long long *counters, cudaStream_t st);
 
-#define PB 64                 // panel width (obs per panel kernel)
-#define GS 8                  // lanes per row
-
-template <typename T, int MC>
-struct RowRegs {
-    T x[MC];
-};
-
-template <int N>
-__device__ __forceinline__ double group_sum(double v, unsigned mask) {
-#pragma unroll
-    for (int off = N / 2; off > 0; off >>= 1) v += __shfl_xor_sync(mask, v, off);
-    return v;
-}
-
-// scalars of the ob being applied, broadcast through shared memory
-struct ObScalars {
-    double ux, uy, uz, inv_hw, a_max;
-    double innov, c1, beta;
-    int assim;
-};
-
-template <typename T, int MC>
-__global__ void __launch_bounds__(PB *GS, 1)
-obs_panel_kernel(T *__restrict__ Ym, T *__restrict__ Yp, const double *__restrict__ ob_value,
-                 const double *__restrict__ ob_error, const uint8_t *__restrict__ ob_assim,
-                 const double *__restrict__ geo, int64_t nobs, int nens, int64_t b0, int loc_mode,
-                 double *__restrict__ rec, unsigned long long *__restrict__ counters) {
-    // Serial chain, one step per ob.  Everything that does not depend on the evolving rows is taken out of
-    // the loop: the PB x PB pairwise localisation weights are evaluated in parallel first, and the broadcast
-    // buffers are double-buffered so that a step needs one barrier.
-    __shared__ T s_ye[2][GS * MC];
-    __shared__ ObScalars s_ob[2];
-    __shared__ double s_W[PB * PB];          // s_W[k*PB + j]: weight of ob k at row j (j > k)
-    __shared__ double s_g[5][PB];
-
-    const int g = threadIdx.x / GS;          // row within the panel
-    const int s = threadIdx.x % GS;
-    const int lane = threadIdx.x % 32;
-    const unsigned gmask = 0xffu << (lane & ~(GS - 1));
-    const int64_t j = b0 + g;
-    const bool valid = j < nobs;
-    const int nb = (int)((nobs - b0) < PB ? (nobs - b0) : PB);
-
-    T x[MC];
-#pragma unroll
-    for (int i = 0; i < MC; ++i) {
-        const int m = s + GS * i;
-        x[i] = (valid && m < nens) ? Yp[j * nens + m] : (T)0;
-    }
-    double mj = valid ? (double)Ym[j] : 0.0;
-    for (int i = threadIdx.x; i < PB; i += PB * GS) {
-        const int64_t kk = (b0 + i < nobs) ? b0 + i : nobs - 1;
-        s_g[0][i] = geo[GEO_UX * nobs + kk];
-        s_g[1][i] = geo[GEO_UY * nobs + kk];
-        s_g[2][i] = geo[GEO_UZ * nobs + kk];
-        s_g[3][i] = geo[GEO_INVHW * nobs + kk];
-        s_g[4][i] = geo[GEO_AMAX * nobs + kk];
-    }
-    __syncthreads();
-    for (int idx = threadIdx.x; idx < PB * PB; idx += PB * GS) {
-        const int k = idx / PB, jj = idx % PB;
-        double w = 0.0;
-        if (jj > k && jj < nb) {
-            w = 1.0;
-            if (loc_mode == EXB_LOC_GC)
-                w = loc_weight(hav_a(s_g[0][jj], s_g[1][jj], s_g[2][jj], s_g[0][k], s_g[1][k], s_g[2][k]),
-                               s_g[3][k], s_g[4][k]);
-        }
-        s_W[idx] = w;
-    }
-    // per-ob inputs of this row when it becomes the active ob (only lane s == 0 of the group uses them)
-    double my_val = 0.0, my_err = 1.0, my_wself = 1.0;
-    int my_assim = 0;
-    if (valid && s == 0) {
-        my_val = ob_value[j];
-        my_err = ob_error[j];
-        my_assim = ob_assim[j] != 0;
-        my_wself = (loc_mode == EXB_LOC_GC) ? loc_weight(0.0, s_g[3][g], s_g[4][g]) : 1.0;
-    }
-    unsigned long long npairs = 0;
-    __syncthreads();
-
-    for (int k = 0; k < nb; ++k) {
-        const int buf = k & 1;
-        if (g == k) {
-            // ensrf.py:63-70: mye, ye, varye = np.var(ye) (ddof 0), here as E[x^2] - mean^2
-            double s0 = 0.0, s1 = 0.0, q0 = 0.0, q1 = 0.0;
-#pragma unroll
-            for (int i = 0; i < MC; i += 2) {
-                const double a = (double)x[i];
-                s0 += a; q0 += a * a;
-                if (i + 1 < MC) { const double b = (double)x[i + 1]; s1 += b; q1 += b * b; }
-            }
-            double sum = s0 + s1, sq = q0 + q1;
-#pragma unroll
-            for (int off = GS / 2; off > 0; off >>= 1) {
-                sum += __shfl_xor_sync(gmask, sum, off);
-                sq += __shfl_xor_sync(gmask, sq, off);
-            }
-#pragma unroll
-            for (int i = 0; i < MC; ++i) s_ye[buf][s * MC + i] = x[i];
-            if (s == 0) {
-                const int64_t kk = b0 + k;
-                const double inv_n = 1.0 / (double)nens;
-                const double mean = sum * inv_n;
-                const double varye = fmax(sq * inv_n - mean * mean, 0.0);
-                const double innov = my_val - mj;                            // ensrf.py:86
-                const double kdenom = varye + my_err;                         // ensrf.py:91
-                const double c1 = 1.0 / ((double)(nens - 1) * kdenom);        // ensrf.py:95, :119
-                const double beta = 1.0 / (1.0 + sqrt(my_err / kdenom));      // ensrf.py:135
-                s_ob[buf].innov = innov; s_ob[buf].c1 = c1; s_ob[buf].beta = beta; s_ob[buf].assim = my_assim;
-                rec[REC_PRIOR_MEAN * nobs + kk] = mj;                         // ensrf.py:66
-                rec[REC_PRIOR_VAR * nobs + kk] = varye;                       // ensrf.py:70
-                rec[REC_INNOV * nobs + kk] = innov;
-                rec[REC_C1 * nobs + kk] = c1;
-                rec[REC_BETA * nobs + kk] = beta;
-                rec[REC_ASSIM * nobs + kk] = my_assim ? 1.0 : 0.0;
-                if (my_assim) {
-                    // the ob's own row: weight at distance 0, kcov = ye.ye/(N-1)  (ensrf.py:144-147)
-                    const double kmat = my_wself * sq * c1;
-                    const double shrink = 1.0 - beta * kmat;
-                    rec[REC_POST_MEAN * nobs + kk] = mj + kmat * innov;
-                    rec[REC_POST_VAR * nobs + kk] = varye * shrink * shrink;
-                    if (my_wself != 0.0) npairs++;
-                } else {
-                    rec[REC_POST_MEAN * nobs + kk] = nan("");
-                    rec[REC_POST_VAR * nobs + kk] = nan("");
-                }
-            }
-        }
-        __syncthreads();
-        if (g > k && valid && s_ob[buf].assim) {
-            const double w = s_W[k * PB + g];
-            if (w != 0.0) {
-                T ye[MC];
-                T d0 = 0, d1 = 0, d2 = 0, d3 = 0;
-#pragma unroll
-                for (int i = 0; i < MC; ++i) ye[i] = s_ye[buf][s * MC + i];
-#pragma unroll
-                for (int i = 0; i < MC; i += 4) {
-                    d0 += x[i] * ye[i];
-                    if (i + 1 < MC) d1 += x[i + 1] * ye[i + 1];
-                    if (i + 2 < MC) d2 += x[i + 2] * ye[i + 2];
-                    if (i + 3 < MC) d3 += x[i + 3] * ye[i + 3];
-                }
-                const double dot = group_sum<GS>((double)((d0 + d1) + (d2 + d3)), gmask);
-                const double kmat = w * dot * s_ob[buf].c1;         // loc * kcov / kdenom, ensrf.py:115-119
-                mj += kmat * s_ob[buf].innov;                       // ensrf.py:130
-                const T f = (T)(s_ob[buf].beta * kmat);             // ensrf.py:136
-#pragma unroll
-                for (int i = 0; i < MC; ++i) x[i] -= f * ye[i];     // ensrf.py:141
-                if (s == 0) npairs++;
-            }
-        }
-    }
-    if (valid) {
-#pragma unroll
-        for (int i = 0; i < MC; ++i) {
-            const int m = s + GS * i;
-            if (m < nens) Yp[j * nens + m] = x[i];
-        }
-        if (s == 0) Ym[j] = (T)mj;
-    }
-    if (counters && npairs) atomicAdd(&counters[0], npairs);
-}
-
-// Rows j >= b0+PB apply the (frozen) panel obs in order.
-#define TR_THREADS 256
-template <typename T, int MC>
-__global__ void __launch_bounds__(TR_THREADS)
-obs_trailing_kernel(T *__restrict__ Ym, T *__restrict__ Yp, const double *__restrict__ geo,
-                    const double *__restrict__ rec, int64_t nobs, int nens, int64_t b0, int loc_mode,
-                    unsigned long long *__restrict__ counters) {
-    __shared__ double s_geo[5][PB];      // ux uy uz inv_hw a_max
-    __shared__ double s_sc[3][PB];       // innov c1 beta
-    __shared__ int s_assim[PB];
-    const int nb = PB;                   // only launched for full panels
-    for (int i = threadIdx.x; i < PB; i += TR_THREADS) {
-        const int64_t kk = b0 + i;
-        s_geo[0][i] = geo[GEO_UX * nobs + kk];
-        s_geo[1][i] = geo[GEO_UY * nobs + kk];
-        s_geo[2][i] = geo[GEO_UZ * nobs + kk];
-        s_geo[3][i] = geo[GEO_INVHW * nobs + kk];
-        s_geo[4][i] = geo[GEO_AMAX * nobs + kk];
-        s_sc[0][i] = rec[REC_INNOV * nobs + kk];
-        s_sc[1][i] = rec[REC_C1 * nobs + kk];
-        s_sc[2][i] = rec[REC_BETA * nobs + kk];
-        s_assim[i] = rec[REC_ASSIM * nobs + kk] != 0.0;
-    }
-    __syncthreads();
-
-    const int s = threadIdx.x % GS;
-    const int lane = threadIdx.x % 32;
-    const int gbase = lane & ~(GS - 1);
-    const unsigned gmask = 0xffu << gbase;
-    const int64_t j = b0 + PB + blockIdx.x * (int64_t)(TR_THREADS / GS) + threadIdx.x / GS;
-    const bool valid = j < nobs;
-    double ux = 0, uy = 0, uz = 0;
-    if (valid) { ux = geo[GEO_UX * nobs + j]; uy = geo[GEO_UY * nobs + j]; uz = geo[GEO_UZ * nobs + j]; }
-
-    T x[MC];
-    double mj = 0.0;
-    bool loaded = false, dirty = false;
-    unsigned long long npairs = 0;
-
-    for (int k0 = 0; k0 < nb; k0 += GS) {
-        // each lane of the group tests one of the next GS panel obs against this row
-        const int kt = k0 + s;
-        double wk = 0.0;
-        if (valid && s_assim[kt]) {
-            wk = 1.0;
-            if (loc_mode == EXB_LOC_GC)
-                wk = loc_weight(hav_a(ux, uy, uz, s_geo[0][kt], s_geo[1][kt], s_geo[2][kt]), s_geo[3][kt], s_geo[4][kt]);
-        }
-        if (!__any_sync(0xffffffffu, wk != 0.0)) continue;
-#pragma unroll
-        for (int q = 0; q < GS; ++q) {
-            const double w = __shfl_sync(0xffffffffu, wk, gbase + q);
-            if (w != 0.0) {
-                const int k = k0 + q;
-                if (!loaded) {
-#pragma unroll
-                    for (int i = 0; i < MC; ++i) {
-                        const int m = s + GS * i;
-                        x[i] = (m < nens) ? Yp[j * nens + m] : (T)0;
-                    }
-                    mj = (double)Ym[j];
-                    loaded = true;
-                }
-                const T *yrow = Yp + (b0 + k) * nens;
-                T ye[MC];
-                double dot = 0.0;
-#pragma unroll
-                for (int i = 0; i < MC; ++i) {
-                    const int m = s + GS * i;
-                    ye[i] = (m < nens) ? yrow[m] : (T)0;
-                    dot += (double)(x[i] * ye[i]);
-                }
-                dot = group_sum<GS>(dot, gmask);
-                const double kmat = w * dot * s_sc[1][k];
-                mj += kmat * s_sc[0][k];
-                const T f = (T)(s_sc[2][k] * kmat);
-#pragma unroll
-                for (int i = 0; i < MC; ++i) x[i] -= f * ye[i];
-                dirty = true;
-                if (s == 0) npairs++;
-            }
-        }
-    }
-    if (dirty) {
-#pragma unroll
-        for (int i = 0; i < MC; ++i) {
-            const int m = s + GS * i;
-            if (m < nens) Yp[j * nens + m] = x[i];
-        }
-        if (s == 0) Ym[j] = (T)mj;
-    }
-    if (counters && npairs) atomicAdd(&counters[0], npairs);
-}
-
-template <typename T, int MC>
-static int obs_solve_mc(T *Ym, T *Yp, const double *ob_value, const double *ob_error, const uint8_t *ob_assim,
-                        const double *geo, int64_t nobs, int nens, int loc_mode, double *rec,
-                        unsigned long long *counters, cudaStream_t st) {
-    for (int64_t b0 = 0; b0 < nobs; b0 += PB) {
-        obs_panel_kernel<T, MC><<<1, PB * GS, 0, st>>>(Ym, Yp, ob_value, ob_error, ob_assim, geo, nobs, nens, b0,
-                                                       loc_mode, rec, counters);
-        exb_count_launches(1);
-        const int64_t rest = nobs - (b0 + PB);
-        if (rest > 0) {
-            const unsigned grid = (unsigned)ceil_div64(rest, TR_THREADS / GS);
-            obs_trailing_kernel<T, MC><<<grid, TR_THREADS, 0, st>>>(Ym, Yp, geo, rec, nobs, nens, b0, loc_mode, counters);
-            exb_count_launches(1);
-        }
-    }
-    return exb_check_launch("obs_solve kernels");
-}
-
 template <typename T>
 static int obs_solve_impl(T *Ym, T *Yp, const double *ob_value, const double *ob_error, const uint8_t *ob_assim,
                           const double *geo, int64_t nobs, int nens, int loc_mode, double *rec,
@@ -318,37 +34,18 @@ static int obs_solve_impl(T *Ym, T *Yp, const double *ob_value, const double *ob
         return EXB_ERR_UNSUPPORTED;
     }
     cudaStream_t st = (cudaStream_t)stream;
-    {
-        // EXB_OBS_IMPL = dag | persistent | launches (default: auto)
-        //   dag         dependency-driven solve (obs_solve_dag.cu): the serial chain shrinks to the longest
-        //               dependency path; auto uses it whenever localisation is on and the graph is not dense
-        //   persistent  one cooperative kernel walking panels of 64 obs (obs_solve_persistent.cu); auto's choice
-        //               without localisation, where every ob depends on every earlier one
-        //   launches    kernel-per-panel path below, also the fallback when cooperative launch is unavailable
-        const char *impl = getenv("EXB_OBS_IMPL");
-        const bool want_dag = impl ? strcmp(impl, "dag") == 0 : loc_mode == EXB_LOC_GC;
-        if (want_dag) {
-            const int rc = exb_obs_solve_dag<T>(Ym, Yp, ob_value, ob_error, ob_assim, geo, nobs, nens, loc_mode, rec,
-                                                counters, st, impl != nullptr, plan);
-            if (rc != EXB_ERR_UNSUPPORTED) return rc;
-        }
-        if (!(impl && strcmp(impl, "launches") == 0)) {
-            const int rc = exb_obs_solve_persistent<T>(Ym, Yp, ob_value, ob_error, ob_assim, geo, nobs, nens, loc_mode,
-                                                       rec, counters, st);
-            if (rc != EXB_ERR_UNSUPPORTED) return rc;
-        }
+    const char *impl = getenv("EXB_OBS_IMPL");
+    const bool dag = impl && strcmp(impl, "dag") == 0;
+    if (impl && !dag && strcmp(impl, "persistent") != 0) {
+        exb_set_error("exb_obs_solve: EXB_OBS_IMPL=%s; the accepted values are dag and persistent", impl);
+        return EXB_ERR_ARG;
     }
-    const int mc = (nens + GS - 1) / GS;
-#define EXB_DISPATCH(M) \
-    if (mc <= M) return obs_solve_mc<T, M>(Ym, Yp, ob_value, ob_error, ob_assim, geo, nobs, nens, loc_mode, rec, counters, st)
-    EXB_DISPATCH(4);
-    EXB_DISPATCH(7);
-    EXB_DISPATCH(13);
-    EXB_DISPATCH(19);
-    EXB_DISPATCH(25);
-    EXB_DISPATCH(32);
-#undef EXB_DISPATCH
-    return EXB_ERR_UNSUPPORTED;
+    if (dag || (!impl && loc_mode == EXB_LOC_GC)) {
+        const int rc = exb_obs_solve_dag<T>(Ym, Yp, ob_value, ob_error, ob_assim, geo, nobs, nens, loc_mode, rec,
+                                            counters, st, dag, plan);
+        if (rc != EXB_ERR_UNSUPPORTED) return rc;
+    }
+    return exb_obs_solve_persistent<T>(Ym, Yp, ob_value, ob_error, ob_assim, geo, nobs, nens, loc_mode, rec, counters, st);
 }
 
 extern "C" int exb_obs_solve_f64(double *Ym, double *Yp, const double *ob_value, const double *ob_error,

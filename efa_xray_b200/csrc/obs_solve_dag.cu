@@ -210,10 +210,9 @@ struct DgArgs {
     int *ticket;
     int *status;                 // != 0: watchdog fired (value = 1 + index of the record that never arrived)
     unsigned long long watchdog_ns;
-    int local_gpu_scope;         // distributed variant: gpu-scope stores for the rank's own copy of a record (EXB_DAG_LOCAL_GPU)
-    int hot_poll;                // poll the record itself while waiting for the last predecessor of a batch (EXB_DAG_HOT)
     int64_t nobs, row_begin, row_end;
     int nens, loc_mode;
+    double inv_n;                // 1 / nens (IEEE division on the host, as on the device): a parameter holds no register
     // distributed variant (DIST): the rows dg_row(deal, t) are solved here; records are published into the P / S
     // buffers of every GPU of the group (peer memory over NVLink), readers always poll their own copy
     int world, rank;
@@ -406,7 +405,7 @@ __device__ __forceinline__ bool dg_step(const DgArgs<T> &a, int lane, DgRow<T, M
     constexpr int NW = DgCfg<T, MC>::NW;
     constexpr int PER = DgWord<T>::PER;
     if (!dg_ready<T, MC>(cur)) {
-        if (r.m == 0 && a.hot_poll) {
+        if (r.m == 0) {
             // The last entry of a batch of 32 predecessors is where a row sits while it is the next link of the
             // dependency chain: poll the record itself, without back-off, so that the hop does not pay a sleep interval
             // plus a second round trip to L2 after the wake-up.  (Few warps are in this state at a time.)
@@ -467,7 +466,6 @@ __global__ void __launch_bounds__(DG_WARPS * 32, DG_MINBLOCKS) dag_solve_kernel(
     const int lane = threadIdx.x & 31;
     const int64_t nobs = a.nobs;
     const int nens = a.nens;
-    const double inv_n = 1.0 / (double)nens;
     const bool gc = a.loc_mode == EXB_LOC_GC;
     unsigned long long npairs = 0;
 
@@ -552,7 +550,7 @@ __global__ void __launch_bounds__(DG_WARPS * 32, DG_MINBLOCKS) dag_solve_kernel(
                     const int dst = (a.rank + q) % a.world;
                     unsigned long long *p = reinterpret_cast<unsigned long long *>(static_cast<T *>(a.P_peer[dst]) + (j * 32 + lane) * MC);
                     if (lane * MC < nens) {
-                        if (q == 0 && a.local_gpu_scope) {
+                        if (q == 0) {
                             if constexpr (NW % 4 == 0) {
 #pragma unroll
                                 for (int c = 0; c < NW; c += 4) dg_st32(p + c, pw[c], pw[c + 1], pw[c + 2], pw[c + 3]);
@@ -576,8 +574,8 @@ __global__ void __launch_bounds__(DG_WARPS * 32, DG_MINBLOCKS) dag_solve_kernel(
         for (int q = 0; q < MC; ++q) { const double v = (double)r.x[q]; s0 += v; q0 += v * v; }
         const double rs = dg_warp_sum(s0), rq = dg_warp_sum(q0);
         const double mj = r.mj;
-        const double mean = rs * inv_n;
-        const double varye = fmax(rq * inv_n - mean * mean, 0.0);                    // np.var, ddof 0
+        const double mean = rs * a.inv_n;
+        const double varye = fmax(rq * a.inv_n - mean * mean, 0.0);                    // np.var, ddof 0
         const double innov = my_val - mj;
         const double kdenom = varye + my_err;
         const double c1 = 1.0 / ((double)(nens - 1) * kdenom);
@@ -589,7 +587,7 @@ __global__ void __launch_bounds__(DG_WARPS * 32, DG_MINBLOCKS) dag_solve_kernel(
             } else {
                 for (int q = 0; q < a.world; ++q) {
                     const int dst = (a.rank + q) % a.world;
-                    if (q == 0 && a.local_gpu_scope) dg_st16(static_cast<double *>(a.S_peer[dst]) + j * 2, s0w, s1w);
+                    if (q == 0) dg_st16(static_cast<double *>(a.S_peer[dst]) + j * 2, s0w, s1w);
                     else dg_st16_sys(static_cast<double *>(a.S_peer[dst]) + j * 2, s0w, s1w);
                 }
             }
@@ -628,11 +626,6 @@ __global__ void __launch_bounds__(DG_WARPS * 32, DG_MINBLOCKS) dag_solve_kernel(
 // ------------------------------------------------------------------------------------------
 // host side
 // ------------------------------------------------------------------------------------------
-static int dg_hot_poll() {
-    const char *e = getenv("EXB_DAG_HOT");
-    return e ? atoi(e) : 1;
-}
-
 static unsigned long long dg_watchdog_ns(int64_t nobs) {
     double sec = DG_WATCHDOG_S + 1e-4 * (double)nobs;
     if (const char *e = getenv("EXB_WATCHDOG_S")) { const double v = atof(e); if (v > 0.0) sec = v; }
@@ -857,13 +850,11 @@ int exb_obs_solve_dag(T *Ym, T *Yp, const double *ob_value, const double *ob_err
         EXB_CUDA(cudaMemsetAsync(sd, 0, sizeof(int), st));      // stream-ordered: an earlier solve's verdict is its own
         a.status = sd;
         a.watchdog_ns = dg_watchdog_ns(nobs);
-        a.hot_poll = dg_hot_poll();
-        a.local_gpu_scope = getenv("EXB_DAG_LOCAL_GPU") ? atoi(getenv("EXB_DAG_LOCAL_GPU")) : 1;
     }
     a.Ym = Ym; a.Yp = Yp; a.ob_value = ob_value; a.ob_error = ob_error; a.ob_assim = ob_assim; a.geo = geo; a.rec = rec;
     a.counters = counters; a.off = pl->off; a.list = nullptr; a.list_base = 0; a.P = nullptr; a.S = nullptr;
     a.ticket = nullptr; a.nobs = nobs; a.row_begin = 0; a.row_end = nobs; a.nens = nens;
-    a.loc_mode = loc_mode;
+    a.loc_mode = loc_mode; a.inv_n = 1.0 / (double)nens;
     a.world = 1; a.rank = 0; a.deal = DgDeal{1, 1, 0};
     for (int q = 0; q < 8; ++q) { a.P_peer[q] = nullptr; a.S_peer[q] = nullptr; }
     int rc = EXB_ERR_UNSUPPORTED;
@@ -908,13 +899,11 @@ static int dg_solve_dist(void *plan, T *Ym, T *Yp, const double *ob_value, const
         EXB_CUDA(cudaMemsetAsync(sd, 0, sizeof(int), st));      // stream-ordered: an earlier solve's verdict is its own
         a.status = sd;
         a.watchdog_ns = dg_watchdog_ns(nobs);
-        a.hot_poll = dg_hot_poll();
-        a.local_gpu_scope = getenv("EXB_DAG_LOCAL_GPU") ? atoi(getenv("EXB_DAG_LOCAL_GPU")) : 1;
     }
     a.Ym = Ym; a.Yp = Yp; a.ob_value = ob_value; a.ob_error = ob_error; a.ob_assim = ob_assim; a.geo = geo; a.rec = rec;
     a.counters = counters; a.off = pl->off; a.list = nullptr; a.list_base = 0; a.P = nullptr; a.S = nullptr;
     a.ticket = nullptr; a.nobs = nobs; a.row_begin = 0; a.row_end = nobs; a.nens = nens;
-    a.loc_mode = loc_mode;
+    a.loc_mode = loc_mode; a.inv_n = 1.0 / (double)nens;
     a.world = world; a.rank = rank; a.deal = pl->deal;
     for (int q = 0; q < 8; ++q) { a.P_peer[q] = q < world ? P_peers[q] : nullptr; a.S_peer[q] = q < world ? S_peers[q] : nullptr; }
     int rc = EXB_ERR_UNSUPPORTED;

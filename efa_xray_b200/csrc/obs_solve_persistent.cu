@@ -1,7 +1,17 @@
 // Obs-space serial solve as ONE persistent cooperative kernel.
 //
-// Same blocked right-looking algorithm as obs_solve.cu (panel of PS_PB obs strictly in order, then every
-// later row applies the panel), but without a kernel launch per step:
+// The Nobs obs-space rows of the reference's augmented state (assimilation.py:149-150) only ever read
+// other obs-space rows (ensrf.py:61-64, :95, :141), so they are evolved here on their own, in the
+// reference's serial order, and leave behind one record per ob (ye_k and a few scalars) from which
+// the state sweep (state_update.cu) can update every state row independently.
+//
+// Blocked right-looking form of the serial loop, panel width PS_PB: the obs k = b0..b0+PS_PB-1 of a panel are
+// processed strictly in order with the panel's rows in registers (the only truly serial part of the whole
+// analysis), then every later row j >= b0+PS_PB applies the panel's obs in order.  Rows j < k are never read
+// again by the reference (ensrf.py:61-64 reads row k at step k only), so they are not updated; row k is frozen
+// at step k and therefore ends up holding ye_k.
+//
+// One kernel runs the whole solve, without a launch per panel:
 //   CTA 0            the PANEL WORKER: walks the panels b = 0, 1, ... ; for each one it loads the 64 rows of
 //                    chunk b, applies the previous panel to them itself, runs the 64 serial steps with the rows
 //                    in registers, publishes the records, and sets panel_done = b+1 (release).
@@ -25,7 +35,6 @@
 #define PS_THREADS (PS_PB * PS_GS)
 #define PS_MAXBATCH 8
 #define PS_CTL_PAD 32
-#define PS_MAXCHUNKS 256       // chunks one trailing worker can own
 
 template <int N>
 __device__ __forceinline__ double ps_group_sum(double v, unsigned mask) {
@@ -306,12 +315,13 @@ __global__ void __launch_bounds__(PS_THREADS, 1) obs_solve_persistent_kernel(con
     } else {
         // =========================== TRAILING WORKER ===========================
         const int NW = gridDim.x - 1, w = blockIdx.x - 1;
-        __shared__ int s_upto[PS_MAXCHUNKS];             // progress of this worker's chunks (slot i -> chunk w + i*NW)
-        const int nmine = (a.npanels > w) ? (a.npanels - w + NW - 1) / NW : 0;
-        for (int i = tid; i < PS_MAXCHUNKS; i += PS_THREADS) s_upto[i] = 0;
+        if (w >= a.npanels) return;
+        extern __shared__ int s_upto[];                  // progress of this worker's chunks (slot i -> chunk w + i*NW)
+        const int nmine = (a.npanels - w + NW - 1) / NW;
+        for (int i = tid; i < nmine; i += PS_THREADS) s_upto[i] = 0;
         __syncthreads();
         int first = 0;                                   // (thread 0 only) slots below `first` are finished
-        while (nmine > 0 && nmine <= PS_MAXCHUNKS) {
+        while (true) {
             if (tid == 0) {
                 int slot = -1, tgt = 0;
                 while (true) {
@@ -360,25 +370,38 @@ __global__ void __launch_bounds__(PS_THREADS, 1) obs_solve_persistent_kernel(con
 
 template <typename T, int MC>
 static int ps_launch(PsArgs<T> &a, cudaStream_t st) {
+    const void *kernel = (const void *)obs_solve_persistent_kernel<T, MC>;
     int dev = 0, sms = 0, coop = 0, per_sm = 0;
     EXB_CUDA(cudaGetDevice(&dev));
     EXB_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
     EXB_CUDA(cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, dev));
-    if (!coop) return EXB_ERR_UNSUPPORTED;
-    EXB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, obs_solve_persistent_kernel<T, MC>, PS_THREADS, 0));
-    if (per_sm < 1) return EXB_ERR_UNSUPPORTED;
-    int grid = sms * per_sm;
-    if (grid > a.npanels + 1) grid = a.npanels + 1;
-    if (grid < 2) grid = 2;
-    if ((a.npanels + (grid - 2)) / (grid - 1) > PS_MAXCHUNKS) return EXB_ERR_UNSUPPORTED;    // too many chunks per worker
+    if (!coop) {
+        exb_set_error("obs_solve_persistent: device %d does not support cooperative launch", dev);
+        return EXB_ERR_UNSUPPORTED;
+    }
+    // A trailing worker keeps one progress word per chunk it owns in dynamic shared memory.  It is sized for one CTA
+    // per SM, the fewest workers the launch can have; more CTAs per SM only give each worker fewer chunks.
+    const auto clamp_grid = [&](int g) { return g > a.npanels + 1 ? a.npanels + 1 : (g < 2 ? 2 : g); };
+    int grid = clamp_grid(sms);
+    const size_t smem = sizeof(int) * (size_t)((a.npanels + grid - 2) / (grid - 1));
+    cudaFuncAttributes fa;
+    EXB_CUDA(cudaFuncGetAttributes(&fa, kernel));
+    if (fa.sharedSizeBytes + smem > 48 * 1024)
+        EXB_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    EXB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, PS_THREADS, smem));
+    if (per_sm < 1) {
+        exb_set_error("obs_solve_persistent: a CTA of %d threads with %zu bytes of shared memory does not fit an SM",
+                      PS_THREADS, fa.sharedSizeBytes + smem);
+        return EXB_ERR_UNSUPPORTED;
+    }
+    grid = clamp_grid(sms * per_sm);
     int *ctl = nullptr;
     const size_t ctl_bytes = sizeof(int) * (PS_CTL_PAD + (size_t)a.npanels + 1);
     EXB_CUDA(exb_malloc_async(&ctl, ctl_bytes, st));
     EXB_CUDA(cudaMemsetAsync(ctl, 0, ctl_bytes, st));
     a.ctl = ctl;
     void *params[] = {(void *)&a};
-    cudaError_t e = cudaLaunchCooperativeKernel((const void *)obs_solve_persistent_kernel<T, MC>, dim3(grid), dim3(PS_THREADS),
-                                                params, 0, st);
+    cudaError_t e = cudaLaunchCooperativeKernel(kernel, dim3(grid), dim3(PS_THREADS), params, smem, st);
     exb_count_launches(1);
     cudaFreeAsync(ctl, st);
     if (e != cudaSuccess) {

@@ -314,11 +314,8 @@ template <typename T>
 static int su_dispatch(SuParams &p, cudaStream_t st) {
     int bestS = 0, bestMC = 0;
     double best = 1e30;
-    int forceS = 0, forceMC = 0;
-    if (const char *e = getenv("EXB_SU_S")) forceS = atoi(e);
-    if (const char *e = getenv("EXB_SU_MC")) forceMC = atoi(e);
 #define SU_CONSIDER(S_, MC_)                                                              \
-    if (S_ * MC_ >= p.nens && (!forceS || forceS == S_) && (!forceMC || forceMC == MC_)) { \
+    if (S_ * MC_ >= p.nens) {                                                             \
         /* padded members, plus the cross-lane reduction and per-ob scalar work */        \
         const double cost = (double)S_ * MC_ + S_ * (4.0 + 1.5 * (S_ == 2 ? 1 : S_ == 4 ? 2 : 3)); \
         if (cost < best) { best = cost; bestS = S_; bestMC = MC_; }                       \

@@ -421,7 +421,7 @@ def sweep_plan_wanted():
 
 def obs_plan_wanted(loc_mode):
     import os
-    return loc_mode == LOC_GC and os.environ.get('EXB_OBS_IMPL', 'dag') == 'dag' and os.environ.get('EXB_OBS_PLAN', '1') != '0'
+    return loc_mode == LOC_GC and os.environ.get('EXB_OBS_IMPL', 'dag') == 'dag'
 
 
 def state_update(xm, Xp, nlev, ny, nx, grid_u, Yp, rec, geo, nobs, loc_mode, counters, sfx, ob_begin=0, ob_end=None):

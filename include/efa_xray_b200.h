@@ -157,8 +157,9 @@ int exb_recombine_f32(float *X, const float *xm, int64_t nrows, int nens, void *
  *        Ym[k]    = mye_k (ensrf.py:63);  rec = per-ob records (see top).
  * counters (device uint64[2], may be NULL): [0] += number of (ob k, obs row j >= k) pairs with
  * non-zero localisation weight = sum_k |F_o(k)| of SURVEY.md section 8d.
- * Three implementations with identical results up to summation order (environment EXB_OBS_IMPL = dag |
- * persistent | launches; default: dag with localisation, persistent without): see DESIGN.md section 4.2. */
+ * Two implementations with identical results up to summation order (environment EXB_OBS_IMPL = dag |
+ * persistent; default: dag with localisation unless its dependency graph is more than half dense, persistent
+ * otherwise; any other value is EXB_ERR_ARG): see DESIGN.md section 4.2. */
 int exb_obs_solve_f64(double *Ym, double *Yp, const double *ob_value, const double *ob_error,
                       const uint8_t *ob_assimilate, const double *obgeo, int64_t nobs, int nens,
                       int loc_mode, double *rec, unsigned long long *counters, void *stream);

@@ -302,28 +302,101 @@ def _run_obs_solve(obs, Ym, Yp, loc_mode, impl, dtype='f64', budget=None):
     return ym.cpu().numpy(), yp.cpu().numpy(), rec.cpu().numpy(), int(counters[0].item())
 
 
+def _oracle_obs_solve(obs, Ym, Yp, loc_mode):
+    """oracle.obs_space_solve (the reference's serial loop on the obs rows, ensrf.py:61-149) on device-side inputs."""
+    from oracle import ensrf_oracle as O
+    return O.obs_space_solve(Ym.cpu().numpy(), Yp.cpu().numpy(), obs.value, obs.error, obs.halfwidth, obs.lat, obs.lon,
+                             obs.assimilate.astype(bool), loc='GC' if loc_mode else None)
+
+
+def _check_obs_solve(got, want, assim):
+    """A device obs-space solve (ym, ye rows, records) against the oracle: ye rows, means and the seven record fields
+    at 1e-9 or tighter.  Innovation, c1 and beta only exist for assimilated obs in the oracle."""
+    ym, ye, rec = got[:3]
+    a = np.asarray(assim, dtype=bool)
+    assert np.abs(ye - want['ye']).max() <= 1e-9 * np.abs(want['ye']).max()
+    np.testing.assert_allclose(ym, want['prior_mean'], rtol=1e-10)
+    np.testing.assert_allclose(rec[0], want['prior_mean'], rtol=1e-10)
+    np.testing.assert_allclose(rec[1], want['prior_var'], rtol=1e-9)
+    np.testing.assert_allclose(rec[2], want['post_mean'], rtol=1e-10, equal_nan=True)
+    np.testing.assert_allclose(rec[3], want['post_var'], rtol=1e-9, equal_nan=True)
+    # innovations are differences of O(280 K) numbers: absolute tolerance from the means
+    np.testing.assert_allclose(rec[4][a], want['innov'][a], rtol=1e-9, atol=1e-10 * 300.0)
+    nens = ye.shape[1]
+    np.testing.assert_allclose(rec[5][a], 1.0 / ((nens - 1) * want['kdenom'][a]), rtol=1e-9)
+    np.testing.assert_allclose(rec[6][a], want['beta'][a], rtol=1e-9)
+    np.testing.assert_array_equal(rec[7], a.astype(np.float64))
+
+
 @pytest.mark.parametrize('kw,loc_mode', [
     (dict(ny=46, nx=90, nmem=50, nobs=700, cutoff_km=2500.0, seed=31, frac_skip=0.05, mixed_radius=True), 1),
     (dict(ny=46, nx=90, nmem=100, nobs=3000, cutoff_km=800.0, seed=32, mixed_error=True), 1),
     (dict(ny=37, nx=72, nmem=130, nobs=300, cutoff_km=3000.0, seed=33, frac_skip=0.1), 1),
     (dict(ny=37, nx=72, nmem=20, nobs=200, seed=34), 0),
 ])
-def test_obs_solve_variants_agree(kw, loc_mode):
-    """The dependency-driven obs-space solve, the persistent panel kernel and the kernel-per-panel path evolve
-    the same closed obs-row subsystem (SURVEY.md section 0) in the same serial order: records, ye rows,
-    diagnostics and pair counts must agree; the dependency-driven one also when its predecessor lists are
-    cut into many row blocks."""
+def test_obs_solve_variants_match_oracle(kw, loc_mode):
+    """The persistent panel kernel and the dependency-driven obs-space solve, the latter also with its predecessor
+    lists cut into many row blocks, evolve the closed obs-row subsystem (SURVEY.md section 0) in the reference's
+    serial order: records, ye rows and diagnostics match the oracle, and the runs agree with each other, pair counts
+    included."""
+    import itertools
     case = make_case(**kw)
     obs, Ym, Yp = _obs_block(case)
-    ref = _run_obs_solve(obs, Ym, Yp, loc_mode, 'launches')
+    want = _oracle_obs_solve(obs, Ym, Yp, loc_mode)
     runs = [_run_obs_solve(obs, Ym, Yp, loc_mode, 'persistent'), _run_obs_solve(obs, Ym, Yp, loc_mode, 'dag'),
             _run_obs_solve(obs, Ym, Yp, loc_mode, 'dag', budget=997)]
-    scale = np.abs(ref[1]).max()
-    for ym, yp, rec, npairs in runs:
+    for run in runs:
+        _check_obs_solve(run, want, obs.assimilate)
+    scale = np.abs(want['ye']).max()
+    for (ym, yp, rec, npairs), ref in itertools.combinations(runs, 2):
         assert npairs == ref[3]
         np.testing.assert_allclose(ym, ref[0], rtol=1e-11)
         assert np.abs(yp - ref[1]).max() <= 1e-11 * scale
         np.testing.assert_allclose(rec, ref[2], rtol=1e-9, atol=1e-12, equal_nan=True)
+
+
+def test_persistent_solve_beyond_256_chunks_per_worker():
+    """The persistent solve with more than 256 chunks of 64 obs per trailing worker (nobs = 64 x 260 x SMs; one CTA
+    per SM), 8 members, no localisation.  Only the first and the last 512 obs are assimilated.  (1) The pair counter
+    counts every later row of every assimilated ob, so every chunk saw every assimilated panel; (2) the assimilated
+    obs match the oracle run on them alone, since a skipped ob changes no row; (3) sampled skipped rows, some in chunks
+    past slot 256 of their worker, match the oracle on the first 512 obs followed by those rows."""
+    import torch
+    from oracle import ensrf_oracle as O
+    from efa_xray_b200 import engine
+    dev = torch.device('cuda', 0)
+    sms = torch.cuda.get_device_properties(dev).multi_processor_count
+    nobs, nens, na = 64 * 260 * sms, 8, 512
+    rng = np.random.default_rng(91)
+    Yp0 = rng.standard_normal((nobs, nens))
+    Yp0 -= Yp0.mean(axis=1, keepdims=True)
+    Ym0 = 280.0 + rng.standard_normal(nobs)
+    assim = np.zeros(nobs, dtype=np.uint8)
+    assim[:na] = assim[-na:] = 1
+    zeros = np.zeros(nobs, dtype=np.int64)
+    obs = engine.ObsArrays(value=Ym0 + rng.standard_normal(nobs), error=rng.uniform(0.5, 2.0, nobs),
+                           lat=rng.uniform(-80.0, 80.0, nobs), lon=rng.uniform(0.0, 360.0, nobs),
+                           halfwidth=np.full(nobs, 1000.0), assimilate=assim, row0=zeros, row1=zeros,
+                           tw0=np.ones(nobs), tw1=np.zeros(nobs))
+    ym, ye, rec, npairs = _run_obs_solve(obs, torch.as_tensor(Ym0, device=dev), torch.as_tensor(Yp0, device=dev), 0,
+                                         'persistent')
+    # (1)
+    ks = np.flatnonzero(assim)
+    assert npairs == int((nobs - ks).sum())
+
+    def oracle_on(idx):
+        return O.obs_space_solve(Ym0[idx], Yp0[idx], obs.value[idx], obs.error[idx], obs.halfwidth[idx], obs.lat[idx],
+                                 obs.lon[idx], assim[idx].astype(bool), loc=None)
+    # (2)
+    _check_obs_solve((ym[ks], ye[ks], rec[:, ks]), oracle_on(ks), assim[ks])
+    # (3) chunk p belongs to slot p // (SMs - 1) of its worker
+    tail = 64 * 256 * (sms - 1)
+    js = np.unique(np.concatenate([rng.integers(na, tail, 31), rng.integers(tail, nobs - na, 31), [na, nobs - na - 1]]))
+    want = oracle_on(np.concatenate([np.arange(na), js]))
+    scale = np.abs(want['ye'][na:]).max()
+    assert np.abs(ye[js] - want['ye'][na:]).max() <= 1e-9 * scale
+    np.testing.assert_allclose(rec[0][js], want['prior_mean'][na:], rtol=1e-10)
+    np.testing.assert_allclose(rec[1][js], want['prior_var'][na:], rtol=1e-9)
 
 
 def test_obs_solve_dag_fp32():
@@ -578,7 +651,6 @@ def test_dag_solve_matches_oracle_on_config3_prefix(nobs, cutoff_km):
     on the obs rows, ensrf.py:61-149) on the first `nobs` observations of BASELINE config 3: truncating the ob
     list is exact because ob k never depends on later obs.  Records, ye rows and diagnostics at 1e-9.  20 000 obs
     at 2000 km: dependency chain ~1e3; 5 000 obs at 5000 km: every ob sees ~15 % of the earlier ones."""
-    from oracle import ensrf_oracle as O
     c3 = _config3()
     case = c3['case']
     obs_all, Ym, Yp = c3['obs_block']
@@ -587,21 +659,10 @@ def test_dag_solve_matches_oracle_on_config3_prefix(nobs, cutoff_km):
     if cutoff_km != 2000.0:
         obs = dataclasses.replace(obs, halfwidth=np.full(nobs, 0.5 * cutoff_km))
     ym, yp = Ym[:nobs].contiguous(), Yp[:nobs].contiguous()
-    got_ym, got_ye, rec, npairs = _run_obs_solve(obs, ym, yp, 1, 'dag')
-    want = O.obs_space_solve(ym.cpu().numpy(), yp.cpu().numpy(), obs.value, obs.error, obs.halfwidth, obs.lat, obs.lon,
-                             obs.assimilate.astype(bool), loc='GC')
-    scale = np.abs(want['ye']).max()
-    assert np.abs(got_ye - want['ye']).max() <= 1e-9 * scale
-    np.testing.assert_allclose(rec[0], want['prior_mean'], rtol=1e-10)
-    np.testing.assert_allclose(rec[1], want['prior_var'], rtol=1e-9)
-    np.testing.assert_allclose(rec[2], want['post_mean'], rtol=1e-10, equal_nan=True)
-    np.testing.assert_allclose(rec[3], want['post_var'], rtol=1e-9, equal_nan=True)
-    # innovations are differences of O(280 K) numbers: absolute tolerance from the means
-    np.testing.assert_allclose(rec[4], want['innov'], rtol=1e-9, atol=1e-10 * 300.0)
-    nens = yp.shape[1]
-    np.testing.assert_allclose(rec[5], 1.0 / ((nens - 1) * want['kdenom']), rtol=1e-9)
-    np.testing.assert_allclose(rec[6], want['beta'], rtol=1e-9)
-    assert npairs > nobs
+    got = _run_obs_solve(obs, ym, yp, 1, 'dag')
+    assert obs.assimilate.all()
+    _check_obs_solve(got, _oracle_obs_solve(obs, ym, yp, 1), obs.assimilate)
+    assert got[3] > nobs
 
 
 def _sharded_analysis(case, nshards, Yfull=None):
