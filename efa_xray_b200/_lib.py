@@ -34,6 +34,12 @@ SIGNATURES = {
     'exb_inflate_f32': [_p, _i64, _int, _p, _i64, _i64, _p],
     'exb_recombine_f64': [_p, _p, _i64, _int, _p],
     'exb_recombine_f32': [_p, _p, _i64, _int, _p],
+    'exb_row_spread_f64': [_p, _i64, _i64, _i64, _i64, _int, _p, _p],
+    'exb_row_spread_f32': [_p, _i64, _i64, _i64, _i64, _int, _p, _p],
+    'exb_relax_rtps_f64': [_p, _p, _p, _i64, _i64, _i64, _i64, _int, _p],
+    'exb_relax_rtps_f32': [_p, _p, _p, _i64, _i64, _i64, _i64, _int, _p],
+    'exb_relax_rtpp_f64': [_p, _p, _p, _i64, _i64, _i64, _i64, _int, _p],
+    'exb_relax_rtpp_f32': [_p, _p, _p, _i64, _i64, _i64, _i64, _int, _p],
     'exb_obs_solve_f64': [_p, _p, _p, _p, _p, _p, _i64, _int, _int, _p, _p, _p],
     'exb_obs_solve_f32': [_p, _p, _p, _p, _p, _p, _i64, _int, _int, _p, _p, _p],
     'exb_obs_solve_async_status': [],

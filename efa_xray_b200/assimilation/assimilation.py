@@ -134,6 +134,49 @@ class Assimilation():
             return (fac[:, :, None, None] * field[None]).ravel()
         return fac.ravel()
 
+    @staticmethod
+    def _check_alpha(a, what):
+        if isinstance(a, bool) or not isinstance(a, (int, float, np.integer, np.floating)):
+            raise ValueError('relaxation alpha %s must be a float, got %r' % (what, a))
+        if not 0.0 <= float(a) <= 1.0:                            # NaN fails here too
+            raise ValueError('relaxation alpha %s must lie in [0, 1], got %r' % (what, a))
+
+    def _validate_relaxation(self, relaxation):
+        """None, ('rtps', a) or ('rtpp', a) with a a float in [0, 1] or a dict {variable name: float}; raises
+        ValueError otherwise.  Only reads the state's variable names (no device work)."""
+        if relaxation is None:
+            return
+        if not isinstance(relaxation, (tuple, list)) or len(relaxation) != 2:
+            raise ValueError("relaxation must be None, ('rtps', alpha) or ('rtpp', alpha), got %r" % (relaxation,))
+        kind, alpha = relaxation
+        if kind not in engine.RELAX_KINDS:
+            raise ValueError('relaxation kind must be one of %r, got %r' % (engine.RELAX_KINDS, kind))
+        if isinstance(alpha, dict):
+            varnames = self.prior.vars()
+            for k, v in alpha.items():
+                if k not in varnames:
+                    raise ValueError('relaxation names %r, which is not a state variable %r' % (k, varnames))
+                self._check_alpha(v, 'of %r' % (k,))
+        else:
+            self._check_alpha(alpha, '')
+
+    def _relaxation_levels(self, relaxation):
+        """(kind, alpha per level) for engine.analysis_*, or None: one alpha per (variable, time) level, in the
+        order of the state rows (as _inflation_factors orders inflation factors); variables a dict does not name get
+        0."""
+        if relaxation is None:
+            return None
+        kind, alpha = relaxation
+        st = self.prior
+        varnames = st.vars()
+        a = np.zeros((len(varnames), st.ntimes()))
+        if isinstance(alpha, dict):
+            for k, v in alpha.items():
+                a[varnames.index(k), :] = float(v)
+        else:
+            a[:] = float(alpha)
+        return kind, a.ravel()
+
     def _host_matrix(self):
         """[Nstate, Nens] host matrix of the prior in to_vect layout: the state's own block when it has one (no
         copy; callers only read it or hand it to the device), else a stacked copy."""
@@ -234,12 +277,13 @@ class Assimilation():
         return post_state, self.obs
 
 
-def update(prior_state, obs, inflate=None, loc=False, nproc=1, verbose=False):
+def update(prior_state, obs, inflate=None, loc=False, nproc=1, verbose=False, relaxation=None):
     """Module-level entry point (assimilation.py:176-222).  In the reference this calls an undefined
     enkf_update; here it runs the EnSRF.  nproc is accepted for signature compatibility: the GPU path does
-    not fork worker processes."""
+    not fork worker processes.  relaxation: posterior relaxation, as for EnSRF."""
     from .ensrf import EnSRF
-    return EnSRF(prior_state, obs, nproc=nproc, inflation=inflate, verbose=verbose, loc=loc).update()
+    return EnSRF(prior_state, obs, nproc=nproc, inflation=inflate, verbose=verbose, loc=loc,
+                 relaxation=relaxation).update()
 
 
 def randomize_obs_order(obs, seed=None):

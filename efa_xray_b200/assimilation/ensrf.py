@@ -10,19 +10,35 @@ from .. import engine
 
 
 class EnSRF(Assimilation):
-    """EnSRF(state, obs, nproc=1, inflation=None, verbose=True, loc=False).update() -> (post_state, obs).
+    """EnSRF(state, obs, nproc=1, inflation=None, verbose=True, loc=False, relaxation=None).update()
+    -> (post_state, obs).
 
     Same contract as the reference (ensrf.py:28-33, assimilation.py:171): `obs` is the caller's list,
     mutated in place with prior_mean / prior_var / post_mean / post_var / assimilated (ensrf.py:66-70,
     :144-149); `post_state` is a new EnsembleState; the prior is only modified by inflation.
     Observations are assimilated strictly in list order.  `dtype` ('f64' or 'f32') selects the device
     arithmetic; results are returned in the state's own dtype.
+
+    `relaxation` (not in the reference) relaxes the analysis back toward the prior after the serial loop, to
+    counter the loss of spread of repeated analyses:
+      None                 no relaxation (default)
+      ('rtps', alpha)      relaxation to prior spread (Whitaker & Hamill 2012):
+                           x = m_a + x'_a * (1 + alpha * (sigma_b - sigma_a) / sigma_a)
+      ('rtpp', alpha)      relaxation to prior perturbations (Zhang et al. 2004):
+                           x = m_a + (1 - alpha) * x'_a + alpha * x'_b
+    alpha is a float in [0, 1] or a dict {variable name: float}; variables the dict does not name get 0.  The prior
+    (m_b, x'_b, sigma_b) is the state as the serial loop receives it, i.e. after prior inflation.  The analysis mean
+    is unchanged, and rows without spread or that the analysis did not change are left as they are.  The per-ob
+    diagnostics (prior_mean, prior_var, post_mean, post_var) are those of the serial loop: they are not re-evaluated
+    after relaxation.  Invalid values raise ValueError here, before any device work.
     """
 
-    def __init__(self, state, obs, nproc=1, inflation=None, verbose=True, loc=False, dtype='f64'):
+    def __init__(self, state, obs, nproc=1, inflation=None, verbose=True, loc=False, dtype='f64', relaxation=None):
         Assimilation.__init__(self, state, obs, nproc, inflation, verbose)
         self.loc = loc
         self.dtype = dtype
+        self._validate_relaxation(relaxation)
+        self.relaxation = relaxation
         self.last_result = None
 
     def update(self):
@@ -58,7 +74,7 @@ class EnSRF(Assimilation):
             host = np.array(st.to_vect(), order='C', copy=True)
             out_blk, owner, out = None, None, host
         res = engine.analysis_host(host, nlev, None, None, obs, loc_mode, device=dev, dtype=tdtype,
-                                   grid=st._grid_tables(), out=out)
+                                   grid=st._grid_tables(), out=out, relaxation=self._relaxation_levels(self.relaxation))
         self._check_exact(res.n_exact)
         self.last_result = res
 

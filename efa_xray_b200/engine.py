@@ -6,7 +6,7 @@ torch.distributed only; every arithmetic step is a kernel of libefa_xray_b200.
 
 Sequence (reference: assimilation/ensrf.py:33-151, assimilation/assimilation.py:120-171):
     upload  ->  [inflate]  ->  ob priors H.x  ->  mean/perturbation split  ->  obs-space serial solve
-            ->  state sweep (per latitude band)  ->  recombine  ->  download
+            ->  state sweep (per latitude band)  ->  recombine  ->  [relax]  ->  download
 """
 from __future__ import annotations
 
@@ -454,6 +454,80 @@ def fused_sweep_available(dtype, nens):
     return os.environ.get('EXB_SU_IMPL', 'pipe') == 'pipe'
 
 
+RELAX_KINDS = ('rtps', 'rtpp')
+
+
+def relaxation_device(relaxation, nlev, device):
+    """(kind, alpha per level) -> (kind, the alphas as a float64 tensor on `device`), or None when there is nothing to
+    relax (relaxation None, or every alpha 0).  The alphas go up in one copy from page-locked memory, so the call does
+    not wait for the host: callers that stream the state in on another stream call this first (analysis_host), or the
+    copy would queue behind the state.  A pair whose alphas are already a device tensor is returned as it is."""
+    if relaxation is None:
+        return None
+    torch = _torch()
+    kind, alpha = relaxation
+    if kind not in RELAX_KINDS:
+        raise ValueError('relaxation kind must be one of %r, got %r' % (RELAX_KINDS, kind))
+    if isinstance(alpha, torch.Tensor) and alpha.device.type == 'cuda':
+        return relaxation
+    a = np.ascontiguousarray(alpha, dtype=np.float64).ravel()
+    if a.shape != (nlev,):
+        raise ValueError('relaxation needs one alpha per level (%d), got shape %r' % (nlev, a.shape))
+    if not ((a >= 0.0) & (a <= 1.0)).all():
+        raise ValueError('relaxation alphas must lie in [0, 1], got %r' % (a,))
+    if not a.any():
+        return None
+    return kind, torch.from_numpy(a).pin_memory().to(device, non_blocking=True)
+
+
+class _Relaxation:
+    """RTPS / RTPP of the state rows after the serial loop (DESIGN.md section 4.6), applied row range by row range:
+    before(pa, pb) records what the prior rows [pa, pb) of every level look like (sigma_b per row for RTPS, a copy of
+    the rows for RTPP) and must run before the sweep changes them; after(pa, pb) relaxes them once the analysis is
+    there.  Both run on the current stream.  ms() is the device time of the passes."""
+
+    def __init__(self, relaxation, X, nlev, timing):
+        torch = _torch()
+        self.kind, self.alpha = relaxation
+        self.X, self.nlev = X, nlev
+        self.npts = X.shape[0] // nlev
+        self.nens = X.shape[1]
+        self.sfx = _sfx(X.dtype)
+        if self.kind == 'rtps':
+            self.sigma_b = torch.empty(X.shape[0], dtype=torch.float64, device=X.device)
+        else:
+            self.Xb = torch.empty_like(X)
+        self.events = [] if timing else None
+
+    def _timed(self, fn):
+        if self.events is None:
+            return fn()
+        torch = _torch()
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record()
+        fn()
+        e1.record()
+        self.events.append((e0, e1))
+
+    def before(self, pa, pb):
+        def run():
+            if self.kind == 'rtps':
+                _lib.call('exb_row_spread_' + self.sfx, _lib.ptr(self.X), self.nlev, self.npts, pa, pb, self.nens,
+                          _lib.ptr(self.sigma_b), _lib.stream_ptr())
+            else:
+                shape = (self.nlev, self.npts, self.nens)
+                self.Xb.view(shape)[:, pa:pb].copy_(self.X.view(shape)[:, pa:pb])
+        self._timed(run)
+
+    def after(self, pa, pb):
+        prior = self.sigma_b if self.kind == 'rtps' else self.Xb
+        self._timed(lambda: _lib.call('exb_relax_%s_%s' % (self.kind, self.sfx), _lib.ptr(self.X), _lib.ptr(prior),
+                                      _lib.ptr(self.alpha), self.nlev, self.npts, pa, pb, self.nens, _lib.stream_ptr()))
+
+    def ms(self):
+        return sum(e0.elapsed_time(e1) for e0, e1 in self.events)
+
+
 _OBS_FIELDS = ('value', 'error', 'lat', 'lon', 'halfwidth', 'tw0', 'tw1', 'row0', 'row1')
 _STAGING = {}
 
@@ -507,7 +581,7 @@ def upload_obs(obs: ObsArrays, device, loc_mode):
 
 def analysis_device(X, nlev, grid: GridTables, obs: ObsArrays, loc_mode, inflation=None, timing=True,
                     band=None, group=None, Y=None, sweep_bands=None, on_band_done=None, before_band=None,
-                    obs_device=None):
+                    obs_device=None, relaxation=None):
     """Serial EnSRF analysis of a device-resident ensemble, in place.
 
     X        torch tensor [nlev*ny*nx, nens] (float64 or float32) on a CUDA device, to_vect layout
@@ -515,6 +589,10 @@ def analysis_device(X, nlev, grid: GridTables, obs: ObsArrays, loc_mode, inflati
              only that latitude band, [nlev*(y1-y0)*nx, nens], of a state sharded over the ranks of `group`;
              `grid` always describes the full grid.
     inflation  None, or a numpy array of per-level multiplicative factors (length nlev).
+    relaxation  None, or (kind, alpha per level): posterior relaxation of the state rows after the serial loop,
+             kind 'rtps' (relaxation to prior spread) or 'rtpp' (relaxation to prior perturbations), relative to the
+             prior as the sweep receives it (after inflation); DESIGN.md section 4.6.  Every alpha 0 launches nothing.
+             The per-ob diagnostics stay those of the serial loop.  res.ms gains 'relax' when it ran.
     sweep_bands  optional list of (ya, yb) row ranges of the shard: the fused sweep is issued range by range and
              on_band_done(ya, yb) is called after each launch has been enqueued (e.g. to start its download),
              before_band(ya, yb) before it (e.g. to wait for its upload).
@@ -550,6 +628,8 @@ def analysis_device(X, nlev, grid: GridTables, obs: ObsArrays, loc_mode, inflati
         # (small host-to-device copies: callers that stream the state in on another stream do them first and pass
         # the result, or they would queue behind the state in the copy engine)
         obs_dev, geo = obs_device if obs_device is not None else upload_obs(obs, dev, loc_mode)
+        relaxation = relaxation_device(relaxation, nlev, dev)
+        relax = _Relaxation(relaxation, X, nlev, timing) if relaxation is not None else None
         tm.mark('setup_upload')
         try:
             # predecessor lists of the obs-space solve: geometry only, started on a side stream now so that they are
@@ -581,6 +661,8 @@ def analysis_device(X, nlev, grid: GridTables, obs: ObsArrays, loc_mode, inflati
                 # (the device computes them meanwhile)
                 splan = SweepPlan(grid_u, nlev, ny, nx, obs_dev, geo, obs.nobs, loc_mode)
             if not fused:
+                if relax is not None:
+                    relax.before(0, ny * nx)
                 xm = torch.empty(nrows, dtype=X.dtype, device=dev)
                 _lib.call('exb_split_mean_pert_' + sfx, _lib.ptr(X), _lib.ptr(xm), nrows, nens, _lib.stream_ptr())
             tm.mark('setup_plans')
@@ -603,7 +685,11 @@ def analysis_device(X, nlev, grid: GridTables, obs: ObsArrays, loc_mode, inflati
                 for ya, yb in (sweep_bands or [(0, ny)]):
                     if before_band is not None:
                         before_band(ya, yb)
+                    if relax is not None:
+                        relax.before(ya * nx, yb * nx)
                     state_sweep_fused(X, nlev, ny, nx, grid_u, Yp, rec, geo, obs.nobs, loc_mode, counters, ya, yb, plan=splan)
+                    if relax is not None:
+                        relax.after(ya * nx, yb * nx)
                     if on_band_done is not None:
                         on_band_done(ya, yb)
                 tm.mark('state_update')
@@ -611,6 +697,8 @@ def analysis_device(X, nlev, grid: GridTables, obs: ObsArrays, loc_mode, inflati
                 state_update(xm, X, nlev, ny, nx, grid_u, Yp, rec, geo, obs.nobs, loc_mode, counters, sfx)
                 tm.mark('state_update')
                 _lib.call('exb_recombine_' + sfx, _lib.ptr(X), _lib.ptr(xm), nrows, nens, _lib.stream_ptr())
+                if relax is not None:
+                    relax.after(0, ny * nx)
             tm.mark('recombine')
             rec_h = rec.cpu().numpy()
             _lib.call('exb_obs_solve_async_status')
@@ -621,9 +709,12 @@ def analysis_device(X, nlev, grid: GridTables, obs: ObsArrays, loc_mode, inflati
                 plan.destroy()
             if splan is not None:
                 splan.destroy()
+    ms = tm.result()
+    if relax is not None and timing:
+        ms['relax'] = relax.ms()
     return AnalysisResult(prior_mean=rec_h[0], prior_var=rec_h[1], post_mean=rec_h[2], post_var=rec_h[3],
                           assimilated=rec_h[7] != 0.0, n_exact=nex_h, state_pairs=int(cnt[1]) * nlev,
-                          obs_pairs=int(cnt[0]), ms=tm.result(), obs_solve=which)
+                          obs_pairs=int(cnt[0]), ms=ms, obs_solve=which)
 
 
 def sweep_band_schedule(nlev, ny, nx, nbands=None):
@@ -647,7 +738,7 @@ def sweep_band_schedule(nlev, ny, nx, nbands=None):
 
 
 def analysis_host(X_host, nlev, lat2d, lon2d, obs: ObsArrays, loc_mode, inflation=None, device='cuda:0',
-                  dtype=None, grid=None, out=None, pipeline=True, band=None, group=None):
+                  dtype=None, grid=None, out=None, pipeline=True, band=None, group=None, relaxation=None):
     """Host-buffer entry: X_host is a numpy array or CPU torch tensor [nlev*ny*nx, nens]; it is uploaded,
     analysed on `device`, and the analysis is written to `out` (default: back into X_host).  Pinned host
     memory makes the copies asynchronous.  With the fused float64 sweep (and pipeline=True) the state is swept
@@ -659,7 +750,10 @@ def analysis_host(X_host, nlev, lat2d, lon2d, obs: ObsArrays, loc_mode, inflatio
     With band=(y0, y1) X_host / out hold only that latitude band of a host-resident state sharded over the ranks of
     `group` (one process per GPU): every rank moves its own band over its own PCIe link, the partial ob priors are
     all-reduced (NCCL), the obs-space solve is distributed over the ranks through NVLink peer memory (or replicated, see
-    res.obs_solve) and no other data crosses between ranks."""
+    res.obs_solve) and no other data crosses between ranks.
+
+    relaxation: as for analysis_device; with the band pipeline each band is relaxed between its sweep and its
+    download."""
     torch = _torch()
     _lib.require_device()
     Xh = X_host if isinstance(X_host, torch.Tensor) else torch.from_numpy(X_host)
@@ -688,6 +782,7 @@ def analysis_host(X_host, nlev, lat2d, lon2d, obs: ObsArrays, loc_mode, inflatio
             bands = sweep_band_schedule(nlev, ny_loc, grid.nx)
             ev[0].record()
             obs_device = upload_obs(obs, torch.device(device), loc_mode)
+            relaxation = relaxation_device(relaxation, nlev, torch.device(device))
             Y = None
             if inflation is None and Xh.is_pinned():
                 # PCIe is used by one thing at a time: first the gather (25 % of the state in 800-byte pieces),
@@ -719,7 +814,8 @@ def analysis_host(X_host, nlev, lat2d, lon2d, obs: ObsArrays, loc_mode, inflatio
                         O3[lev, ya * grid.nx:yb * grid.nx].copy_(X3[lev, ya * grid.nx:yb * grid.nx], non_blocking=True)
 
             res = analysis_device(X, nlev, grid, obs, loc_mode, inflation, Y=Y, sweep_bands=bands, band=band, group=group,
-                                  before_band=wait_upload, on_band_done=download, obs_device=obs_device)
+                                  before_band=wait_upload, on_band_done=download, obs_device=obs_device,
+                                  relaxation=relaxation)
             ev[2].record()
             main.wait_stream(copy_out)
             ev[3].record()
@@ -731,7 +827,7 @@ def analysis_host(X_host, nlev, lat2d, lon2d, obs: ObsArrays, loc_mode, inflatio
             if dtype is not None and X.dtype != dtype:
                 X = X.to(dtype)
             ev[1].record()
-            res = analysis_device(X, nlev, grid, obs, loc_mode, inflation, band=band, group=group)
+            res = analysis_device(X, nlev, grid, obs, loc_mode, inflation, band=band, group=group, relaxation=relaxation)
             ev[2].record()
             Oh.copy_(X.to(Oh.dtype) if X.dtype != Oh.dtype else X, non_blocking=True)
             ev[3].record()

@@ -149,6 +149,28 @@ int exb_inflate_f32(float *X, int64_t nrows, int nens, const double *factor_host
 int exb_recombine_f64(double *X, const double *xm, int64_t nrows, int nens, void *stream);
 int exb_recombine_f32(float *X, const float *xm, int64_t nrows, int nens, void *stream);
 
+/* ---- posterior relaxation of the state rows after the serial loop (DESIGN.md section 4.6) -------------
+ * The rows are those of levels lev < nlev, points [p_begin, p_end) of a shard X[nlev*npts][nens]: rows
+ * lev*npts + p, so one call covers a latitude band of every level.  nens >= 2 (EXB_ERR_ARG otherwise).
+ * Arithmetic is float64; float storage is rounded once on write.  alpha_dev is a DEVICE array of nlev values. */
+/* sigma_out[lev*npts + p] = ensemble standard deviation (ddof = 1) of that row; other entries are untouched. */
+int exb_row_spread_f64(const double *X, int64_t nlev, int64_t npts, int64_t p_begin, int64_t p_end, int nens,
+                       double *sigma_out, void *stream);
+int exb_row_spread_f32(const float *X, int64_t nlev, int64_t npts, int64_t p_begin, int64_t p_end, int nens,
+                       double *sigma_out, void *stream);
+/* RTPS, relaxation to prior spread: x = m_a + x'_a (1 + alpha (sigma_b - sigma_a) / sigma_a), with sigma_b from
+ * exb_row_spread_* on the prior.  A row is not written when alpha = 0, sigma_a = 0, or sigma_a == sigma_b. */
+int exb_relax_rtps_f64(double *X, const double *sigma_b, const double *alpha_dev, int64_t nlev, int64_t npts,
+                       int64_t p_begin, int64_t p_end, int nens, void *stream);
+int exb_relax_rtps_f32(float *X, const double *sigma_b, const double *alpha_dev, int64_t nlev, int64_t npts,
+                       int64_t p_begin, int64_t p_end, int nens, void *stream);
+/* RTPP, relaxation to prior perturbations: x = m_a + (1 - alpha) x'_a + alpha x'_b, with Xb the prior laid out as X.
+ * A row is not written when alpha = 0, sigma_a = 0, or every member equals the prior's. */
+int exb_relax_rtpp_f64(double *X, const double *Xb, const double *alpha_dev, int64_t nlev, int64_t npts,
+                       int64_t p_begin, int64_t p_end, int nens, void *stream);
+int exb_relax_rtpp_f32(float *X, const float *Xb, const double *alpha_dev, int64_t nlev, int64_t npts,
+                       int64_t p_begin, int64_t p_end, int nens, void *stream);
+
 /* ---- the serial loop, split in two (SURVEY.md section 0: the obs rows are a closed subsystem) --- */
 /* Obs-space serial solve: the rows Nstate..Nstate+Nobs-1 of the reference's augmented state evolved
  * through the whole loop ensrf.py:50-149 in the given (serial) order.
