@@ -135,8 +135,32 @@ template <int NT3> __host__ __device__ constexpr int s2_yst() { return ((8 * NT3
 // doubles of the ye-row region of a stage: 8 rows at q*YST + (q>>1)*4
 template <int NT3> __host__ __device__ constexpr int s2_ydoubles() { return 8 * s2_yst<NT3>() + 16; }
 
-// Stage layout (doubles): y rows [s2_ydoubles] | block = om[8][G] (ob-major) | Gram[64]
-template <int NT3, typename TS>
+// Columns of a row of Yw and of the state rows in registers.  Lane c of a row holds columns 2c and 2c+1 of every
+// 8-column tile t, as x[2t] and x[2t+1], and k-step h of tile t in step 1 covers the columns 2c+h of the four lanes.
+// s2_slot gives the member slot that column 2c+h of tile t holds: slot m < nens is member m, slot 8*NT3-1 the
+// pseudo-member (the mean), any other slot a zero pad.  LK is the number of k-steps of the last tile that carry members
+// (nens - 8*(NT3-1) members there: none -> 0, 1..4 -> 1, 5..7 -> 2).  With LK == 1 the last tile is stored
+// transposed, slot 4h+c in column 2c+h: its members sit in the even columns, the odd ones hold the pads and the mean,
+// and step 1 and the Gram matrix skip that k-step.  Every tile before the last is in member order.
+template <int NT3, int LK> __host__ __device__ constexpr int s2_slot(int t, int c, int h) {
+    return (LK == 1 && t == NT3 - 1) ? 8 * t + 4 * h + c : 8 * t + 2 * c + h;
+}
+template <int NT3> static int s2_last_ksteps(int nens) {
+    const int r = nens - 8 * (NT3 - 1);
+    return r <= 0 ? 0 : r <= 4 ? 1 : 2;
+}
+
+// Tail of a batch block (after om[G][8]), in doubles: what phase B reads besides the weights, packed for vector loads.
+//   [S2_TCORR + 4n + c]  B operand of the correction DMMA of lane (n, c): G[n][c] for n >= 4, zero for n < 4 (so the
+//                        first 8 doubles are zeros: inactive rows read them as their weights)
+//   [S2_TREC ..+12]      the recurrence's coefficients G10 G20 G21 G30 G31 G32 G54 G64 G65 G74 G75 G76
+//   [S2_TMASK]           low 32 bits: bit w set when warp w has a row with a non-zero weight for an ob of the batch
+#define S2_TCORR 0
+#define S2_TREC 32
+#define S2_TMASK 44
+
+// Stage layout (doubles): y rows [s2_ydoubles] | block = om[G][8] (point-major) | tail[64]
+template <int NT3, int LK, typename TS>
 __global__ void __launch_bounds__(S2_NW * 32, 1) state_sweep_2p_kernel(const S2Params p) {
     constexpr int NW = S2_NW;
     constexpr int NTH = NW * 32;             // threads per CTA
@@ -157,8 +181,8 @@ __global__ void __launch_bounds__(S2_NW * 32, 1) state_sweep_2p_kernel(const S2P
     unsigned long long *s_full = reinterpret_cast<unsigned long long *>(s_xch + NW * 32); // [S2_MAXSTAGES]
     unsigned long long *s_empty = s_full + S2_MAXSTAGES;                                      // [S2_MAXSTAGES]
     int *s_cand = reinterpret_cast<int *>(s_empty + S2_MAXSTAGES);                            // [S2_CAND]
-    int *s_gvalid = s_cand + S2_CAND;                                                         // [ROWS]
-    int *s_wcnt = s_gvalid + ROWS;                                                         // [NW]
+    int *s_gwarps = s_cand + S2_CAND;                                                         // [ROWS]
+    int *s_wcnt = s_gwarps + ROWS;                                                         // [NW]
     int *s_misc = s_wcnt + NW;                                                             // [4]
     float *s_bound = reinterpret_cast<float *>(s_misc + 4);                                   // [4]
 
@@ -186,10 +210,16 @@ __global__ void __launch_bounds__(S2_NW * 32, 1) state_sweep_2p_kernel(const S2P
     unsigned gbatch = 0;                         // batches that have gone through the ring so far (same in every thread)
     unsigned long long npairs = 0;
 
-    // phase clocks of thread 0 (only with p.prof): 0 patch setup, 1 scan, 2 blocks, 3 rows in/out, 4 phase B, 5 barriers
-    long long pt0 = 0, pacc[10] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
+    // phase clocks of thread 0 (only with p.prof): 0 patch setup, 1 scan, 2 blocks, 3 rows in/out, 4 phase B, 5 barriers;
+    // prof[10]: batches
+    // (the sums live in shared memory: as a register array they would take registers or stack from the loops)
+    __shared__ long long pacc[10];
+    long long pt0 = 0;
 #define S2_TICK(slot) do { if (p.prof && tid == 0) { const long long t_ = clock64(); pacc[slot] += t_ - pt0; pt0 = t_; } } while (0)
-    if (p.prof && tid == 0) pt0 = clock64();
+    if (p.prof && tid == 0) {
+        for (int i = 0; i < 10; ++i) pacc[i] = 0;
+        pt0 = clock64();
+    }
     for (;;) {
         // ---- next patch -----------------------------------------------------------------------------------
         __syncthreads();                          // everybody is done with the previous patch's shared state
@@ -223,7 +253,10 @@ __global__ void __launch_bounds__(S2_NW * 32, 1) state_sweep_2p_kernel(const S2P
             s_gu[tid] = p.grid_u[pt];
             s_gu[ROWS + tid] = p.grid_u[p.npts + pt];
             s_gu[2 * ROWS + tid] = p.grid_u[2 * p.npts + pt];
-            s_gvalid[tid] = ok;
+            // the warps that hold the point's rows of this level chunk (row slots tid*Lc + l, l < the chunk's levels);
+            // zero for a point outside the launch's rows or the grid
+            const int r0 = tid * Lc, r1 = r0 + min(Lc, p.nlev - l0) - 1;
+            s_gwarps[tid] = ok ? (int)(((2u << (r1 >> 3)) - 1u) & ~((1u << (r0 >> 3)) - 1u)) : 0;
         }
         __syncthreads();
         if (warp == 0) {
@@ -275,7 +308,7 @@ __global__ void __launch_bounds__(S2_NW * 32, 1) state_sweep_2p_kernel(const S2P
                 row = (int64_t)(l0 + l) * p.npts + (int64_t)gy * p.nx + gx;
             }
         }
-        const int gslot = active ? g : 0;
+        const int gslot = active ? g : G;          // om[G] of a block is the zeros at the start of its tail
         double x[2 * NT3];
         bool loaded = false, dirty = false;
 
@@ -335,7 +368,8 @@ __global__ void __launch_bounds__(S2_NW * 32, 1) state_sweep_2p_kernel(const S2P
             }
 
             // =============================== PHASE A (2): one block per batch ===============================
-            // Block of batch b (doubles): om[8][G] (ob-major: omega of ob q at grid point g) | Gram[64].
+            // Block of batch b (doubles): om[G][8] (point-major: omega of ob q at grid point g in g*8 + q) | tail[64]
+            // (see S2_TCORR).
             {
                 double *sob = s_sob + warp * 48;
                 // scalars of the obs of a batch, held by lanes 0..7; loaded one batch ahead
@@ -394,13 +428,23 @@ __global__ void __launch_bounds__(S2_NW * 32, 1) state_sweep_2p_kernel(const S2P
                         npb += (w != 0.0) ? 1 : 0;
                         return w * o45.y;
                     };
+                    // wm: the warps whose rows got a non-zero weight (bits of s_gwarps), for phase B to skip the others
+                    unsigned wm = 0u;
                     const int nfull = G >> 5, R = G & 31;
                     for (int sl = 0; sl < nfull; ++sl) {
                         const int gg = lane + 32 * sl;
                         const double gx = s_gu[gg], gy = s_gu[ROWS + gg], gz = s_gu[2 * ROWS + gg];
-                        const bool gval = s_gvalid[gg] != 0;
-#pragma unroll 2
-                        for (int q = 0; q < 8; ++q) gblk[q * G + gg] = weigh(gx, gy, gz, q, gval && q < nq);
+                        const int gw = s_gwarps[gg];
+                        const bool gval = gw != 0;
+                        bool hit = false;
+#pragma unroll 1
+                        for (int q = 0; q < 8; q += 2) {
+                            const double w0 = weigh(gx, gy, gz, q, gval && q < nq);
+                            const double w1 = weigh(gx, gy, gz, q + 1, gval && q + 1 < nq);
+                            hit |= (w0 != 0.0) | (w1 != 0.0);
+                            *reinterpret_cast<double2 *>(gblk + 8 * gg + q) = make_double2(w0, w1);
+                        }
+                        wm |= hit ? (unsigned)gw : 0u;
                     }
                     if (R) {
                         // pairs i = q * R + r of the last R points: q = i / R by a multiplication (exact for i < 2^20 / R)
@@ -410,15 +454,17 @@ __global__ void __launch_bounds__(S2_NW * 32, 1) state_sweep_2p_kernel(const S2P
                             const int i = lane + 32 * it, ic = min(i, npr - 1);
                             const int q = (int)(((unsigned)ic * rdiv) >> 20);
                             const int gg = g0 + ic - q * R;
+                            const int gw = s_gwarps[gg];
                             const double w = weigh(s_gu[gg], s_gu[ROWS + gg], s_gu[2 * ROWS + gg], q,
-                                                   i < npr && q < nq && s_gvalid[gg] != 0);
-                            if (i < npr) gblk[q * G + gg] = w;
+                                                   i < npr && q < nq && gw != 0);
+                            wm |= (w != 0.0) ? (unsigned)gw : 0u;
+                            if (i < npr) gblk[8 * gg + q] = w;
                         }
                     }
                     if (lc == 0) npairs += (unsigned long long)npb;
                     S2_TICK(7);
-                    // Gram matrix of the batch (members only: the pseudo-member column is masked): row n of the batch,
-                    // this lane's two members of every 8-member tile, operands straight from Yw (L2)
+                    // Gram matrix of the batch (members only: the pseudo-member column is masked or skipped): row n of the
+                    // batch, this lane's two columns of every 8-column tile, operands straight from Yw (L2)
                     {
                         double g0 = 0.0, g1 = 0.0, h0 = 0.0, h1 = 0.0;
                         const int krow = __shfl_sync(0xffffffffu, cur.kk, n);
@@ -426,11 +472,24 @@ __global__ void __launch_bounds__(S2_NW * 32, 1) state_sweep_2p_kernel(const S2P
 #pragma unroll
                         for (int t = 0; t < NT3; ++t) {
                             const double2 v = __ldg(reinterpret_cast<const double2 *>(yrow + 8 * t));
-                            const double v1 = (t == NT3 - 1 && c == 3) ? 0.0 : v.y;
-                            s2_dmma(g0, g1, v.x, v.x);
-                            s2_dmma(h0, h1, v1, v1);
+                            if (t < NT3 - 1 || LK >= 1) s2_dmma(g0, g1, v.x, v.x);
+                            if (t < NT3 - 1 || LK == 2) {
+                                const double v1 = (t == NT3 - 1 && c == 3) ? 0.0 : v.y;
+                                s2_dmma(h0, h1, v1, v1);
+                            }
                         }
-                        *reinterpret_cast<double2 *>(gblk + 8 * G + n * 8 + 2 * c) = make_double2(g0 + h0, g1 + h1);
+                        // lane (n, c) holds G[n][2c], G[n][2c+1]: scatter them into the tail's layout
+                        const double gx = g0 + h0, gy = g1 + h1;
+                        double *gt = gblk + 8 * G;
+                        if (c < 2)
+                            *reinterpret_cast<double2 *>(gt + S2_TCORR + 4 * n + 2 * c) =
+                                n >= 4 ? make_double2(gx, gy) : make_double2(0.0, 0.0);
+                        const int lo = n & 4;                                   // G[n][j], lo <= j < n: recurrence
+                        double *gr = gt + S2_TREC + 6 * (n >> 2) + (n - lo) * (n - lo - 1) / 2 - lo;
+                        if (2 * c >= lo && 2 * c < n) gr[2 * c] = gx;
+                        if (2 * c + 1 >= lo && 2 * c + 1 < n) gr[2 * c + 1] = gy;
+                        wm = __reduce_or_sync(0xffffffffu, wm);
+                        if (lane == 0) *reinterpret_cast<unsigned *>(gt + S2_TMASK) = wm;
                     }
                     cur = nxt;
                     S2_TICK(8);
@@ -454,7 +513,7 @@ __global__ void __launch_bounds__(S2_NW * 32, 1) state_sweep_2p_kernel(const S2P
                     for (int t = 0; t < NT3; ++t) {
 #pragma unroll
                         for (int h = 0; h < 2; ++h) {
-                            const int m = 8 * t + 2 * c + h;
+                            const int m = s2_slot<NT3, LK>(t, c, h);
                             double v = 0.0;
                             if (active && m < nens) { v = (double)gXp[row * nens + m]; sum += v; }
                             x[2 * t + h] = v;
@@ -469,7 +528,7 @@ __global__ void __launch_bounds__(S2_NW * 32, 1) state_sweep_2p_kernel(const S2P
                         for (int t = 0; t < NT3; ++t) {
 #pragma unroll
                             for (int h = 0; h < 2; ++h) {
-                                const int m = 8 * t + 2 * c + h;
+                                const int m = s2_slot<NT3, LK>(t, c, h);
                                 if (m < nens) x[2 * t + h] -= mean;
                             }
                         }
@@ -517,32 +576,27 @@ __global__ void __launch_bounds__(S2_NW * 32, 1) state_sweep_2p_kernel(const S2P
                     s2_mbar_wait_full(s_full + rs, rpar);
                     const double *sy = s_ring + (size_t)rs * SD;
                     const double *som = sy + YD;
-                    const double *Gb = som + 8 * G;
+                    const double *Gt = som + 8 * G;
 
-                    // omega of this row's grid point for the 8 obs of the batch (ob-major block: om[q][G])
-                    double om[8];
-#pragma unroll
-                    for (int i = 0; i < 8; ++i) {
-                        const double v = som[i * G + gslot];
-                        om[i] = active ? v : 0.0;
-                    }
-                    // any weight non-zero?  (integer test of the bit patterns: the FP64 pipe is the contended one)
-                    long long anyb = 0;
-#pragma unroll
-                    for (int i = 0; i < 8; ++i) anyb |= __double_as_longlong(om[i]);
-                    const bool any = (anyb << 1) != 0;
-                    if (__any_sync(0xffffffffu, any)) {
+                    // does any row of this warp have a non-zero weight for an ob of the batch?  (phase A's warp mask)
+                    if ((*reinterpret_cast<const unsigned *>(Gt + S2_TMASK) >> warp) & 1u) {
+                        // omega of this row's grid point for the 8 obs of the batch (point-major block: om[G][8])
+                        const double2 *omp = reinterpret_cast<const double2 *>(som + 8 * gslot);
+                        const double2 om01 = omp[0], om23 = omp[1], om45 = omp[2], om67 = omp[3];
                         // step 1: g[row][ob] = x[row] . y_ob   (one accumulator chain: four warps per sub-partition keep
-                        // the pipe fed, and the two halves need not be added afterwards)
+                        // the pipe fed, and the two halves need not be added afterwards); k-steps of the last tile
+                        // without members are skipped (s2_slot)
                         double ga0 = 0.0, ga1 = 0.0;
                         {
-                            const double *yrow = sy + n * YST + (n >> 1) * 4 + 2 * c;     // B operand: ob = n, members of lane c
+                            const double *yrow = sy + n * YST + (n >> 1) * 4 + 2 * c;     // B operand: ob = n, columns of lane c
 #pragma unroll
                             for (int t = 0; t < NT3; ++t) {
                                 const double2 v = *reinterpret_cast<const double2 *>(yrow + 8 * t);
-                                const double a1 = (t == NT3 - 1 && c == 3) ? 0.0 : x[2 * t + 1];   // mask the mean
-                                s2_dmma(ga0, ga1, x[2 * t], v.x);
-                                s2_dmma(ga0, ga1, a1, v.y);
+                                if (t < NT3 - 1 || LK >= 1) s2_dmma(ga0, ga1, x[2 * t], v.x);
+                                if (t < NT3 - 1 || LK == 2) {
+                                    const double a1 = (t == NT3 - 1 && c == 3) ? 0.0 : x[2 * t + 1];   // mask the mean
+                                    s2_dmma(ga0, ga1, a1, v.y);
+                                }
                             }
                         }
                         // lane c of a row holds g[row][2c], g[row][2c+1]: the row's 4 lanes exchange them through shared
@@ -557,28 +611,32 @@ __global__ void __launch_bounds__(S2_NW * 32, 1) state_sweep_2p_kernel(const S2P
                             gq[0] = t0.x; gq[1] = t0.y; gq[2] = t1.x; gq[3] = t1.y;
                         }
                         // step 2: the serial recurrence inside the batch (per row; every lane of the row computes it)
+                        // (coefficients G10 G20 | G21 G30 | G31 G32 | G54 G64 | G65 G74 | G75 G76)
+                        const double2 *gr = reinterpret_cast<const double2 *>(Gt + S2_TREC);
+                        const double2 r0 = gr[0], r1 = gr[1], r2 = gr[2];
                         double e[8];
-                        e[0] = om[0] * gq[0];
-                        e[1] = om[1] * (gq[1] - Gb[8] * e[0]);
-                        e[2] = om[2] * (gq[2] - Gb[16] * e[0] - Gb[17] * e[1]);
-                        e[3] = om[3] * (gq[3] - Gb[24] * e[0] - Gb[25] * e[1] - Gb[26] * e[2]);
+                        e[0] = om01.x * gq[0];
+                        e[1] = om01.y * (gq[1] - r0.x * e[0]);
+                        e[2] = om23.x * (gq[2] - r0.y * e[0] - r1.x * e[1]);
+                        e[3] = om23.y * (gq[3] - r1.y * e[0] - r2.x * e[1] - r2.y * e[2]);
                         const double ea = -s2_sel4(e[0], e[1], e[2], e[3], c);     // -e[c]: A operand below and in step 3
                         {
                             // obs 4..7 see obs 0..3 through one more 8x8x4 product on top of their own dots: the
                             // accumulator starts from g (lanes c = 2, 3 hold g[row][4..7] in fragment layout), A = -e,
-                            // B[k][j] = G[j][k] for the columns j = 4..7
+                            // B[k][j] = G[j][k] for the columns j = 4..7 and zero for j = 0..3
                             double k0 = ga0, k1 = ga1;
-                            s2_dmma(k0, k1, ea, (n >= 4) ? Gb[n * 8 + c] : 0.0);
+                            s2_dmma(k0, k1, ea, Gt[S2_TCORR + lane]);
                             __syncwarp();                           // everybody has read obs 0..3
                             xg[c] = make_double2(k0, k1);
                             __syncwarp();
                             const double2 t2 = xg[2], t3 = xg[3];
                             gq[4] = t2.x; gq[5] = t2.y; gq[6] = t3.x; gq[7] = t3.y;
                         }
-                        e[4] = om[4] * gq[4];
-                        e[5] = om[5] * (gq[5] - Gb[44] * e[4]);
-                        e[6] = om[6] * (gq[6] - Gb[52] * e[4] - Gb[53] * e[5]);
-                        e[7] = om[7] * (gq[7] - Gb[60] * e[4] - Gb[61] * e[5] - Gb[62] * e[6]);
+                        const double2 r3 = gr[3], r4 = gr[4], r5 = gr[5];
+                        e[4] = om45.x * gq[4];
+                        e[5] = om45.y * (gq[5] - r3.x * e[4]);
+                        e[6] = om67.x * (gq[6] - r3.y * e[4] - r4.x * e[5]);
+                        e[7] = om67.y * (gq[7] - r4.y * e[4] - r5.x * e[5] - r5.y * e[6]);
                         const double ea0 = ea;                 // A operand of the first k-step: -e[c]
                         const double ea1 = -s2_sel4(e[4], e[5], e[6], e[7], c);
 
@@ -620,7 +678,7 @@ __global__ void __launch_bounds__(S2_NW * 32, 1) state_sweep_2p_kernel(const S2P
                 for (int t = 0; t < NT3; ++t) {
 #pragma unroll
                     for (int h = 0; h < 2; ++h) {
-                        const int m = 8 * t + 2 * c + h;
+                        const int m = s2_slot<NT3, LK>(t, c, h);
                         if (m < nens) gXp[row * nens + m] = (TS)(x[2 * t + h] + mean);          // assimilation.py:168 when fused
                         else if (m == PC && !fused) gxm[row] = (TS)x[2 * t + h];
                     }
@@ -632,6 +690,7 @@ __global__ void __launch_bounds__(S2_NW * 32, 1) state_sweep_2p_kernel(const S2P
         S2_TICK(3);
 #pragma unroll
         for (int i = 0; i < 10; ++i) atomicAdd(&p.prof[i], (unsigned long long)pacc[i]);
+        atomicAdd(&p.prof[10], (unsigned long long)gbatch);
     }
     if (p.counters) {
 #pragma unroll
@@ -640,19 +699,22 @@ __global__ void __launch_bounds__(S2_NW * 32, 1) state_sweep_2p_kernel(const S2P
     }
 }
 
-// Yw[k][:] = (ye_k widened to double, zeros, -innov_k/beta_k in the last column); row nobs = zeros
-template <typename TS>
-__global__ void sweep_rows_kernel(const TS *__restrict__ Yp, const double *__restrict__ rec, int64_t nobs, int nens, int yw,
+// Yw[k][:] = (ye_k widened to double, zeros, -innov_k/beta_k in the last column), columns in the order of s2_slot;
+// row nobs = zeros
+template <int NT3, int LK, typename TS>
+__global__ void sweep_rows_kernel(const TS *__restrict__ Yp, const double *__restrict__ rec, int64_t nobs, int nens,
                                   double *__restrict__ Yw) {
+    constexpr int YW = 8 * NT3;
     const int64_t k = blockIdx.x;
-    for (int m = threadIdx.x; m < yw; m += blockDim.x) {
+    for (int col = threadIdx.x; col < YW; col += blockDim.x) {
+        const int m = s2_slot<NT3, LK>(col >> 3, (col & 7) >> 1, col & 1);
         double v = 0.0;
         if (k < nobs) {
             if (m < nens) v = (double)Yp[k * nens + m];
-            else if (m == yw - 1 && rec[REC_ASSIM * nobs + k] != 0.0)
+            else if (m == YW - 1 && rec[REC_ASSIM * nobs + k] != 0.0)
                 v = -rec[REC_INNOV * nobs + k] / rec[REC_BETA * nobs + k];       // xam = xbm + kmat*innov rides along (ensrf.py:130)
         }
-        Yw[k * yw + m] = v;
+        Yw[k * YW + col] = v;
     }
 }
 
@@ -854,7 +916,7 @@ static void s2_patch_shape(int64_t nlev, int64_t ny, int64_t nx, int *Lc_out, in
     *Lc_out = Lc; *bty_out = bty; *btx_out = btx;
 }
 
-template <int NT3, typename TS>
+template <int NT3, int LK, typename TS>
 static int s2_launch(S2Params &p, const TS *Yp, cudaStream_t st, const ExbSweepPlan *plan) {
     constexpr int NTH = S2_NW * 32, ROWS = S2_NW * 8;
     int Lc, bty, btx;
@@ -880,7 +942,7 @@ static int s2_launch(S2Params &p, const TS *Yp, cudaStream_t st, const ExbSweepP
     if (S < 4) return EXB_ERR_UNSUPPORTED;
     p.nstages = S;
     const size_t smem = fixed + sizeof(double) * (size_t)S * p.stage_doubles;
-    EXB_CUDA(cudaFuncSetAttribute(state_sweep_2p_kernel<NT3, TS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    EXB_CUDA(cudaFuncSetAttribute(state_sweep_2p_kernel<NT3, LK, TS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
 
     const int64_t npatches = (int64_t)p.ntx * p.npr * p.nlc;
     if (npatches >= 0x7fffffff) {
@@ -925,22 +987,22 @@ static int s2_launch(S2Params &p, const TS *Yp, cudaStream_t st, const ExbSweepP
         exb_set_error("exb_state_sweep: work buffers -> %s", cudaGetErrorString(e));
         rc = EXB_ERR_CUDA;
     } else {
-        sweep_rows_kernel<TS><<<(unsigned)(p.nobs + 1), 128, 0, st>>>(Yp, p.rec, p.nobs, p.nens, YW, Yw);
+        sweep_rows_kernel<NT3, LK, TS><<<(unsigned)(p.nobs + 1), 128, 0, st>>>(Yp, p.rec, p.nobs, p.nens, Yw);
         p.Yw = Yw; p.scratch = scratch; p.ticket = ticket;
         p.abort_flag = exb_status_slot_last_dev();
         unsigned long long *prof = nullptr;
         if (getenv("EXB_S2_PROF") && atoi(getenv("EXB_S2_PROF"))) {       // debugging aid: per-phase clocks of warp 0
-            if (cudaMalloc(&prof, 10 * sizeof(unsigned long long)) == cudaSuccess) cudaMemsetAsync(prof, 0, 10 * sizeof(unsigned long long), st);
+            if (cudaMalloc(&prof, 11 * sizeof(unsigned long long)) == cudaSuccess) cudaMemsetAsync(prof, 0, 11 * sizeof(unsigned long long), st);
             else prof = nullptr;
         }
         p.prof = prof;
         p.cand_cap = S2_CAND;
         if (const char *e = getenv("EXB_S2_CAP")) { const int v = atoi(e); if (v >= 2 * NTH && v <= S2_CAND) p.cand_cap = v; }
-        state_sweep_2p_kernel<NT3, TS><<<(unsigned)grid, NTH, smem, st>>>(p);
+        state_sweep_2p_kernel<NT3, LK, TS><<<(unsigned)grid, NTH, smem, st>>>(p);
         exb_count_launches(2);
         rc = exb_check_launch("state_sweep_2p_kernel");
         if (prof) {
-            unsigned long long h[10];
+            unsigned long long h[11];
             cudaStreamSynchronize(st);
             cudaMemcpy(h, prof, sizeof(h), cudaMemcpyDeviceToHost);
             cudaFree(prof);
@@ -950,6 +1012,10 @@ static int s2_launch(S2Params &p, const TS *Yp, cudaStream_t st, const ExbSweepP
             fprintf(stderr, "[s2 prof] grid %d patches %d: setup %.1f%% scan %.1f%% park+fence %.1f%% rows %.1f%% phaseB %.1f%% barriers %.1f%% | blocks: scalars %.1f%% omega %.1f%% gram %.1f%% rest %.1f%%  (%.3e clk per CTA)\n",
                     grid, p.npatches, 100 * h[0] / tot, 100 * h[1] / tot, 100 * h[2] / tot, 100 * h[3] / tot, 100 * h[4] / tot, 100 * h[5] / tot,
                     100 * h[6] / tot, 100 * h[7] / tot, 100 * h[8] / tot, 100 * h[9] / tot, tot / grid);
+            // clocks per (row, batch): a CTA takes its batches one after the other, over all of its ROWS row slots
+            const double rb = (double)(h[10] > 0 ? h[10] : 1) * ROWS;
+            fprintf(stderr, "[s2 prof] %llu batches: %.2f clk per (row, batch), phase B %.2f, blocks %.2f (omega %.2f, gram %.2f)\n",
+                    h[10], tot / rb, h[4] / rb, (h[6] + h[7] + h[8] + h[9]) / rb, h[7] / rb, h[8] / rb);
         }
     }
     if (Yw) cudaFreeAsync(Yw, st);
@@ -957,6 +1023,16 @@ static int s2_launch(S2Params &p, const TS *Yp, cudaStream_t st, const ExbSweepP
     if (ticket) cudaFreeAsync(ticket, st);
     sweep_free_lists(lists, st);
     return rc;
+}
+
+// the instantiation for the members in the last tile (s2_slot)
+template <int NT3, typename TS>
+static int s2_launch_lk(S2Params &p, const TS *Yp, cudaStream_t st, const ExbSweepPlan *plan) {
+    switch (s2_last_ksteps<NT3>(p.nens)) {
+    case 0: return s2_launch<NT3, 0, TS>(p, Yp, st, plan);
+    case 1: return s2_launch<NT3, 1, TS>(p, Yp, st, plan);
+    default: return s2_launch<NT3, 2, TS>(p, Yp, st, plan);
+    }
 }
 
 // Called from state_update.cu.  TS is the storage type of state and ye rows (float64, or float32 with float64
@@ -976,10 +1052,10 @@ int exb_state_sweep_2p(TS *xm, TS *Xp, int64_t nlev, int64_t ny, int64_t nx, int
     p.y_begin = (int)y_begin; p.y_end = (int)y_end;
     p.kloc = exb_loc_const();
     const int need = (nens + 1 + 7) / 8;            // 8-member tiles incl. the pseudo-member
-    if (need <= 4) return s2_launch<4, TS>(p, Yp, st, plan);
-    if (need <= 7) return s2_launch<7, TS>(p, Yp, st, plan);
-    if (need <= 10) return s2_launch<10, TS>(p, Yp, st, plan);
-    if (need <= 13) return s2_launch<13, TS>(p, Yp, st, plan);
+    if (need <= 4) return s2_launch_lk<4, TS>(p, Yp, st, plan);
+    if (need <= 7) return s2_launch_lk<7, TS>(p, Yp, st, plan);
+    if (need <= 10) return s2_launch_lk<10, TS>(p, Yp, st, plan);
+    if (need <= 13) return s2_launch_lk<13, TS>(p, Yp, st, plan);
     return EXB_ERR_UNSUPPORTED;                       // larger ensembles: state_update_mma.cu / state_update.cu
 }
 
