@@ -51,6 +51,12 @@ SIGNATURES = {
     'exb_obs_plan_destroy': [_p],
     'exb_obs_solve_planned_f64': [_p, _p, _p, _p, _p, _p, _p, _i64, _int, _int, _p, _p, _p],
     'exb_obs_solve_planned_f32': [_p, _p, _p, _p, _p, _p, _p, _i64, _int, _int, _p, _p, _p],
+    'exb_obs_solve_qc_f64': [_p, _p, _p, _p, _p, _p, _p, _i64, _int, _int, _p, _p, _p],
+    'exb_obs_solve_qc_f32': [_p, _p, _p, _p, _p, _p, _p, _i64, _int, _int, _p, _p, _p],
+    'exb_obs_solve_planned_qc_f64': [_p, _p, _p, _p, _p, _p, _p, _p, _i64, _int, _int, _p, _p, _p],
+    'exb_obs_solve_planned_qc_f32': [_p, _p, _p, _p, _p, _p, _p, _p, _i64, _int, _int, _p, _p, _p],
+    'exb_obs_solve_dist_qc_f64': [_p, _p, _p, _p, _p, _p, _p, _p, _i64, _int, _int, _p, _p, _int, _int, _p, _p, _p],
+    'exb_obs_solve_dist_qc_f32': [_p, _p, _p, _p, _p, _p, _p, _p, _i64, _int, _int, _p, _p, _int, _int, _p, _p, _p],
     'exb_state_update_f64': [_p, _p, _i64, _i64, _i64, _int, _p, _p, _p, _p, _i64, _i64, _i64, _int, _p, _p],
     'exb_state_update_f32': [_p, _p, _i64, _i64, _i64, _int, _p, _p, _p, _p, _i64, _i64, _i64, _int, _p, _p],
     'exb_state_sweep_f64': [_p, _i64, _i64, _i64, _int, _p, _p, _p, _p, _i64, _i64, _i64, _i64, _i64, _int, _p, _p],

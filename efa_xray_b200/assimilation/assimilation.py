@@ -42,9 +42,11 @@ class Assimilation():
         raise ValueError("loc must be None, False or 'GC' (got %r); other localisation types are not "
                          "defined by the reference (observation/observation.py:82)" % (loc,))
 
-    def _obs_arrays(self, loc_mode):
+    def _obs_arrays(self, loc_mode, outlier_threshold=None):
         """Structure-of-arrays view of self.obs with the forward-operator bookkeeping per ob.  One pass over the list
-        (operator.attrgetter pulls the eight attributes of an ob in C); everything after that is vectorised."""
+        (operator.attrgetter pulls the eight attributes of an ob in C); everything after that is vectorised.
+        outlier_threshold (validated by _validate_outlier_threshold) becomes the per-ob threshold array: the float for
+        every ob, or a dict's value for the obs of that variable and inf (not checked) for the others."""
         from operator import attrgetter
         st = self.prior
         obs = self.obs
@@ -82,11 +84,19 @@ class Assimilation():
             if any(r is None for r in radii):
                 abs(None)                                # numpy would turn None into NaN silently
             hw = np.abs(np.array(radii, dtype=np.float64))
+        thr = np.zeros(0)                                             # no check
+        if isinstance(outlier_threshold, dict):
+            per_var = np.full(len(varnames), np.inf)
+            for k, t in outlier_threshold.items():
+                per_var[varnames.index(k)] = float(t)
+            thr = per_var[var]
+        elif outlier_threshold is not None:
+            thr = np.full(n, float(outlier_threshold))
         return engine.ObsArrays(
             value=np.array(value, dtype=np.float64), error=np.array(error, dtype=np.float64),
             lat=np.array(lat, dtype=np.float64), lon=np.array(lon, dtype=np.float64),
             halfwidth=hw, assimilate=assim,
-            row0=(var * nt + tlo) * (ny * nx), row1=(var * nt + thi) * (ny * nx), tw0=wlo, tw1=whi)
+            row0=(var * nt + tlo) * (ny * nx), row1=(var * nt + thi) * (ny * nx), tw0=wlo, tw1=whi, threshold=thr)
 
     _DIM_KEYS = ['validtime', 'lat', 'lon', 'x', 'y']
 
@@ -159,6 +169,27 @@ class Assimilation():
                 self._check_alpha(v, 'of %r' % (k,))
         else:
             self._check_alpha(alpha, '')
+
+    @staticmethod
+    def _check_threshold(t, what):
+        if isinstance(t, bool) or not isinstance(t, (int, float, np.integer, np.floating)):
+            raise ValueError('outlier threshold %s must be a float, got %r' % (what, t))
+        if not 0.0 < float(t) < np.inf:                           # NaN fails here too
+            raise ValueError('outlier threshold %s must be positive and finite, got %r' % (what, t))
+
+    def _validate_outlier_threshold(self, outlier_threshold):
+        """None, a positive finite float, or a dict {variable name: positive finite float}; raises ValueError
+        otherwise.  Only reads the state's variable names (no device work)."""
+        if outlier_threshold is None:
+            return
+        if isinstance(outlier_threshold, dict):
+            varnames = self.prior.vars()
+            for k, t in outlier_threshold.items():
+                if k not in varnames:
+                    raise ValueError('outlier_threshold names %r, which is not a state variable %r' % (k, varnames))
+                self._check_threshold(t, 'of %r' % (k,))
+        else:
+            self._check_threshold(outlier_threshold, '')
 
     def _relaxation_levels(self, relaxation):
         """(kind, alpha per level) for engine.analysis_*, or None: one alpha per (variable, time) level, in the
@@ -277,13 +308,14 @@ class Assimilation():
         return post_state, self.obs
 
 
-def update(prior_state, obs, inflate=None, loc=False, nproc=1, verbose=False, relaxation=None):
+def update(prior_state, obs, inflate=None, loc=False, nproc=1, verbose=False, relaxation=None, outlier_threshold=None):
     """Module-level entry point (assimilation.py:176-222).  In the reference this calls an undefined
     enkf_update; here it runs the EnSRF.  nproc is accepted for signature compatibility: the GPU path does
-    not fork worker processes.  relaxation: posterior relaxation, as for EnSRF."""
+    not fork worker processes.  relaxation: posterior relaxation, outlier_threshold: outlier quality control, both as
+    for EnSRF."""
     from .ensrf import EnSRF
     return EnSRF(prior_state, obs, nproc=nproc, inflation=inflate, verbose=verbose, loc=loc,
-                 relaxation=relaxation).update()
+                 relaxation=relaxation, outlier_threshold=outlier_threshold).update()
 
 
 def randomize_obs_order(obs, seed=None):

@@ -10,8 +10,8 @@ from .. import engine
 
 
 class EnSRF(Assimilation):
-    """EnSRF(state, obs, nproc=1, inflation=None, verbose=True, loc=False, relaxation=None).update()
-    -> (post_state, obs).
+    """EnSRF(state, obs, nproc=1, inflation=None, verbose=True, loc=False, relaxation=None,
+    outlier_threshold=None).update() -> (post_state, obs).
 
     Same contract as the reference (ensrf.py:28-33, assimilation.py:171): `obs` is the caller's list,
     mutated in place with prior_mean / prior_var / post_mean / post_var / assimilated (ensrf.py:66-70,
@@ -31,14 +31,29 @@ class EnSRF(Assimilation):
     is unchanged, and rows without spread or that the analysis did not change are left as they are.  The per-ob
     diagnostics (prior_mean, prior_var, post_mean, post_var) are those of the serial loop: they are not re-evaluated
     after relaxation.  Invalid values raise ValueError here, before any device work.
+
+    `outlier_threshold` (not in the reference) keeps gross observation errors out of the analysis, as DART's
+    outlier threshold does, but checked inside the serial loop:
+      None                 no check (default)
+      t                    a positive finite float: the threshold of every ob
+      {variable: t}        a threshold per variable; obs of variables the dict does not name are not checked
+    An ob k with assimilate_this is rejected when |value - prior_mean| > t * sqrt(prior_var + error), with the prior
+    of ob k as the serial loop sees it, i.e. after obs 0..k-1 have been assimilated.  A rejected ob is treated as if
+    assimilate_this were False: prior_mean and prior_var are set, post_mean and post_var are not, assimilated is
+    False, and neither the state nor any later ob's prior feels it.  assimilate_this itself is left alone.  Invalid
+    values raise ValueError here, before any device work.  (A check against the priors before the loop needs no
+    library support: compute_ob_priors and assimilate_this.)
     """
 
-    def __init__(self, state, obs, nproc=1, inflation=None, verbose=True, loc=False, dtype='f64', relaxation=None):
+    def __init__(self, state, obs, nproc=1, inflation=None, verbose=True, loc=False, dtype='f64', relaxation=None,
+                 outlier_threshold=None):
         Assimilation.__init__(self, state, obs, nproc, inflation, verbose)
         self.loc = loc
         self.dtype = dtype
         self._validate_relaxation(relaxation)
         self.relaxation = relaxation
+        self._validate_outlier_threshold(outlier_threshold)
+        self.outlier_threshold = outlier_threshold
         self.last_result = None
 
     def update(self):
@@ -56,7 +71,7 @@ class EnSRF(Assimilation):
         nlev = st.nvars() * st.ntimes()
 
         if self.verbose: print("Computing observation priors")
-        obs = self._obs_arrays(loc_mode)
+        obs = self._obs_arrays(loc_mode, self.outlier_threshold)
         tdtype = {'f64': torch.float64, 'f32': torch.float32}[self.dtype]
         if self.verbose: print("Beginning observation loop")
         # The prior is read where it lies (the state's contiguous, page-locked block: no to_vect copy, and the prior

@@ -15,16 +15,17 @@
 
 template <typename T>
 int exb_obs_solve_dag(T *Ym, T *Yp, const double *ob_value, const double *ob_error, const uint8_t *ob_assim,
-                      const double *geo, int64_t nobs, int nens, int loc_mode, double *rec,
+                      const double *ob_thr, const double *geo, int64_t nobs, int nens, int loc_mode, double *rec,
                       unsigned long long *counters, cudaStream_t st, bool force, void *plan);
 template <typename T>
 int exb_obs_solve_persistent(T *Ym, T *Yp, const double *ob_value, const double *ob_error, const uint8_t *ob_assim,
-                             const double *geo, int64_t nobs, int nens, int loc_mode, double *rec,
+                             const double *ob_thr, const double *geo, int64_t nobs, int nens, int loc_mode, double *rec,
                              unsigned long long *counters, cudaStream_t st);
 
+// ob_thr: outlier threshold per ob (device array), or NULL for no check (DESIGN.md section 4.7)
 template <typename T>
 static int obs_solve_impl(T *Ym, T *Yp, const double *ob_value, const double *ob_error, const uint8_t *ob_assim,
-                          const double *geo, int64_t nobs, int nens, int loc_mode, double *rec,
+                          const double *ob_thr, const double *geo, int64_t nobs, int nens, int loc_mode, double *rec,
                           unsigned long long *counters, void *stream, void *plan = nullptr) {
     EXB_REQUIRE(Ym && Yp && ob_value && ob_error && ob_assim && geo && rec, "null pointer");
     EXB_REQUIRE(nobs > 0 && nens >= 2, "need nobs > 0 and nens >= 2");
@@ -41,32 +42,65 @@ static int obs_solve_impl(T *Ym, T *Yp, const double *ob_value, const double *ob
         return EXB_ERR_ARG;
     }
     if (dag || (!impl && loc_mode == EXB_LOC_GC)) {
-        const int rc = exb_obs_solve_dag<T>(Ym, Yp, ob_value, ob_error, ob_assim, geo, nobs, nens, loc_mode, rec,
+        const int rc = exb_obs_solve_dag<T>(Ym, Yp, ob_value, ob_error, ob_assim, ob_thr, geo, nobs, nens, loc_mode, rec,
                                             counters, st, dag, plan);
         if (rc != EXB_ERR_UNSUPPORTED) return rc;
     }
-    return exb_obs_solve_persistent<T>(Ym, Yp, ob_value, ob_error, ob_assim, geo, nobs, nens, loc_mode, rec, counters, st);
+    return exb_obs_solve_persistent<T>(Ym, Yp, ob_value, ob_error, ob_assim, ob_thr, geo, nobs, nens, loc_mode, rec, counters,
+                                       st);
 }
 
 extern "C" int exb_obs_solve_f64(double *Ym, double *Yp, const double *ob_value, const double *ob_error,
                                  const uint8_t *ob_assim, const double *obgeo, int64_t nobs, int nens,
                                  int loc_mode, double *rec, unsigned long long *counters, void *stream) {
-    return obs_solve_impl<double>(Ym, Yp, ob_value, ob_error, ob_assim, obgeo, nobs, nens, loc_mode, rec, counters, stream);
+    return obs_solve_impl<double>(Ym, Yp, ob_value, ob_error, ob_assim, nullptr, obgeo, nobs, nens, loc_mode, rec, counters,
+                                  stream);
 }
 extern "C" int exb_obs_solve_f32(float *Ym, float *Yp, const double *ob_value, const double *ob_error,
                                  const uint8_t *ob_assim, const double *obgeo, int64_t nobs, int nens,
                                  int loc_mode, double *rec, unsigned long long *counters, void *stream) {
-    return obs_solve_impl<float>(Ym, Yp, ob_value, ob_error, ob_assim, obgeo, nobs, nens, loc_mode, rec, counters, stream);
+    return obs_solve_impl<float>(Ym, Yp, ob_value, ob_error, ob_assim, nullptr, obgeo, nobs, nens, loc_mode, rec, counters,
+                                 stream);
 }
 
 // Same with a plan built earlier (exb_obs_plan_create), e.g. on a side stream while the ob priors were computed.
 extern "C" int exb_obs_solve_planned_f64(void *plan, double *Ym, double *Yp, const double *ob_value, const double *ob_error,
                                          const uint8_t *ob_assim, const double *obgeo, int64_t nobs, int nens, int loc_mode,
                                          double *rec, unsigned long long *counters, void *stream) {
-    return obs_solve_impl<double>(Ym, Yp, ob_value, ob_error, ob_assim, obgeo, nobs, nens, loc_mode, rec, counters, stream, plan);
+    return obs_solve_impl<double>(Ym, Yp, ob_value, ob_error, ob_assim, nullptr, obgeo, nobs, nens, loc_mode, rec, counters,
+                                  stream, plan);
 }
 extern "C" int exb_obs_solve_planned_f32(void *plan, float *Ym, float *Yp, const double *ob_value, const double *ob_error,
                                          const uint8_t *ob_assim, const double *obgeo, int64_t nobs, int nens, int loc_mode,
                                          double *rec, unsigned long long *counters, void *stream) {
-    return obs_solve_impl<float>(Ym, Yp, ob_value, ob_error, ob_assim, obgeo, nobs, nens, loc_mode, rec, counters, stream, plan);
+    return obs_solve_impl<float>(Ym, Yp, ob_value, ob_error, ob_assim, nullptr, obgeo, nobs, nens, loc_mode, rec, counters,
+                                 stream, plan);
+}
+
+// With the outlier check: ob_threshold is a device array of one threshold per ob (NULL: no check).
+extern "C" int exb_obs_solve_qc_f64(double *Ym, double *Yp, const double *ob_value, const double *ob_error,
+                                    const uint8_t *ob_assim, const double *ob_threshold, const double *obgeo, int64_t nobs,
+                                    int nens, int loc_mode, double *rec, unsigned long long *counters, void *stream) {
+    return obs_solve_impl<double>(Ym, Yp, ob_value, ob_error, ob_assim, ob_threshold, obgeo, nobs, nens, loc_mode, rec,
+                                  counters, stream);
+}
+extern "C" int exb_obs_solve_qc_f32(float *Ym, float *Yp, const double *ob_value, const double *ob_error,
+                                    const uint8_t *ob_assim, const double *ob_threshold, const double *obgeo, int64_t nobs,
+                                    int nens, int loc_mode, double *rec, unsigned long long *counters, void *stream) {
+    return obs_solve_impl<float>(Ym, Yp, ob_value, ob_error, ob_assim, ob_threshold, obgeo, nobs, nens, loc_mode, rec,
+                                 counters, stream);
+}
+extern "C" int exb_obs_solve_planned_qc_f64(void *plan, double *Ym, double *Yp, const double *ob_value,
+                                            const double *ob_error, const uint8_t *ob_assim, const double *ob_threshold,
+                                            const double *obgeo, int64_t nobs, int nens, int loc_mode, double *rec,
+                                            unsigned long long *counters, void *stream) {
+    return obs_solve_impl<double>(Ym, Yp, ob_value, ob_error, ob_assim, ob_threshold, obgeo, nobs, nens, loc_mode, rec,
+                                  counters, stream, plan);
+}
+extern "C" int exb_obs_solve_planned_qc_f32(void *plan, float *Ym, float *Yp, const double *ob_value,
+                                            const double *ob_error, const uint8_t *ob_assim, const double *ob_threshold,
+                                            const double *obgeo, int64_t nobs, int nens, int loc_mode, double *rec,
+                                            unsigned long long *counters, void *stream) {
+    return obs_solve_impl<float>(Ym, Yp, ob_value, ob_error, ob_assim, ob_threshold, obgeo, nobs, nens, loc_mode, rec,
+                                 counters, stream, plan);
 }

@@ -45,7 +45,7 @@
 
 template <typename T>
 int exb_obs_solve_dag(T *Ym, T *Yp, const double *ob_value, const double *ob_error, const uint8_t *ob_assim,
-                      const double *geo, int64_t nobs, int nens, int loc_mode, double *rec,
+                      const double *ob_thr, const double *geo, int64_t nobs, int nens, int loc_mode, double *rec,
                       unsigned long long *counters, cudaStream_t st, bool force, void *plan);
 
 __device__ __forceinline__ int64_t ceil_div64_dev(int64_t a, int64_t b) { return (a + b - 1) / b; }
@@ -199,6 +199,7 @@ struct DgArgs {
     const double *ob_value;
     const double *ob_error;
     const uint8_t *ob_assim;
+    const double *ob_thr;        // outlier threshold per ob (QC instantiations only)
     const double *geo;
     double *rec;
     unsigned long long *counters;
@@ -459,7 +460,17 @@ __device__ __forceinline__ bool dg_step(const DgArgs<T> &a, int lane, DgRow<T, M
     return more;
 }
 
-template <typename T, int MC, bool DIST>
+// |innov| > t sqrt(kdenom) in float64 with a correctly rounded sqrt (DESIGN.md section 4.7).  Not inlined, and called
+// by lane 0 only: inlined, the threshold load and the sqrt's slow path raised the register pressure of the whole
+// kernel and added spills to the predecessor loop.
+__device__ __noinline__ bool dg_outlier(const double *thr, int64_t j, double innov, double kdenom) {
+    return fabs(innov) > thr[j] * sqrt(kdenom);
+}
+
+// QC: outlier check of every assimilated ob against its in-loop prior (DESIGN.md section 4.7).  A rejected ob still
+// publishes its record, with scalars (0, 0): its successors' lists were built from the user flags and wait for it,
+// and zero scalars make their update by it exactly the identity.
+template <typename T, int MC, bool DIST, bool QC>
 __global__ void __launch_bounds__(DG_WARPS * 32, DG_MINBLOCKS) dag_solve_kernel(const DgArgs<T> a) {
     constexpr int NW = DgCfg<T, MC>::NW;
     constexpr int PER = DgWord<T>::PER;
@@ -580,8 +591,11 @@ __global__ void __launch_bounds__(DG_WARPS * 32, DG_MINBLOCKS) dag_solve_kernel(
         const double kdenom = varye + my_err;
         const double c1 = 1.0 / ((double)(nens - 1) * kdenom);
         const double beta = 1.0 / (1.0 + sq_err * rsqrt(kdenom));                    // 1/(1+sqrt(R/kdenom))
+        bool rej = false;                 // outlier: only lane 0 decides, and only lane 0 publishes and records
         if (act && lane == 0) {
-            const unsigned long long s0w = dg_pack_scalar(c1 * innov), s1w = dg_pack_scalar(c1 * beta);
+            if constexpr (QC) rej = dg_outlier(a.ob_thr, j, innov, kdenom);
+            const unsigned long long s0w = rej ? 0ull : dg_pack_scalar(c1 * innov);
+            const unsigned long long s1w = rej ? 0ull : dg_pack_scalar(c1 * beta);
             if (!DIST) {
                 dg_st16(a.S + j * 2, s0w, s1w);
             } else {
@@ -603,10 +617,10 @@ __global__ void __launch_bounds__(DG_WARPS * 32, DG_MINBLOCKS) dag_solve_kernel(
             a.rec[REC_PRIOR_MEAN * nobs + j] = mj;                                   // ensrf.py:66
             a.rec[REC_PRIOR_VAR * nobs + j] = varye;                                 // ensrf.py:70
             a.rec[REC_INNOV * nobs + j] = innov;
-            a.rec[REC_C1 * nobs + j] = c1;
+            a.rec[REC_C1 * nobs + j] = rej ? 0.0 : c1;
             a.rec[REC_BETA * nobs + j] = beta;
-            a.rec[REC_ASSIM * nobs + j] = act ? 1.0 : 0.0;
-            if (act) {
+            a.rec[REC_ASSIM * nobs + j] = act && !rej ? 1.0 : 0.0;
+            if (act && !rej) {
                 // the ob's own row: weight at distance 0, kcov = ye.ye/(N-1)   (ensrf.py:144-147)
                 const double wself = gc ? loc_weight(0.0, a.geo[GEO_INVHW * nobs + j], a.geo[GEO_AMAX * nobs + j]) : 1.0;
                 const double kmat = wself * rq * c1;
@@ -758,12 +772,12 @@ static int dg_plan_build(const double *geo, const uint8_t *ob_assim, int64_t nob
     return rc2;
 }
 
-template <typename T, int MC, bool DIST>
+template <typename T, int MC, bool DIST, bool QC>
 static int dg_run(DgArgs<T> a, const ExbObsPlan &pl, cudaStream_t st) {
     int dev = 0, sms = 0, per_sm = 0;
     EXB_CUDA(cudaGetDevice(&dev));
     EXB_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-    EXB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, dag_solve_kernel<T, MC, DIST>, DG_WARPS * 32, 0));
+    EXB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, dag_solve_kernel<T, MC, DIST, QC>, DG_WARPS * 32, 0));
     if (per_sm < 1) return EXB_ERR_UNSUPPORTED;
     const int64_t nobs = a.nobs;
     const std::vector<int64_t> &off_h = pl.off_h;
@@ -814,17 +828,26 @@ static int dg_run(DgArgs<T> a, const ExbObsPlan &pl, cudaStream_t st) {
         int64_t grid = (int64_t)sms * per_sm;
         const int64_t need = ceil_div64(DIST ? pl.nrows + 1 : nrows, DG_WARPS);
         if (grid > need) grid = need;
-        dag_solve_kernel<T, MC, DIST><<<(unsigned)grid, DG_WARPS * 32, 0, st>>>(a);
+        dag_solve_kernel<T, MC, DIST, QC><<<(unsigned)grid, DG_WARPS * 32, 0, st>>>(a);
         exb_count_launches(1);
     }
     return exb_check_launch("dag_solve_kernel");
+}
+
+// members per lane (MC) and outlier check (a.ob_thr != NULL) -> kernel instantiation
+template <typename T, bool DIST>
+static int dg_dispatch(const DgArgs<T> &a, const ExbObsPlan &pl, cudaStream_t st) {
+    const bool qc = a.ob_thr != nullptr;
+    if (a.nens <= 128) return qc ? dg_run<T, 4, DIST, true>(a, pl, st) : dg_run<T, 4, DIST, false>(a, pl, st);
+    if (a.nens <= 256) return qc ? dg_run<T, 8, DIST, true>(a, pl, st) : dg_run<T, 8, DIST, false>(a, pl, st);
+    return EXB_ERR_UNSUPPORTED;
 }
 
 // force = false: returns EXB_ERR_UNSUPPORTED when the dependency graph is too dense for this method to pay
 // (the caller then uses the panel kernel).  plan may be null (a temporary one is built on st).
 template <typename T>
 int exb_obs_solve_dag(T *Ym, T *Yp, const double *ob_value, const double *ob_error, const uint8_t *ob_assim,
-                      const double *geo, int64_t nobs, int nens, int loc_mode, double *rec,
+                      const double *ob_thr, const double *geo, int64_t nobs, int nens, int loc_mode, double *rec,
                       unsigned long long *counters, cudaStream_t st, bool force, void *plan_in) {
     ExbObsPlan *pl = static_cast<ExbObsPlan *>(plan_in), *tmp = nullptr;
     if (!pl) {
@@ -851,15 +874,14 @@ int exb_obs_solve_dag(T *Ym, T *Yp, const double *ob_value, const double *ob_err
         a.status = sd;
         a.watchdog_ns = dg_watchdog_ns(nobs);
     }
-    a.Ym = Ym; a.Yp = Yp; a.ob_value = ob_value; a.ob_error = ob_error; a.ob_assim = ob_assim; a.geo = geo; a.rec = rec;
+    a.Ym = Ym; a.Yp = Yp; a.ob_value = ob_value; a.ob_error = ob_error; a.ob_assim = ob_assim; a.ob_thr = ob_thr;
+    a.geo = geo; a.rec = rec;
     a.counters = counters; a.off = pl->off; a.list = nullptr; a.list_base = 0; a.P = nullptr; a.S = nullptr;
     a.ticket = nullptr; a.nobs = nobs; a.row_begin = 0; a.row_end = nobs; a.nens = nens;
     a.loc_mode = loc_mode; a.inv_n = 1.0 / (double)nens;
     a.world = 1; a.rank = 0; a.deal = DgDeal{1, 1, 0};
     for (int q = 0; q < 8; ++q) { a.P_peer[q] = nullptr; a.S_peer[q] = nullptr; }
-    int rc = EXB_ERR_UNSUPPORTED;
-    if (nens <= 128) rc = dg_run<T, 4, false>(a, *pl, st);
-    else if (nens <= 256) rc = dg_run<T, 8, false>(a, *pl, st);
+    const int rc = dg_dispatch<T, false>(a, *pl, st);
     if (!tmp) {
         cudaEventRecord(pl->used, st);
         pl->was_used = true;
@@ -878,8 +900,8 @@ int exb_obs_solve_dag(T *Ym, T *Yp, const double *ob_value, const double *ob_err
 // rank's own rows only: the caller zeroes the others and sums over the group.
 template <typename T>
 static int dg_solve_dist(void *plan, T *Ym, T *Yp, const double *ob_value, const double *ob_error, const uint8_t *ob_assim,
-                         const double *geo, int64_t nobs, int nens, int loc_mode, double *rec, unsigned long long *counters,
-                         int rank, int world, void *const *P_peers, void *const *S_peers, cudaStream_t st) {
+                         const double *ob_thr, const double *geo, int64_t nobs, int nens, int loc_mode, double *rec,
+                         unsigned long long *counters, int rank, int world, void *const *P_peers, void *const *S_peers, cudaStream_t st) {
     EXB_REQUIRE(plan && Ym && Yp && ob_value && ob_error && ob_assim && geo && rec && P_peers && S_peers, "null pointer");
     EXB_REQUIRE(world >= 1 && world <= 8 && rank >= 0 && rank < world, "bad rank / world");
     ExbObsPlan *pl = static_cast<ExbObsPlan *>(plan);
@@ -900,15 +922,14 @@ static int dg_solve_dist(void *plan, T *Ym, T *Yp, const double *ob_value, const
         a.status = sd;
         a.watchdog_ns = dg_watchdog_ns(nobs);
     }
-    a.Ym = Ym; a.Yp = Yp; a.ob_value = ob_value; a.ob_error = ob_error; a.ob_assim = ob_assim; a.geo = geo; a.rec = rec;
+    a.Ym = Ym; a.Yp = Yp; a.ob_value = ob_value; a.ob_error = ob_error; a.ob_assim = ob_assim; a.ob_thr = ob_thr;
+    a.geo = geo; a.rec = rec;
     a.counters = counters; a.off = pl->off; a.list = nullptr; a.list_base = 0; a.P = nullptr; a.S = nullptr;
     a.ticket = nullptr; a.nobs = nobs; a.row_begin = 0; a.row_end = nobs; a.nens = nens;
     a.loc_mode = loc_mode; a.inv_n = 1.0 / (double)nens;
     a.world = world; a.rank = rank; a.deal = pl->deal;
     for (int q = 0; q < 8; ++q) { a.P_peer[q] = q < world ? P_peers[q] : nullptr; a.S_peer[q] = q < world ? S_peers[q] : nullptr; }
-    int rc = EXB_ERR_UNSUPPORTED;
-    if (nens <= 128) rc = dg_run<T, 4, true>(a, *pl, st);
-    else if (nens <= 256) rc = dg_run<T, 8, true>(a, *pl, st);
+    const int rc = dg_dispatch<T, true>(a, *pl, st);
     cudaEventRecord(pl->used, st);
     pl->was_used = true;
     return rc;
@@ -918,15 +939,29 @@ extern "C" int exb_obs_solve_dist_f64(void *plan, double *Ym, double *Yp, const 
                                       const uint8_t *ob_assim, const double *obgeo, int64_t nobs, int nens, int loc_mode,
                                       double *rec, unsigned long long *counters, int rank, int world, void *const *P_peers,
                                       void *const *S_peers, void *stream) {
-    return dg_solve_dist<double>(plan, Ym, Yp, ob_value, ob_error, ob_assim, obgeo, nobs, nens, loc_mode, rec, counters, rank,
-                                 world, P_peers, S_peers, (cudaStream_t)stream);
+    return dg_solve_dist<double>(plan, Ym, Yp, ob_value, ob_error, ob_assim, nullptr, obgeo, nobs, nens, loc_mode, rec, counters,
+                                 rank, world, P_peers, S_peers, (cudaStream_t)stream);
 }
 extern "C" int exb_obs_solve_dist_f32(void *plan, float *Ym, float *Yp, const double *ob_value, const double *ob_error,
                                       const uint8_t *ob_assim, const double *obgeo, int64_t nobs, int nens, int loc_mode,
                                       double *rec, unsigned long long *counters, int rank, int world, void *const *P_peers,
                                       void *const *S_peers, void *stream) {
-    return dg_solve_dist<float>(plan, Ym, Yp, ob_value, ob_error, ob_assim, obgeo, nobs, nens, loc_mode, rec, counters, rank,
-                                world, P_peers, S_peers, (cudaStream_t)stream);
+    return dg_solve_dist<float>(plan, Ym, Yp, ob_value, ob_error, ob_assim, nullptr, obgeo, nobs, nens, loc_mode, rec, counters,
+                                rank, world, P_peers, S_peers, (cudaStream_t)stream);
+}
+extern "C" int exb_obs_solve_dist_qc_f64(void *plan, double *Ym, double *Yp, const double *ob_value, const double *ob_error,
+                                         const uint8_t *ob_assim, const double *ob_threshold, const double *obgeo, int64_t nobs,
+                                         int nens, int loc_mode, double *rec, unsigned long long *counters, int rank, int world,
+                                         void *const *P_peers, void *const *S_peers, void *stream) {
+    return dg_solve_dist<double>(plan, Ym, Yp, ob_value, ob_error, ob_assim, ob_threshold, obgeo, nobs, nens, loc_mode, rec,
+                                 counters, rank, world, P_peers, S_peers, (cudaStream_t)stream);
+}
+extern "C" int exb_obs_solve_dist_qc_f32(void *plan, float *Ym, float *Yp, const double *ob_value, const double *ob_error,
+                                         const uint8_t *ob_assim, const double *ob_threshold, const double *obgeo, int64_t nobs,
+                                         int nens, int loc_mode, double *rec, unsigned long long *counters, int rank, int world,
+                                         void *const *P_peers, void *const *S_peers, void *stream) {
+    return dg_solve_dist<float>(plan, Ym, Yp, ob_value, ob_error, ob_assim, ob_threshold, obgeo, nobs, nens, loc_mode, rec,
+                                counters, rank, world, P_peers, S_peers, (cudaStream_t)stream);
 }
 
 extern "C" int exb_obs_plan_create(const double *obgeo, const uint8_t *ob_assim, int64_t nobs, int loc_mode, void *stream,
@@ -961,6 +996,8 @@ extern "C" int exb_obs_plan_destroy(void *plan) {
 }
 
 template int exb_obs_solve_dag<double>(double *, double *, const double *, const double *, const uint8_t *, const double *,
-                                       int64_t, int, int, double *, unsigned long long *, cudaStream_t, bool, void *);
+                                       const double *, int64_t, int, int, double *, unsigned long long *, cudaStream_t, bool,
+                                       void *);
 template int exb_obs_solve_dag<float>(float *, float *, const double *, const double *, const uint8_t *, const double *,
-                                      int64_t, int, int, double *, unsigned long long *, cudaStream_t, bool, void *);
+                                      const double *, int64_t, int, int, double *, unsigned long long *, cudaStream_t, bool,
+                                      void *);

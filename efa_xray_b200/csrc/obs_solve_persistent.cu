@@ -63,6 +63,7 @@ struct PsArgs {
     const double *ob_value;
     const double *ob_error;
     const uint8_t *ob_assim;
+    const double *ob_thr;        // outlier threshold per ob (QC instantiations only)
     const double *geo;
     double *rec;
     unsigned long long *counters;
@@ -158,7 +159,16 @@ struct PsObScalars {
     double innov, c1, beta, sum, sq;
 };
 
-template <typename T, int MC>
+// |innov| > t sqrt(kdenom) in float64 with a correctly rounded sqrt (DESIGN.md section 4.7).  Not inlined: inlined, the
+// threshold load and the sqrt's slow path added spills to the instantiations above 152 members.
+__device__ __noinline__ bool ps_outlier(const double *thr, int64_t k, double innov, double kdenom) {
+    return fabs(innov) > thr[k] * sqrt(kdenom);
+}
+
+// QC: outlier check of every assimilated ob against its in-loop prior (DESIGN.md section 4.7).  The panel worker hands
+// the rest of its panel zero scalars for a rejected ob (an exact identity update) and records it as not assimilated,
+// so the trailing workers skip it.
+template <typename T, int MC, bool QC>
 __global__ void __launch_bounds__(PS_THREADS, 1) obs_solve_persistent_kernel(const PsArgs<T> a) {
     __shared__ PsShared sh;
     __shared__ T s_ye[2][PS_GS * MC];
@@ -260,15 +270,17 @@ __global__ void __launch_bounds__(PS_THREADS, 1) obs_solve_persistent_kernel(con
                         const double kdenom = varye + my_err;
                         const double c1 = 1.0 / ((double)(nens - 1) * kdenom);
                         const double beta = 1.0 / (1.0 + my_serr * rsqrt(kdenom));      // 1/(1+sqrt(R/kdenom))
-                        s_ob[buf].innov = innov; s_ob[buf].c1 = c1; s_ob[buf].beta = beta;
+                        bool rej = false;                                               // |innov| > t sqrt(kdenom)
+                        if constexpr (QC) rej = act && ps_outlier(a.ob_thr, kk, innov, kdenom);
+                        s_ob[buf].innov = rej ? 0.0 : innov; s_ob[buf].c1 = rej ? 0.0 : c1; s_ob[buf].beta = beta;
                         s_ob[buf].sum = rs; s_ob[buf].sq = rq;
                         a.rec[REC_PRIOR_MEAN * nobs + kk] = mj;                          // ensrf.py:66
                         a.rec[REC_PRIOR_VAR * nobs + kk] = varye;                        // ensrf.py:70
                         a.rec[REC_INNOV * nobs + kk] = innov;
-                        a.rec[REC_C1 * nobs + kk] = c1;
+                        a.rec[REC_C1 * nobs + kk] = rej ? 0.0 : c1;
                         a.rec[REC_BETA * nobs + kk] = beta;
-                        a.rec[REC_ASSIM * nobs + kk] = act ? 1.0 : 0.0;
-                        if (act) {
+                        a.rec[REC_ASSIM * nobs + kk] = act && !rej ? 1.0 : 0.0;
+                        if (act && !rej) {
                             // the ob's own row: weight at distance 0, kcov = ye.ye/(N-1)   (ensrf.py:144-147)
                             const double kmat = my_wself * rq * c1;
                             const double shrink = 1.0 - beta * kmat;
@@ -370,7 +382,8 @@ __global__ void __launch_bounds__(PS_THREADS, 1) obs_solve_persistent_kernel(con
 
 template <typename T, int MC>
 static int ps_launch(PsArgs<T> &a, cudaStream_t st) {
-    const void *kernel = (const void *)obs_solve_persistent_kernel<T, MC>;
+    const void *kernel = a.ob_thr ? (const void *)obs_solve_persistent_kernel<T, MC, true>
+                                  : (const void *)obs_solve_persistent_kernel<T, MC, false>;
     int dev = 0, sms = 0, coop = 0, per_sm = 0;
     EXB_CUDA(cudaGetDevice(&dev));
     EXB_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
@@ -413,10 +426,11 @@ static int ps_launch(PsArgs<T> &a, cudaStream_t st) {
 
 template <typename T>
 int exb_obs_solve_persistent(T *Ym, T *Yp, const double *ob_value, const double *ob_error, const uint8_t *ob_assim,
-                             const double *geo, int64_t nobs, int nens, int loc_mode, double *rec,
+                             const double *ob_thr, const double *geo, int64_t nobs, int nens, int loc_mode, double *rec,
                              unsigned long long *counters, cudaStream_t st) {
     PsArgs<T> a;
-    a.Ym = Ym; a.Yp = Yp; a.ob_value = ob_value; a.ob_error = ob_error; a.ob_assim = ob_assim; a.geo = geo;
+    a.Ym = Ym; a.Yp = Yp; a.ob_value = ob_value; a.ob_error = ob_error; a.ob_assim = ob_assim; a.ob_thr = ob_thr;
+    a.geo = geo;
     a.rec = rec; a.counters = counters; a.ctl = nullptr; a.nobs = nobs; a.nens = nens; a.loc_mode = loc_mode;
     a.npanels = (int)((nobs + PS_PB - 1) / PS_PB);
     const int mc = (nens + PS_GS - 1) / PS_GS;
@@ -432,6 +446,8 @@ int exb_obs_solve_persistent(T *Ym, T *Yp, const double *ob_value, const double 
 }
 
 template int exb_obs_solve_persistent<double>(double *, double *, const double *, const double *, const uint8_t *,
-                                              const double *, int64_t, int, int, double *, unsigned long long *, cudaStream_t);
+                                              const double *, const double *, int64_t, int, int, double *, unsigned long long *,
+                                              cudaStream_t);
 template int exb_obs_solve_persistent<float>(float *, float *, const double *, const double *, const uint8_t *,
-                                             const double *, int64_t, int, int, double *, unsigned long long *, cudaStream_t);
+                                             const double *, const double *, int64_t, int, int, double *, unsigned long long *,
+                                             cudaStream_t);

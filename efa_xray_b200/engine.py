@@ -34,6 +34,13 @@ class ObsArrays:
     row1: np.ndarray             # first state row of (variable, upper time level)
     tw0: np.ndarray              # time weights of the two levels (state/ensemble.py:202-224)
     tw1: np.ndarray
+    # outlier threshold per ob (inf: not checked); empty, the default: no check at all (DESIGN.md 4.7).  Every field
+    # is a per-ob array, so a slice of every field is the ObsArrays of those obs.
+    threshold: np.ndarray = field(default_factory=lambda: np.zeros(0))
+
+    @property
+    def qc(self):
+        return len(self.threshold) > 0
 
     @property
     def nobs(self):
@@ -245,14 +252,22 @@ class _Timer:
         return out
 
 
+def _qc_args(obs_dev):
+    """('qc_', (threshold pointer,)) for the _qc entries of the obs-space solve when upload_obs staged outlier
+    thresholds, else ('', ())."""
+    thr = obs_dev.get('threshold')
+    return ('qc_', (_lib.ptr(thr),)) if thr is not None else ('', ())
+
+
 def obs_solve(Ym, Yp, obs_dev, geo, nens, loc_mode, rec, counters, sfx, plan=None):
+    qc, thr = _qc_args(obs_dev)
     if plan is not None:
-        _lib.call('exb_obs_solve_planned_' + sfx, plan.handle, _lib.ptr(Ym), _lib.ptr(Yp), _lib.ptr(obs_dev['value']),
-                  _lib.ptr(obs_dev['error']), _lib.ptr(obs_dev['assimilate']), _lib.ptr(geo), Ym.shape[0], nens,
+        _lib.call('exb_obs_solve_planned_' + qc + sfx, plan.handle, _lib.ptr(Ym), _lib.ptr(Yp), _lib.ptr(obs_dev['value']),
+                  _lib.ptr(obs_dev['error']), _lib.ptr(obs_dev['assimilate']), *thr, _lib.ptr(geo), Ym.shape[0], nens,
                   loc_mode, _lib.ptr(rec), _lib.ptr(counters), _lib.stream_ptr())
         return
-    _lib.call('exb_obs_solve_' + sfx, _lib.ptr(Ym), _lib.ptr(Yp), _lib.ptr(obs_dev['value']),
-              _lib.ptr(obs_dev['error']), _lib.ptr(obs_dev['assimilate']), _lib.ptr(geo), Ym.shape[0], nens,
+    _lib.call('exb_obs_solve_' + qc + sfx, _lib.ptr(Ym), _lib.ptr(Yp), _lib.ptr(obs_dev['value']),
+              _lib.ptr(obs_dev['error']), _lib.ptr(obs_dev['assimilate']), *thr, _lib.ptr(geo), Ym.shape[0], nens,
               loc_mode, _lib.ptr(rec), _lib.ptr(counters), _lib.stream_ptr())
 
 
@@ -359,15 +374,17 @@ def obs_solve_distributed(Ym, Yp, obs_dev, geo, nens, loc_mode, rec, counters, s
     c0 = counters[0:1].clone()
     counters[0:1].zero_()
     lib = _lib.load()
-    rc = getattr(lib, 'exb_obs_solve_dist_' + sfx)(
+    qc, thr = _qc_args(obs_dev)
+    rc = getattr(lib, 'exb_obs_solve_dist_' + qc + sfx)(
         plan.handle, _lib.ptr(Ym), _lib.ptr(Yp), _lib.ptr(obs_dev['value']), _lib.ptr(obs_dev['error']),
-        _lib.ptr(obs_dev['assimilate']), _lib.ptr(geo), nobs, nens, loc_mode, _lib.ptr(rec), _lib.ptr(counters), rank, world,
-        pp, sp, _lib.stream_ptr())
+        _lib.ptr(obs_dev['assimilate']), *thr, _lib.ptr(geo), nobs, nens, loc_mode, _lib.ptr(rec), _lib.ptr(counters), rank,
+        world, pp, sp, _lib.stream_ptr())
     if rc == -3:                       # EXB_ERR_UNSUPPORTED: identical decision on every rank (same plan)
         counters[0:1].copy_(c0)
         return False
     if rc != 0:
-        raise _lib.ExbError('exb_obs_solve_dist_%s failed (%d): %s' % (sfx, rc, lib.exb_last_error().decode('utf-8', 'replace')))
+        raise _lib.ExbError('exb_obs_solve_dist_%s%s failed (%d): %s' % (qc, sfx, rc,
+                                                                       lib.exb_last_error().decode('utf-8', 'replace')))
     merge_distributed_records(Ym, rec, counters[0:1], plan.block, rank, world, g)
     counters[0:1].add_(c0)
     # every rank's record buffer holds the published ye row of EVERY ob once all ranks are done (the all-reduces above
@@ -535,11 +552,16 @@ _STAGING = {}
 def upload_obs(obs: ObsArrays, device, loc_mode):
     """Per-ob tables on the device + the obgeo block of exb_obs_prepare.  Everything goes up in ONE copy from a cached
     page-locked staging buffer (nine 8-byte fields + the assimilate flags per ob): small pageable copies cost a
-    host synchronisation each and may not queue behind bulk state copies."""
+    host synchronisation each and may not queue behind bulk state copies.  With outlier thresholds (obs.qc) they are
+    a tenth 8-byte field, d['threshold']; without, d has no such entry and the layout is the nine fields."""
     torch = _torch()
     n = obs.nobs
-    nf = len(_OBS_FIELDS)
-    key = (n, str(device))
+    if obs.qc and np.shape(obs.threshold) != (n,):
+        raise ValueError('ObsArrays.threshold needs one value per ob (%d) or none, got shape %r'
+                         % (n, np.shape(obs.threshold)))
+    fields = _OBS_FIELDS + ('threshold',) if obs.qc else _OBS_FIELDS
+    nf = len(fields)
+    key = (n, nf, str(device))
     ent = _STAGING.get(key)
     if ent is None:
         if len(_STAGING) > 8:
@@ -555,6 +577,8 @@ def upload_obs(obs: ObsArrays, device, loc_mode):
     f64[4] = obs.halfwidth if loc_mode == LOC_GC else 1.0
     f64[5], f64[6] = obs.tw0, obs.tw1
     i64[7], i64[8] = obs.row0, obs.row1
+    if obs.qc:
+        f64[9] = obs.threshold
     hb[nf * n * 8:] = obs.assimilate
     db = torch.empty(nf * n * 8 + n, dtype=torch.uint8, device=device)
     db.copy_(ent['host'], non_blocking=True)
@@ -562,7 +586,7 @@ def upload_obs(obs: ObsArrays, device, loc_mode):
     ent['event'].record()
     df = db[:nf * n * 8].view(torch.float64).view(nf, n)
     di = db[:nf * n * 8].view(torch.int64).view(nf, n)
-    d = {name: (di[i] if name in ('row0', 'row1') else df[i]) for i, name in enumerate(_OBS_FIELDS)}
+    d = {name: (di[i] if name in ('row0', 'row1') else df[i]) for i, name in enumerate(fields)}
     d['assimilate'] = db[nf * n * 8:]
     d['_buffer'] = db
     if loc_mode != LOC_GC:
@@ -593,6 +617,9 @@ def analysis_device(X, nlev, grid: GridTables, obs: ObsArrays, loc_mode, inflati
              kind 'rtps' (relaxation to prior spread) or 'rtpp' (relaxation to prior perturbations), relative to the
              prior as the sweep receives it (after inflation); DESIGN.md section 4.6.  Every alpha 0 launches nothing.
              The per-ob diagnostics stay those of the serial loop.  res.ms gains 'relax' when it ran.
+    obs.threshold  empty (no check), or outlier thresholds per ob: the obs-space solve rejects an ob whose innovation exceeds
+             its threshold times sqrt(prior variance + error) inside the serial loop (DESIGN.md section 4.7);
+             rejected obs come back with assimilated False, and the state sweep applies a zero update for them.
     sweep_bands  optional list of (ya, yb) row ranges of the shard: the fused sweep is issued range by range and
              on_band_done(ya, yb) is called after each launch has been enqueued (e.g. to start its download),
              before_band(ya, yb) before it (e.g. to wait for its upload).

@@ -228,6 +228,37 @@ int exb_obs_solve_dist_f32(void *plan, float *Ym, float *Yp, const double *ob_va
                            double *rec, unsigned long long *counters, int rank, int world, void *const *P_peers,
                            void *const *S_peers, void *stream);
 
+/* Outlier quality control inside the serial loop (DESIGN.md section 4.7): the entries above with one more argument,
+ * ob_threshold, a DEVICE array of one threshold t_k per ob (NULL: no check, exactly the entries above).  An ob k with
+ * ob_assimilate[k] != 0 is rejected when |value_k - mye_k| > t_k * sqrt(varye_k + error_k), evaluated in float64 with
+ * a correctly rounded sqrt on its prior INSIDE the loop (after obs 0..k-1); t_k = +inf never rejects.  A rejected ob
+ * is left out exactly as if its flag were 0: rec 7 = 0.0, post_mean / post_var NaN, no obs row changes; prior_mean,
+ * prior_var, innovation and beta are recorded as usual and rec 5 (1/((Nens-1)*kdenom)) is 0, so that a state sweep
+ * given these records applies an exact zero update for it.  ob_assimilate itself is not modified: predecessor lists and
+ * sweep plans keep being built from it.  The pair counter then counts the pairs the kernels visit, which includes the
+ * pairs of a rejected ob with later obs wherever a kernel reaches them before its rejection is known (all of them in
+ * the dependency-driven solve, those inside its panel in the persistent solve), so it depends on the implementation. */
+int exb_obs_solve_qc_f64(double *Ym, double *Yp, const double *ob_value, const double *ob_error,
+                         const uint8_t *ob_assimilate, const double *ob_threshold, const double *obgeo, int64_t nobs,
+                         int nens, int loc_mode, double *rec, unsigned long long *counters, void *stream);
+int exb_obs_solve_qc_f32(float *Ym, float *Yp, const double *ob_value, const double *ob_error,
+                         const uint8_t *ob_assimilate, const double *ob_threshold, const double *obgeo, int64_t nobs,
+                         int nens, int loc_mode, double *rec, unsigned long long *counters, void *stream);
+int exb_obs_solve_planned_qc_f64(void *plan, double *Ym, double *Yp, const double *ob_value, const double *ob_error,
+                                 const uint8_t *ob_assimilate, const double *ob_threshold, const double *obgeo, int64_t nobs,
+                                 int nens, int loc_mode, double *rec, unsigned long long *counters, void *stream);
+int exb_obs_solve_planned_qc_f32(void *plan, float *Ym, float *Yp, const double *ob_value, const double *ob_error,
+                                 const uint8_t *ob_assimilate, const double *ob_threshold, const double *obgeo, int64_t nobs,
+                                 int nens, int loc_mode, double *rec, unsigned long long *counters, void *stream);
+int exb_obs_solve_dist_qc_f64(void *plan, double *Ym, double *Yp, const double *ob_value, const double *ob_error,
+                              const uint8_t *ob_assimilate, const double *ob_threshold, const double *obgeo, int64_t nobs,
+                              int nens, int loc_mode, double *rec, unsigned long long *counters, int rank, int world,
+                              void *const *P_peers, void *const *S_peers, void *stream);
+int exb_obs_solve_dist_qc_f32(void *plan, float *Ym, float *Yp, const double *ob_value, const double *ob_error,
+                              const uint8_t *ob_assimilate, const double *ob_threshold, const double *obgeo, int64_t nobs,
+                              int nens, int loc_mode, double *rec, unsigned long long *counters, int rank, int world,
+                              void *const *P_peers, void *const *S_peers, void *stream);
+
 /* exb_obs_solve_* only enqueues its kernels (the dependency-driven variant synchronises the stream once, to size
  * its work lists, before the solve itself is launched).  Its kernels wait on each other inside the launch; a
  * watchdog (wall clock, EXB_WATCHDOG_S seconds without progress, default 20 + 1e-4 nobs) ends a wait that can never be
