@@ -13,7 +13,7 @@ from concurrent.futures import ThreadPoolExecutor
 CSRC = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'csrc')
 LIB = os.path.join(CSRC, 'libefa_xray_b200.so')
 SOURCES = ['api.cu', 'setup.cu', 'obs_solve.cu', 'state_update.cu', 'state_update_mma.cu',
-           'obs_solve_persistent.cu', 'obs_solve_dag.cu', 'state_sweep_2p.cu', 'relax.cu']
+           'obs_solve_persistent.cu', 'obs_solve_dag.cu', 'state_sweep_2p.cu', 'relax.cu', 'interp.cu']
 NVCC_FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-O3', '-lineinfo', '-std=c++17',
               '-Xcompiler', '-fPIC', '--expt-relaxed-constexpr']
 

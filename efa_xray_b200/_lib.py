@@ -24,6 +24,8 @@ SIGNATURES = {
     'exb_stencil_search': [_p, _p, _p, _p, _i64, _p, _p, _p, _p, _i64, _p, _p, _p, _p],
     'exb_stencil_search_rect': [_p, _p, _p, _p, _i64, _i64, _p, _p, _p, _p, _i64, _p, _p, _p, _p],
     'exb_pseudo_distance': [_p, _p, _i64, _dbl, _dbl, _p, _p],
+    'exb_stencil_bilinear_rect': [_p, _p, _i64, _i64, _int, _p, _p, _i64, _p, _p, _p, _p],
+    'exb_stencil_bilinear_curv': [_p, _p, _p, _i64, _i64, _p, _p, _i64, _p, _p, _p, _p],
     'exb_stencil_combine': [_p, _p, _p, _p, _p, _p, _i64, _i64, _i64, _i64, _i64, _int, _p, _p, _p],
     'exb_pool_trim': [C.c_uint64],
     'exb_gather_f64': [_p, _i64, _int, _p, _p, _int, _i64, _p, _p],

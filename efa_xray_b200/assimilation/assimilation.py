@@ -20,11 +20,17 @@ class ObTimeOutsideState(AttributeError, ValueError):
 class Assimilation():
     """Computes obs priors and formats the state for the update (assimilation.py:10-171)."""
 
-    def __init__(self, state, obs, nproc=1, inflation=None, verbose=False):
+    def __init__(self, state, obs, nproc=1, inflation=None, verbose=False, forward_operator='reference'):
         """inflation: None, a float (all variables), or a dict of {variable name: float} and/or
         {'validtime' | 'y' | 'x' (| 'lat' | 'lon' when 1-D): array along that dimension}
         (assimilation.py:19-26; the netCDF file-name form needs xarray and is not ported).
-        nproc is accepted and ignored, as in the reference (assimilation.py:31)."""
+        nproc is accepted and ignored, as in the reference (assimilation.py:31).
+        forward_operator (not in the reference): 'reference' (default), the reference's 4-point inverse-distance
+        operator with its time weights, or 'bilinear', bilinear in space on the grid cell that contains the ob and
+        linear in time with correctly oriented weights (DESIGN.md section 4.8; needs 2-D lat/lon).  An unknown name,
+        or 'bilinear' on a state with 1-D lat/lon, raises ValueError here, before any device work."""
+        engine.check_forward_operator(forward_operator, np.ndim(state['lat'].values))
+        self.forward_operator = forward_operator
         self.prior = state
         self.obs = obs
         self.verbose = verbose
@@ -71,7 +77,8 @@ class Assimilation():
         utimes = np.array([np.datetime64(t) for t in uniq], dtype='datetime64[ns]') if uniq else \
             np.zeros(0, dtype='datetime64[ns]')
         times = utimes[codes] if n else np.zeros(0, dtype='datetime64[ns]')
-        tlo, thi, wlo, whi, outside = engine.time_weights(st['validtime'].values, times)
+        tlo, thi, wlo, whi, outside = engine.time_weights(st['validtime'].values, times,
+                                                          swapped=self.forward_operator == 'reference')
         if outside.any():
             print("Interpolation is outside of time range in state!")
             raise ObTimeOutsideState("observation %d (time %s) is outside the state's valid times"
@@ -232,8 +239,11 @@ class Assimilation():
         obs = self._obs_arrays(engine.LOC_NONE)
         X = torch.from_numpy(self._host_matrix()).to(dev)
         grid = self.prior._grid_tables()
-        Y, nex = engine.ob_priors(X, grid, obs, engine._sfx(X.dtype))
-        self._check_exact(int(nex.item()))
+        Y, nex = engine.ob_priors(X, grid, obs, engine._sfx(X.dtype), forward_operator=self.forward_operator)
+        if self.forward_operator == 'bilinear':
+            self._check_outside(int(nex.item()))
+        else:
+            self._check_exact(int(nex.item()))
         Ym = torch.empty(obs.nobs, dtype=X.dtype, device=dev)
         sfx = engine._sfx(X.dtype)
         _lib.call('exb_split_mean_pert_' + sfx, _lib.ptr(Y), _lib.ptr(Ym), obs.nobs, X.shape[1], _lib.stream_ptr())
@@ -245,6 +255,12 @@ class Assimilation():
             raise IndexError('%d observation(s) lie within 1 km of a grid point: the reference raises here '
                              '(state/ensemble.py:195-196); set efa_xray_b200.EXACT_MATCH_POLICY = "nearest" '
                              'to use the nearest point instead' % n_exact)
+
+    @staticmethod
+    def _check_outside(n_outside):
+        if n_outside > 0:
+            raise ValueError("%d observation(s) lie outside the grid, where forward_operator='bilinear' has no cell "
+                             "to interpolate from (DESIGN.md section 4.8)" % n_outside)
 
     def _apply_inflation(self, fac):
         import ctypes as C
@@ -308,14 +324,15 @@ class Assimilation():
         return post_state, self.obs
 
 
-def update(prior_state, obs, inflate=None, loc=False, nproc=1, verbose=False, relaxation=None, outlier_threshold=None):
+def update(prior_state, obs, inflate=None, loc=False, nproc=1, verbose=False, relaxation=None, outlier_threshold=None,
+           forward_operator='reference'):
     """Module-level entry point (assimilation.py:176-222).  In the reference this calls an undefined
     enkf_update; here it runs the EnSRF.  nproc is accepted for signature compatibility: the GPU path does
-    not fork worker processes.  relaxation: posterior relaxation, outlier_threshold: outlier quality control, both as
-    for EnSRF."""
+    not fork worker processes.  relaxation: posterior relaxation, outlier_threshold: outlier quality control,
+    forward_operator: the forward operator H, all as for EnSRF."""
     from .ensrf import EnSRF
     return EnSRF(prior_state, obs, nproc=nproc, inflation=inflate, verbose=verbose, loc=loc,
-                 relaxation=relaxation, outlier_threshold=outlier_threshold).update()
+                 relaxation=relaxation, outlier_threshold=outlier_threshold, forward_operator=forward_operator).update()
 
 
 def randomize_obs_order(obs, seed=None):

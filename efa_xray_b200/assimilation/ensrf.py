@@ -11,7 +11,7 @@ from .. import engine
 
 class EnSRF(Assimilation):
     """EnSRF(state, obs, nproc=1, inflation=None, verbose=True, loc=False, relaxation=None,
-    outlier_threshold=None).update() -> (post_state, obs).
+    outlier_threshold=None, forward_operator='reference').update() -> (post_state, obs).
 
     Same contract as the reference (ensrf.py:28-33, assimilation.py:171): `obs` is the caller's list,
     mutated in place with prior_mean / prior_var / post_mean / post_var / assimilated (ensrf.py:66-70,
@@ -43,11 +43,19 @@ class EnSRF(Assimilation):
     False, and neither the state nor any later ob's prior feels it.  assimilate_this itself is left alone.  Invalid
     values raise ValueError here, before any device work.  (A check against the priors before the loop needs no
     library support: compute_ob_priors and assimilate_this.)
+
+    `forward_operator` (not in the reference) selects the forward operator H (DESIGN.md section 4.8):
+      'reference'          the reference's operator: inverse-distance weights on 4 points under its pseudo-metric,
+                           with its time weights (default; EXACT_MATCH_POLICY applies)
+      'bilinear'           bilinear in space on the grid cell that contains the ob, linear in time with correctly
+                           oriented weights; needs 2-D lat/lon.  An ob outside the grid raises ValueError in
+                           update(), before any ob attribute is written and before the posterior is built.
+    An unknown name, or 'bilinear' on a state with 1-D lat/lon, raises ValueError here, before any device work.
     """
 
     def __init__(self, state, obs, nproc=1, inflation=None, verbose=True, loc=False, dtype='f64', relaxation=None,
-                 outlier_threshold=None):
-        Assimilation.__init__(self, state, obs, nproc, inflation, verbose)
+                 outlier_threshold=None, forward_operator='reference'):
+        Assimilation.__init__(self, state, obs, nproc, inflation, verbose, forward_operator=forward_operator)
         self.loc = loc
         self.dtype = dtype
         self._validate_relaxation(relaxation)
@@ -89,8 +97,10 @@ class EnSRF(Assimilation):
             host = np.array(st.to_vect(), order='C', copy=True)
             out_blk, owner, out = None, None, host
         res = engine.analysis_host(host, nlev, None, None, obs, loc_mode, device=dev, dtype=tdtype,
-                                   grid=st._grid_tables(), out=out, relaxation=self._relaxation_levels(self.relaxation))
+                                   grid=st._grid_tables(), out=out, relaxation=self._relaxation_levels(self.relaxation),
+                                   forward_operator=self.forward_operator)
         self._check_exact(res.n_exact)
+        self._check_outside(res.n_outside)
         self.last_result = res
 
         # per-ob diagnostics back onto the caller's objects (ensrf.py:66-76, :144-149)

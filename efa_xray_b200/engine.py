@@ -55,16 +55,19 @@ class AnalysisResult:
     post_var: np.ndarray
     assimilated: np.ndarray      # bool
     n_exact: int = 0             # obs within 1 km of a selected grid point
+    n_outside: int = 0           # obs outside the grid (forward_operator='bilinear')
     state_pairs: int = 0         # sum_k |F_s(k)|   (state rows with non-zero weight, all levels)
     obs_pairs: int = 0           # sum_k |F_o(k)|
     obs_solve: str = ''          # which obs-space solve ran: 'replicated' | 'distributed(block=b)' | 'single'
     ms: dict = field(default_factory=dict)
 
 
-def time_weights(valid_times, ob_times):
+def time_weights(valid_times, ob_times, swapped=True):
     """Vectorised restatement of the time-weight logic of EnsembleState.interpolate
     (state/ensemble.py:202-224), including its swapped linear weights.  Returns
-    (tlo, thi, wlo, whi, outside) with weights attached to time indices tlo = lastdex-1, thi = lastdex."""
+    (tlo, thi, wlo, whi, outside) with weights attached to time indices tlo = lastdex-1, thi = lastdex.
+    swapped=False gives the correctly oriented linear weights of forward_operator='bilinear':
+    whi = (t - t_lo) / (t_hi - t_lo)."""
     valids = np.asarray(valid_times).astype('datetime64[ns]')
     t = np.asarray(ob_times).astype('datetime64[ns]')
     outside = (t < valids[0]) | (t > valids[-1])
@@ -73,12 +76,57 @@ def time_weights(valid_times, ob_times):
     exact = valids[lastdex] == t
     lo = np.maximum(lastdex - 1, 0)
     totsec = np.abs((valids[lastdex] - valids[lo]) / np.timedelta64(1, 's'))
-    thissec = np.abs((t - valids[lastdex]) / np.timedelta64(1, 's'))
+    if swapped:
+        thissec = np.abs((t - valids[lastdex]) / np.timedelta64(1, 's'))
+    else:
+        thissec = np.abs((t - valids[lo]) / np.timedelta64(1, 's'))
     with np.errstate(divide='ignore', invalid='ignore'):
         frac = thissec.astype(np.float64) / totsec
     whi = np.where(exact, 1.0, frac)                              # timeweights[lastdex]
     wlo = np.where(exact, 0.0, 1.0 - frac)                        # timeweights[lastdex-1]
     return lo.astype(np.int64), lastdex.astype(np.int64), wlo, whi, outside
+
+
+FORWARD_OPERATORS = ('reference', 'bilinear')
+
+
+def check_forward_operator(forward_operator, lat_ndim):
+    """Raise ValueError unless forward_operator is one of FORWARD_OPERATORS and usable on a state whose lat/lon
+    coordinates have `lat_ndim` dimensions ('bilinear' needs 2-D lat/lon)."""
+    if not isinstance(forward_operator, str) or forward_operator not in FORWARD_OPERATORS:
+        raise ValueError('forward_operator must be one of %r, got %r' % (FORWARD_OPERATORS, forward_operator))
+    if forward_operator == 'bilinear' and lat_ndim != 2:
+        raise ValueError("forward_operator='bilinear' needs 2-D lat(y, x) / lon(y, x) coordinates; this state's "
+                         "lat/lon are %d-D" % lat_ndim)
+
+
+def bilinear_axes(lat2d, lon2d):
+    """Which path of the bilinear forward operator serves a 2-D grid (DESIGN.md section 4.8), pure numpy:
+    ('rect', lat_y, lon_unwrapped, periodic) when lat depends on y only and is strictly monotone, and lon depends on x
+    only and is strictly increasing after unwrapping (steps d_i = (lon_x[i+1] - lon_x[i]) mod 360 in (0, 360), span
+    S = sum d_i below 360); periodic when the wrap gap 360 - S is at most max d_i (1 + 1e-9).  Otherwise
+    ('curv', None, None, False)."""
+    lat2d = np.asarray(lat2d, dtype=np.float64)
+    lon2d = np.asarray(lon2d, dtype=np.float64)
+    if lat2d.ndim != 2 or lat2d.shape != lon2d.shape:
+        raise ValueError('the bilinear forward operator needs 2-D lat(y, x) / lon(y, x) of one shape, got %r and %r'
+                         % (lat2d.shape, lon2d.shape))
+    if lat2d.shape[0] < 2 or lat2d.shape[1] < 2:
+        raise ValueError('the bilinear forward operator needs at least 2 x 2 grid points, got %r' % (lat2d.shape,))
+    curv = ('curv', None, None, False)
+    if not ((lat2d == lat2d[:, :1]).all() and (lon2d == lon2d[:1, :]).all()):
+        return curv
+    lat_y, lon_x = lat2d[:, 0], lon2d[0, :]
+    dlat = np.diff(lat_y)
+    if not ((dlat > 0).all() or (dlat < 0).all()):
+        return curv
+    d = np.mod(np.diff(lon_x), 360.0)
+    span = float(np.sum(d))
+    if not ((d > 0).all() and (d < 360.0).all() and span < 360.0):
+        return curv
+    lon_u = lon_x[0] + np.concatenate(([0.0], np.cumsum(d)))
+    periodic = bool(360.0 - span <= d.max() * (1.0 + 1e-9))
+    return 'rect', np.ascontiguousarray(lat_y), lon_u, periodic
 
 
 def _torch():
@@ -136,6 +184,43 @@ class GridTables:
         self.u = torch.empty((3, self.npts), dtype=torch.float64, device=device)
         _lib.call('exb_grid_unitvec', _lib.ptr(self.lat), _lib.ptr(self.lon), self.npts, _lib.ptr(self.u),
                   _lib.stream_ptr())
+        self._host_latlon = None if self.diag else (lat2d, lon2d)
+        self._bilinear = None
+
+    def bilinear_tables(self):
+        """(path, device tables) of the bilinear forward operator, built on first use: ('rect', (lat_y,
+        unwrapped lon_x, periodic)) or ('curv', None), from bilinear_axes."""
+        if self._bilinear is None:
+            if self.diag:
+                raise ValueError("forward_operator='bilinear' needs 2-D lat(y, x) / lon(y, x) coordinates")
+            kind, lat_y, lon_u, periodic = bilinear_axes(*self._host_latlon)
+            tables = (_dev_f64(lat_y, self.device), _dev_f64(lon_u, self.device), int(periodic)) \
+                if kind == 'rect' else None
+            self._bilinear = (kind, tables)
+        return self._bilinear
+
+
+def stencil_bilinear(grid: GridTables, d_lat, d_lon, force_curvilinear=False):
+    """Bilinear stencils (DESIGN.md section 4.8) of the obs at device coordinates d_lat / d_lon -> device tensors
+    idx4 [nobs,4] int64, w4 [nobs,4] float64 and the int32 count of obs outside the grid (idx 0 / w 0 there).
+    force_curvilinear runs the curvilinear path on any 2-D grid."""
+    torch = _torch()
+    dev = grid.device
+    kind, tables = grid.bilinear_tables()
+    nobs = d_lat.shape[0]
+    idx4 = torch.empty((nobs, 4), dtype=torch.int64, device=dev)
+    w4 = torch.empty((nobs, 4), dtype=torch.float64, device=dev)
+    nout = torch.empty(1, dtype=torch.int32, device=dev)
+    if kind == 'rect' and not force_curvilinear:
+        lat_y, lon_u, periodic = tables
+        _lib.call('exb_stencil_bilinear_rect', _lib.ptr(lat_y), _lib.ptr(lon_u), grid.ny, grid.nx, periodic,
+                  _lib.ptr(d_lat), _lib.ptr(d_lon), nobs, _lib.ptr(idx4), _lib.ptr(w4), _lib.ptr(nout),
+                  _lib.stream_ptr())
+    else:
+        _lib.call('exb_stencil_bilinear_curv', _lib.ptr(grid.u), _lib.ptr(grid.lat), _lib.ptr(grid.lon), grid.ny,
+                  grid.nx, _lib.ptr(d_lat), _lib.ptr(d_lon), nobs, _lib.ptr(idx4), _lib.ptr(w4), _lib.ptr(nout),
+                  _lib.stream_ptr())
+    return idx4, w4, nout
 
 
 def stencil_search(grid: GridTables, ob_lat, ob_lon, force_general=False, dev_tables=None):
@@ -184,8 +269,12 @@ def pseudo_distance_order(grid: GridTables, lat, lon, npt):
     return order.cpu().numpy()
 
 
-def ob_priors(X, grid: GridTables, obs: ObsArrays, sfx, nlev=None, band=None, group=None, obs_dev=None):
-    """Y[nobs, nens] = H X for all obs (compute_ob_priors, assimilation/assimilation.py:36-49).
+def ob_priors(X, grid: GridTables, obs: ObsArrays, sfx, nlev=None, band=None, group=None, obs_dev=None,
+              forward_operator='reference'):
+    """(Y[nobs, nens] = H X for all obs, device int32 counter) (compute_ob_priors, assimilation/assimilation.py:36-49).
+    The counter is the number of obs within 1 km of a selected grid point for forward_operator='reference', and the
+    number of obs outside the grid for 'bilinear' (DESIGN.md section 4.8; their rows of Y are 0).  The caller picks
+    the time weights (obs.tw0 / tw1) that go with the operator.
 
     X may also be a PINNED host tensor: the gather kernel then reads the <= 8 stencil rows per ob straight from
     host memory over PCIe (unified addressing), which lets the obs-space solve start while the state is still
@@ -196,14 +285,18 @@ def ob_priors(X, grid: GridTables, obs: ObsArrays, sfx, nlev=None, band=None, gr
     obs_dev: the device copies of the per-ob tables made by upload_obs (saves re-uploading them)."""
     torch = _torch()
     dev = grid.device
+    check_forward_operator(forward_operator, 1 if grid.diag else 2)
     if obs_dev is None or 'row0' not in obs_dev:
         obs_dev = {'lat': _dev_f64(obs.lat, dev), 'lon': _dev_f64(obs.lon, dev),
                    'sinlat': _dev_f64(np.sin(np.radians(obs.lat)), dev), 'coslon': _dev_f64(np.cos(np.radians(obs.lon)), dev),
                    'row0': torch.as_tensor(np.ascontiguousarray(obs.row0, dtype=np.int64)).to(dev),
                    'row1': torch.as_tensor(np.ascontiguousarray(obs.row1, dtype=np.int64)).to(dev),
                    'tw0': _dev_f64(obs.tw0, dev), 'tw1': _dev_f64(obs.tw1, dev)}
-    tables = (obs_dev['lat'], obs_dev['lon'], obs_dev['sinlat'], obs_dev['coslon'])
-    idx4, w4, nex = stencil_search(grid, None, None, dev_tables=tables)
+    if forward_operator == 'bilinear':
+        idx4, w4, nex = stencil_bilinear(grid, obs_dev['lat'], obs_dev['lon'])
+    else:
+        tables = (obs_dev['lat'], obs_dev['lon'], obs_dev['sinlat'], obs_dev['coslon'])
+        idx4, w4, nex = stencil_search(grid, None, None, dev_tables=tables)
     # 8-point stencil = 4 space points x 2 time levels, re-based to the band's shard (index/weight bookkeeping only)
     y0, y1 = band if band is not None else (0, grid.ny)
     idx8 = torch.empty((obs.nobs, 8), dtype=torch.int64, device=dev)
@@ -605,7 +698,7 @@ def upload_obs(obs: ObsArrays, device, loc_mode):
 
 def analysis_device(X, nlev, grid: GridTables, obs: ObsArrays, loc_mode, inflation=None, timing=True,
                     band=None, group=None, Y=None, sweep_bands=None, on_band_done=None, before_band=None,
-                    obs_device=None, relaxation=None):
+                    obs_device=None, relaxation=None, forward_operator='reference'):
     """Serial EnSRF analysis of a device-resident ensemble, in place.
 
     X        torch tensor [nlev*ny*nx, nens] (float64 or float32) on a CUDA device, to_vect layout
@@ -620,6 +713,9 @@ def analysis_device(X, nlev, grid: GridTables, obs: ObsArrays, loc_mode, inflati
     obs.threshold  empty (no check), or outlier thresholds per ob: the obs-space solve rejects an ob whose innovation exceeds
              its threshold times sqrt(prior variance + error) inside the serial loop (DESIGN.md section 4.7);
              rejected obs come back with assimilated False, and the state sweep applies a zero update for them.
+    forward_operator  'reference' (the reference's 4-point inverse-distance operator) or 'bilinear' (DESIGN.md
+             section 4.8; obs.tw0 / tw1 must then be the weights of time_weights(swapped=False)).  With 'bilinear',
+             res.n_outside counts the obs outside the grid: their priors are 0, so callers reject such a result.
     sweep_bands  optional list of (ya, yb) row ranges of the shard: the fused sweep is issued range by range and
              on_band_done(ya, yb) is called after each launch has been enqueued (e.g. to start its download),
              before_band(ya, yb) before it (e.g. to wait for its upload).
@@ -671,8 +767,9 @@ def analysis_device(X, nlev, grid: GridTables, obs: ObsArrays, loc_mode, inflati
             fused = fused_sweep_available(X.dtype, nens)
             grid_u = grid.u if band is None else grid.u[:, y0 * nx:y1 * nx].contiguous()
             if Y is None:
-                Yp, nex = ob_priors(X, grid, obs, sfx, nlev=nlev, band=band, group=group, obs_dev=obs_dev)
-            elif isinstance(Y, tuple):   # (H.x, n_exact) from ob_priors, owned by this call
+                Yp, nex = ob_priors(X, grid, obs, sfx, nlev=nlev, band=band, group=group, obs_dev=obs_dev,
+                                    forward_operator=forward_operator)
+            elif isinstance(Y, tuple):   # (H.x, counter) from ob_priors, owned by this call
                 Yp, nex = Y
             else:       # ob priors H.x computed by the caller (e.g. before the state was scattered)
                 Yp, nex = Y.clone(), torch.zeros(1, dtype=torch.int32, device=dev)
@@ -739,8 +836,10 @@ def analysis_device(X, nlev, grid: GridTables, obs: ObsArrays, loc_mode, inflati
     ms = tm.result()
     if relax is not None and timing:
         ms['relax'] = relax.ms()
+    bilinear = forward_operator == 'bilinear'
     return AnalysisResult(prior_mean=rec_h[0], prior_var=rec_h[1], post_mean=rec_h[2], post_var=rec_h[3],
-                          assimilated=rec_h[7] != 0.0, n_exact=nex_h, state_pairs=int(cnt[1]) * nlev,
+                          assimilated=rec_h[7] != 0.0, n_exact=0 if bilinear else nex_h,
+                          n_outside=nex_h if bilinear else 0, state_pairs=int(cnt[1]) * nlev,
                           obs_pairs=int(cnt[0]), ms=ms, obs_solve=which)
 
 
@@ -765,7 +864,8 @@ def sweep_band_schedule(nlev, ny, nx, nbands=None):
 
 
 def analysis_host(X_host, nlev, lat2d, lon2d, obs: ObsArrays, loc_mode, inflation=None, device='cuda:0',
-                  dtype=None, grid=None, out=None, pipeline=True, band=None, group=None, relaxation=None):
+                  dtype=None, grid=None, out=None, pipeline=True, band=None, group=None, relaxation=None,
+                  forward_operator='reference'):
     """Host-buffer entry: X_host is a numpy array or CPU torch tensor [nlev*ny*nx, nens]; it is uploaded,
     analysed on `device`, and the analysis is written to `out` (default: back into X_host).  Pinned host
     memory makes the copies asynchronous.  With the fused float64 sweep (and pipeline=True) the state is swept
@@ -780,7 +880,7 @@ def analysis_host(X_host, nlev, lat2d, lon2d, obs: ObsArrays, loc_mode, inflatio
     res.obs_solve) and no other data crosses between ranks.
 
     relaxation: as for analysis_device; with the band pipeline each band is relaxed between its sweep and its
-    download."""
+    download.  forward_operator: as for analysis_device."""
     torch = _torch()
     _lib.require_device()
     Xh = X_host if isinstance(X_host, torch.Tensor) else torch.from_numpy(X_host)
@@ -814,7 +914,8 @@ def analysis_host(X_host, nlev, lat2d, lon2d, obs: ObsArrays, loc_mode, inflatio
             if inflation is None and Xh.is_pinned():
                 # PCIe is used by one thing at a time: first the gather (25 % of the state in 800-byte pieces),
                 # then the band uploads, which overlap the obs-space solve and the sweep of earlier bands
-                Y = ob_priors(Xh, grid, obs, _sfx(xdtype), nlev=nlev, band=band, group=group, obs_dev=obs_device[0])
+                Y = ob_priors(Xh, grid, obs, _sfx(xdtype), nlev=nlev, band=band, group=group, obs_dev=obs_device[0],
+                              forward_operator=forward_operator)
             arrived = {}
             copy_in.wait_stream(main)
             with torch.cuda.stream(copy_in):
@@ -842,7 +943,7 @@ def analysis_host(X_host, nlev, lat2d, lon2d, obs: ObsArrays, loc_mode, inflatio
 
             res = analysis_device(X, nlev, grid, obs, loc_mode, inflation, Y=Y, sweep_bands=bands, band=band, group=group,
                                   before_band=wait_upload, on_band_done=download, obs_device=obs_device,
-                                  relaxation=relaxation)
+                                  relaxation=relaxation, forward_operator=forward_operator)
             ev[2].record()
             main.wait_stream(copy_out)
             ev[3].record()
@@ -854,7 +955,8 @@ def analysis_host(X_host, nlev, lat2d, lon2d, obs: ObsArrays, loc_mode, inflatio
             if dtype is not None and X.dtype != dtype:
                 X = X.to(dtype)
             ev[1].record()
-            res = analysis_device(X, nlev, grid, obs, loc_mode, inflation, band=band, group=group, relaxation=relaxation)
+            res = analysis_device(X, nlev, grid, obs, loc_mode, inflation, band=band, group=group, relaxation=relaxation,
+                                  forward_operator=forward_operator)
             ev[2].record()
             Oh.copy_(X.to(Oh.dtype) if X.dtype != Oh.dtype else X, non_blocking=True)
             ev[3].record()

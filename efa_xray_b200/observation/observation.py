@@ -34,9 +34,10 @@ class Observation:
         self.description = description
         self.localize_radius = localize_radius
 
-    def estimate(self, state):
-        """Ensemble estimate of this observation: the state interpolated to the ob (observation.py:40-50)."""
-        return state.interpolate(self.obtype, self.time, self.lat, self.lon)
+    def estimate(self, state, forward_operator='reference'):
+        """Ensemble estimate of this observation: the state interpolated to the ob (observation.py:40-50), with the
+        forward operator of EnsembleState.interpolate."""
+        return state.interpolate(self.obtype, self.time, self.lat, self.lon, forward_operator=forward_operator)
 
     def distance_to_state(self, state):
         """Distance in km from this ob to every grid point (observation.py:53-56)."""

@@ -15,22 +15,23 @@ COLUMNS = ['validtime', 'flead', 'lat', 'lon', 'obtype', 'description', 'ob erro
            'prior mean', 'post mean', 'prior variance', 'post variance']
 
 
-def ob_estimates(state, obs):
+def ob_estimates(state, obs, forward_operator='reference'):
     """[Nobs, Nens] ensemble estimates of every ob (Observation.estimate, observation.py:40-50, for all obs at once)
-    computed on the device."""
-    a = Assimilation(state, obs, verbose=False)
+    computed on the device, with the forward operator of Assimilation (DESIGN.md section 4.8)."""
+    a = Assimilation(state, obs, verbose=False, forward_operator=forward_operator)
     means, perts = a.compute_ob_priors()
     return perts + means[:, None]
 
 
-def obs_assimilation_statistics(prior, post, obs):
+def obs_assimilation_statistics(prior, post, obs, forward_operator='reference'):
     """Builds a pandas dataframe with statistical info about the observations (postprocess.py:8-39):
-    prior/post mean and variance (numpy .var(), ddof 0) of the ensemble estimate of every ob, plus its metadata."""
+    prior/post mean and variance (numpy .var(), ddof 0) of the ensemble estimate of every ob, plus its metadata.
+    Pass the analysis's forward_operator so that the estimates use its H."""
     import pandas as pd
     assert isinstance(prior, EnsembleState)
     assert isinstance(post, EnsembleState)
-    prior_ye = ob_estimates(prior, obs)
-    post_ye = ob_estimates(post, obs)
+    prior_ye = ob_estimates(prior, obs, forward_operator)
+    post_ye = ob_estimates(post, obs, forward_operator)
     t0 = pd.to_datetime(prior['validtime'].values[0])
     oblist = []
     for k, ob in enumerate(obs):

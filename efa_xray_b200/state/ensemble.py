@@ -457,12 +457,17 @@ class EnsembleState(_LabelledDataset):
             flat = idx4.cpu().numpy()[0, :npt]
         return np.unravel_index(flat, self['lat'].shape)
 
-    def interpolate(self, var, time, lat, lon):
+    def interpolate(self, var, time, lat, lon, forward_operator='reference'):
         """Ensemble estimate [nmems] of `var` at (time, lat, lon): 4-point inverse-distance weights in
-        space x linear weights in time (ensemble.py:170-239, weights as the reference computes them)."""
-        from ..engine import ObsArrays, ob_priors, time_weights
+        space x linear weights in time (ensemble.py:170-239, weights as the reference computes them).
+        forward_operator='bilinear' (2-D lat/lon only) interpolates bilinearly on the grid cell that contains the
+        point and linearly in time with correctly oriented weights (DESIGN.md section 4.8); a point outside the grid
+        raises ValueError."""
+        from ..engine import ObsArrays, ob_priors, time_weights, check_forward_operator
         import torch
-        tlo, thi, wlo, whi, outside = time_weights(self['validtime'].values, np.array([np.datetime64(time)]))
+        check_forward_operator(forward_operator, np.ndim(self['lat'].values))
+        tlo, thi, wlo, whi, outside = time_weights(self['validtime'].values, np.array([np.datetime64(time)]),
+                                                   swapped=forward_operator == 'reference')
         if outside[0]:
             print("Interpolation is outside of time range in state!")
             return None
@@ -474,8 +479,12 @@ class EnsembleState(_LabelledDataset):
                         lon=np.array([lon], dtype=np.float64), halfwidth=np.ones(1),
                         assimilate=np.zeros(1, dtype=np.uint8), row0=tlo * ny * nx, row1=thi * ny * nx,
                         tw0=wlo, tw1=whi)
-        Y, nex = ob_priors(X, grid, obs, 'f64' if X.dtype == torch.float64 else 'f32')
-        if int(nex.item()) > 0 and _pkg.EXACT_MATCH_POLICY == 'raise':
+        Y, nex = ob_priors(X, grid, obs, 'f64' if X.dtype == torch.float64 else 'f32', forward_operator=forward_operator)
+        if forward_operator == 'bilinear':
+            if int(nex.item()) > 0:
+                raise ValueError('(%r, %r) lies outside the grid: the bilinear forward operator has no cell to '
+                                 'interpolate from' % (lat, lon))
+        elif int(nex.item()) > 0 and _pkg.EXACT_MATCH_POLICY == 'raise':
             raise IndexError('observation within 1 km of a grid point: the reference raises here '
                              '(state/ensemble.py:195-196); set efa_xray_b200.EXACT_MATCH_POLICY = "nearest" '
                              'to use the nearest point instead')

@@ -111,6 +111,30 @@ int exb_stencil_search_rect(const double *sinlat_y, const double *coslon_x, cons
                             const double *ob_coslon, const double *ob_lat_deg, const double *ob_lon_deg,
                             int64_t nobs, int64_t *idx4, double *w4, int32_t *n_exact, void *stream);
 
+/* Bilinear forward operator (DESIGN.md section 4.8), the opt-in alternative to exb_stencil_search*: for every ob the
+ * 4 corners of the grid cell that contains it, in the order (j,i), (j,i+1), (j+1,i), (j+1,i+1), with the weights
+ * (1-s)(1-t), s(1-t), (1-s)t, st.  idx4 is int64[nobs][4] (flat y*nx+x), w4 double[nobs][4], as
+ * exb_stencil_combine consumes them.  An ob outside the grid gets idx 0 / weight 0 and is counted in n_outside
+ * (device int32[1], required; zeroed on the stream first).
+ *
+ * RECTILINEAR grids: lat_y_deg[ny] strictly monotone (either direction); lon_x_unwrapped[nx] strictly increasing
+ * with a span below 360 degrees.  The ob longitude is taken to L0 + ((lon - L0) mod 360), L0 = lon_x_unwrapped[0].
+ * periodic = 1 adds the closing cell between column nx-1 and column 0 (right edge L0 + 360).  One thread per ob,
+ * binary search on each axis; s and t are linear in degrees. */
+int exb_stencil_bilinear_rect(const double *lat_y_deg, const double *lon_x_unwrapped, int64_t ny, int64_t nx,
+                              int periodic, const double *ob_lat_deg, const double *ob_lon_deg, int64_t nobs,
+                              int64_t *idx4, double *w4, int32_t *n_outside, void *stream);
+
+/* CURVILINEAR grids (2-D lat/lon, e.g. rotated-pole or Lambert-conformal regional grids): the nearest grid point p*
+ * by great-circle distance (largest dot product with grid_u[3][ny*nx] of exb_grid_unitvec; ties: lowest flat index),
+ * then the cells that have p* as a corner, then the rest of the 4x4-cell block around p*, row-major by lower-left
+ * index.  A cell contains the ob when its inverse bilinear coordinates, computed in the (lat, lon) plane with corner
+ * longitudes unwrapped to within 180 degrees of the ob's, lie in [-1e-10, 1 + 1e-10]; they are clamped to [0, 1].
+ * The grid never wraps; cells that contain a pole are not supported. */
+int exb_stencil_bilinear_curv(const double *grid_u, const double *lat_g_deg, const double *lon_g_deg, int64_t ny,
+                              int64_t nx, const double *ob_lat_deg, const double *ob_lon_deg, int64_t nobs,
+                              int64_t *idx4, double *w4, int32_t *n_outside, void *stream);
+
 /* 8-point stencils of the full forward operator: the 4 space points at the two bracketing time levels with the
  * products of space and time weights (state/ensemble.py:202-237).  row0/row1 = first state row of the ob's variable
  * at its lower / upper time level, tw0/tw1 the time weights.  idx8 are row indices into a shard that holds grid rows
