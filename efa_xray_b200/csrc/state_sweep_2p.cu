@@ -67,7 +67,6 @@ struct S2Params {
     int G, Lc, nlc;
     int loc_mode;
     int nstages, stage_doubles, blk_doubles, npatches;
-    int cand_cap;                     // candidates per chunk (<= S2_CAND): bounds the part of the scratch area in use
     ExbLocConst kloc;                 // constants of the localisation weight (parameter block = constant bank)
 };
 
@@ -317,7 +316,7 @@ __global__ void __launch_bounds__(S2_NW * 32, 1) state_sweep_2p_kernel(const S2P
         for (;;) {
             // =============================== PHASE A (1): candidates of this chunk ===============================
             int ncand = 0;
-            while (pos < le && ncand + SCAN <= p.cand_cap) {
+            while (pos < le && ncand + SCAN <= S2_CAND) {
                 const int64_t e0 = pos + 2 * tid;
                 int i0 = -1, i1 = -1;
                 if (e0 < le) i0 = list ? __ldg(list + e0) : (int)e0;
@@ -853,8 +852,7 @@ __global__ void __launch_bounds__(1024) sweep_scan_kernel(const int *__restrict_
 // host side: candidate lists per coarse tile
 // ------------------------------------------------------------------------------------------
 static bool sweep_lists_wanted(int loc_mode, int64_t ob_begin, int64_t ob_end) {
-    const char *nolist = getenv("EXB_SWEEP_NOLIST");
-    return loc_mode == EXB_LOC_GC && !(nolist && atoi(nolist)) && ob_end - ob_begin > 4096;
+    return loc_mode == EXB_LOC_GC && ob_end - ob_begin > 4096;
 }
 
 // Builds, for every coarse tile (SP_CT x SP_CT patches of bty x btx grid points) that intersects grid rows
@@ -996,8 +994,6 @@ static int s2_launch(S2Params &p, const TS *Yp, cudaStream_t st, const ExbSweepP
             else prof = nullptr;
         }
         p.prof = prof;
-        p.cand_cap = S2_CAND;
-        if (const char *e = getenv("EXB_S2_CAP")) { const int v = atoi(e); if (v >= 2 * NTH && v <= S2_CAND) p.cand_cap = v; }
         state_sweep_2p_kernel<NT3, LK, TS><<<(unsigned)grid, NTH, smem, st>>>(p);
         exb_count_launches(2);
         rc = exb_check_launch("state_sweep_2p_kernel");

@@ -16,8 +16,6 @@
 // Q obs in order to its row.
 #include "common.cuh"
 #include <type_traits>
-#include <cstring>
-#include <cstdlib>
 
 int exb_state_update_mma_f64(double *xm, double *Xp, int64_t nlev, int64_t ny, int64_t nx, int nens,
                              const double *grid_u, const double *Yp, const double *rec, const double *obgeo,
@@ -306,30 +304,14 @@ static int su_launch(SuParams &p, cudaStream_t st) {
     return exb_check_launch("state_update_kernel");
 }
 
-// (S, MC) instantiations; the host picks the one with the least padding for the ensemble size
-#define SU_FOR_EACH_VARIANT(F) \
-    F(2, 7) F(2, 13) F(2, 25) F(4, 7) F(4, 13) F(4, 25) F(8, 13) F(8, 25) F(8, 32)
-
+// Eight lanes per row; the host picks the smallest MC with 8 * MC >= nens.  The kernel serves ensembles above 103
+// members (state_update_impl), where 8 lanes per row keep MC at 32 or below up to EXB_MAX_NENS.
 template <typename T>
 static int su_dispatch(SuParams &p, cudaStream_t st) {
-    int bestS = 0, bestMC = 0;
-    double best = 1e30;
-#define SU_CONSIDER(S_, MC_)                                                              \
-    if (S_ * MC_ >= p.nens) {                                                             \
-        /* padded members, plus the cross-lane reduction and per-ob scalar work */        \
-        const double cost = (double)S_ * MC_ + S_ * (4.0 + 1.5 * (S_ == 2 ? 1 : S_ == 4 ? 2 : 3)); \
-        if (cost < best) { best = cost; bestS = S_; bestMC = MC_; }                       \
-    }
-    SU_FOR_EACH_VARIANT(SU_CONSIDER)
-#undef SU_CONSIDER
-    if (!bestS) {
-        exb_set_error("exb_state_update: no kernel variant for nens=%d (max %d)", p.nens, EXB_MAX_NENS);
-        return EXB_ERR_UNSUPPORTED;
-    }
-#define SU_LAUNCH(S_, MC_) \
-    if (bestS == S_ && bestMC == MC_) return su_launch<T, S_, MC_>(p, st);
-    SU_FOR_EACH_VARIANT(SU_LAUNCH)
-#undef SU_LAUNCH
+    if (p.nens <= 8 * 13) return su_launch<T, 8, 13>(p, st);
+    if (p.nens <= 8 * 25) return su_launch<T, 8, 25>(p, st);
+    if (p.nens <= 8 * 32) return su_launch<T, 8, 32>(p, st);
+    exb_set_error("exb_state_update: no kernel variant for nens=%d (max %d)", p.nens, EXB_MAX_NENS);
     return EXB_ERR_UNSUPPORTED;
 }
 
@@ -348,34 +330,23 @@ static int state_update_impl(T *xm, T *Xp, int64_t nlev, int64_t ny, int64_t nx,
     EXB_CUDA(exb_malloc_async(&scan, (size_t)nobs * sizeof(float4), st));
     su_scan_records_kernel<<<(unsigned)ceil_div64(nobs, 256), 256, 0, st>>>(obgeo, rec, nobs, scan);
     exb_count_launches(1);
-    {
-        // FP64 tensor-core sweeps (float32 states: float32 storage, float64 arithmetic in registers).
-        // EXB_SU_IMPL = pipe (default: two-phase, state_sweep_2p.cu) | mma (state_update_mma.cu, float64 only, also the
-        // fallback for ensembles > 103 members) | vector (the kernel below, arithmetic in T)
-        const char *impl = getenv("EXB_SU_IMPL");
-        const bool vec = impl && strcmp(impl, "vector") == 0, mma = impl && strcmp(impl, "mma") == 0;
-        if (!vec && !mma) {
-            int rc = exb_state_sweep_2p<T>(xm, Xp, nlev, ny, nx, nens, grid_u, Yp, rec, obgeo, scan, nobs, ob_begin, ob_end,
-                                           0, ny, loc_mode, counters, st);
-            if (rc != EXB_ERR_UNSUPPORTED) {
-                cudaFreeAsync(scan, st);
-                return rc;
-            }
-        }
-        if (!vec && std::is_same<T, double>::value) {
-            int rc = exb_state_update_mma_f64((double *)xm, (double *)Xp, nlev, ny, nx, nens, grid_u, (const double *)Yp,
-                                              rec, obgeo, scan, nobs, ob_begin, ob_end, loc_mode, counters, st);
-            if (rc != EXB_ERR_UNSUPPORTED) {
-                cudaFreeAsync(scan, st);
-                return rc;
-            }
-        }
+    // FP64 tensor-core sweeps (float32 states: float32 storage, float64 arithmetic in registers): the two-phase
+    // sweep (state_sweep_2p.cu) up to 103 members, then state_update_mma.cu for float64 up to 255 members
+    int rc = exb_state_sweep_2p<T>(xm, Xp, nlev, ny, nx, nens, grid_u, Yp, rec, obgeo, scan, nobs, ob_begin, ob_end,
+                                   0, ny, loc_mode, counters, st);
+    if (rc == EXB_ERR_UNSUPPORTED && std::is_same<T, double>::value)
+        rc = exb_state_update_mma_f64((double *)xm, (double *)Xp, nlev, ny, nx, nens, grid_u, (const double *)Yp,
+                                      rec, obgeo, scan, nobs, ob_begin, ob_end, loc_mode, counters, st);
+    if (rc != EXB_ERR_UNSUPPORTED) {
+        cudaFreeAsync(scan, st);
+        return rc;
     }
+    // the kernel above, arithmetic in T: float32 beyond 103 members, float64 at 256
     SuParams p;
     p.xm = xm; p.Xp = Xp; p.Yp = Yp; p.grid_u = grid_u; p.rec = rec; p.geo = obgeo; p.scan = scan;
     p.counters = counters; p.npts = ny * nx; p.nobs = nobs; p.ob_begin = ob_begin; p.ob_end = ob_end;
     p.nlev = (int)nlev; p.ny = (int)ny; p.nx = (int)nx; p.nens = nens; p.loc_mode = loc_mode;
-    int rc = su_dispatch<T>(p, st);
+    rc = su_dispatch<T>(p, st);
     cudaFreeAsync(scan, st);
     return rc;
 }

@@ -1,4 +1,4 @@
-// State sweep, FP64 tensor-core version (the production path for float64 states).
+// State sweep, FP64 tensor-core version: the float64 path for ensembles of 104 to 255 members.
 //
 // Same tile-stationary organisation as state_update.cu -- a CTA keeps a patch of grid points (all of
 // its levels, 64 state rows) in registers and walks the observations in serial order -- but the
@@ -56,8 +56,8 @@ template <int NT3> __host__ __device__ constexpr int sm_yst() { return ((8 * NT3
 // so that both access patterns (8 rows x 64 B and 4 rows x 32 B) are bank-conflict free
 __device__ __forceinline__ int sm_swz(int q, int m) { return m ^ (((q >> 1) & 1) << 2); }
 
-template <int NT3, int MINB>
-__global__ void __launch_bounds__(SM_NT, MINB)
+template <int NT3>
+__global__ void __launch_bounds__(SM_NT, 1)
 state_update_mma_kernel(const SmParams p) {
     constexpr int YST = sm_yst<NT3>();
 
@@ -360,7 +360,7 @@ state_update_mma_kernel(const SmParams p) {
     if (p.counters && npairs) atomicAdd(&p.counters[1], npairs);
 }
 
-template <int NT3, int MINB>
+template <int NT3>
 static int sm_launch(SmParams &p, cudaStream_t st) {
     constexpr int YST = sm_yst<NT3>();
     const int Lc = p.nlev < SM_ROWS ? p.nlev : SM_ROWS;
@@ -378,15 +378,16 @@ static int sm_launch(SmParams &p, cudaStream_t st) {
     const int nty = (p.ny + bty - 1) / bty;
     const size_t smem = sizeof(double) * ((size_t)SM_Q * YST + SM_ROWS * SM_Q + (SM_Q / 8) * 64 + 3 * SM_ROWS + 6 * SM_Q) +
                         sizeof(int) * (SM_Q + SM_NT + SM_ROWS + SM_NT / 32);
-    EXB_CUDA(cudaFuncSetAttribute(state_update_mma_kernel<NT3, MINB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    EXB_CUDA(cudaFuncSetAttribute(state_update_mma_kernel<NT3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     const int64_t nblocks = (int64_t)p.ntx * nty * p.nlc;
     EXB_REQUIRE(nblocks < 0x7fffffff, "too many patches for one launch");
-    state_update_mma_kernel<NT3, MINB><<<(unsigned)nblocks, SM_NT, smem, st>>>(p);
+    state_update_mma_kernel<NT3><<<(unsigned)nblocks, SM_NT, smem, st>>>(p);
     exb_count_launches(1);
     return exb_check_launch("state_update_mma_kernel");
 }
 
-// Called from state_update.cu for float64 states.  Returns EXB_ERR_UNSUPPORTED if no variant fits.
+// Called from state_update.cu for float64 ensembles the two-phase sweep does not take (more than 103 members).
+// Returns EXB_ERR_UNSUPPORTED if no variant fits (256 members need 33 tiles).
 int exb_state_update_mma_f64(double *xm, double *Xp, int64_t nlev, int64_t ny, int64_t nx, int nens,
                              const double *grid_u, const double *Yp, const double *rec, const double *obgeo,
                              const float4 *scan, int64_t nobs, int64_t ob_begin, int64_t ob_end, int loc_mode,
@@ -396,16 +397,11 @@ int exb_state_update_mma_f64(double *xm, double *Xp, int64_t nlev, int64_t ny, i
     p.counters = counters; p.npts = ny * nx; p.nobs = nobs; p.ob_begin = ob_begin; p.ob_end = ob_end;
     p.nlev = (int)nlev; p.ny = (int)ny; p.nx = (int)nx; p.nens = nens; p.loc_mode = loc_mode;
     const int need = (nens + 1 + 7) / 8;            // 8-member tiles incl. the pseudo-member
-#define SM_TRY(N, B) if (need <= N) return sm_launch<N, B>(p, st)
-    SM_TRY(2, 2);
-    SM_TRY(4, 2);
-    SM_TRY(7, 2);
-    SM_TRY(10, 2);
-    SM_TRY(13, 2);
-    SM_TRY(16, 1);
-    SM_TRY(20, 1);
-    SM_TRY(26, 1);
-    SM_TRY(32, 1);
+#define SM_TRY(N) if (need <= N) return sm_launch<N>(p, st)
+    SM_TRY(16);
+    SM_TRY(20);
+    SM_TRY(26);
+    SM_TRY(32);
 #undef SM_TRY
     return EXB_ERR_UNSUPPORTED;
 }

@@ -524,11 +524,6 @@ def obs_dist_block():
     return max(1, int(os.environ.get('EXB_OBS_DIST_BLOCK', '256')))
 
 
-def sweep_plan_wanted():
-    import os
-    return os.environ.get('EXB_SWEEP_PLAN', '1') != '0'
-
-
 def obs_plan_wanted(loc_mode):
     import os
     return loc_mode == LOC_GC and os.environ.get('EXB_OBS_IMPL', 'dag') == 'dag'
@@ -554,14 +549,15 @@ def state_sweep_fused(X, nlev, ny, nx, grid_u, Yp, rec, geo, nobs, loc_mode, cou
               ny if y_end is None else y_end, loc_mode, _lib.ptr(counters), _lib.stream_ptr())
 
 
-def fused_sweep_available(dtype, nens):
-    """The fused kernel exists for float64 and float32 (storage) ensembles of up to 103 members; EXB_FUSED=0 or EXB_SU_IMPL=mma|vector
-    select the three-call form (split, sweep, recombine)."""
-    import os
-    torch = _torch()
-    if dtype not in (torch.float64, torch.float32) or nens > 103 or os.environ.get('EXB_FUSED', '1') == '0':
-        return False
-    return os.environ.get('EXB_SU_IMPL', 'pipe') == 'pipe'
+# Largest ensemble of the fused sweep: 13 tiles of 8 columns, the last of which also carries the ensemble mean as a
+# pseudo-member (state_sweep_2p.cu), so 8 * 13 - 1 members.
+FUSED_MAX_NENS = 103
+
+
+def fused_sweep_available(nens):
+    """The fused sweep (exb_state_sweep_*) serves float64 and float32 (storage) ensembles of up to FUSED_MAX_NENS
+    members; larger ones take the three-call form (split, exb_state_update_*, recombine)."""
+    return nens <= FUSED_MAX_NENS
 
 
 RELAX_KINDS = ('rtps', 'rtpp')
@@ -764,7 +760,7 @@ def analysis_device(X, nlev, grid: GridTables, obs: ObsArrays, loc_mode, inflati
                                obs_dist_block())
             elif obs_plan_wanted(loc_mode):
                 plan = ObsPlan(obs_dev, geo, obs.nobs, loc_mode)
-            fused = fused_sweep_available(X.dtype, nens)
+            fused = fused_sweep_available(nens)
             grid_u = grid.u if band is None else grid.u[:, y0 * nx:y1 * nx].contiguous()
             if Y is None:
                 Yp, nex = ob_priors(X, grid, obs, sfx, nlev=nlev, band=band, group=group, obs_dev=obs_dev,
@@ -779,7 +775,7 @@ def analysis_device(X, nlev, grid: GridTables, obs: ObsArrays, loc_mode, inflati
             if plan is not None:
                 # the solve is next on the critical path: its lists are filled before the sweep's plan is started
                 plan.finish()
-            if fused and sweep_plan_wanted():
+            if fused:
                 # candidate lists of the sweep: geometry only as well, built on another side stream.  Creating the plan
                 # blocks its caller until the counting pass is done, so it comes after the ob priors have been enqueued
                 # (the device computes them meanwhile)
@@ -868,8 +864,8 @@ def analysis_host(X_host, nlev, lat2d, lon2d, obs: ObsArrays, loc_mode, inflatio
                   forward_operator='reference'):
     """Host-buffer entry: X_host is a numpy array or CPU torch tensor [nlev*ny*nx, nens]; it is uploaded,
     analysed on `device`, and the analysis is written to `out` (default: back into X_host).  Pinned host
-    memory makes the copies asynchronous.  With the fused float64 sweep (and pipeline=True) the state is swept
-    in latitude bands and each finished band is downloaded on a second stream while the next one is swept, so
+    memory makes the copies asynchronous.  With the fused sweep (up to FUSED_MAX_NENS members, pipeline=True and
+    localisation) the state is swept in latitude bands and each finished band is downloaded on a second stream while the next one is swept, so
     only the last band's download is exposed; the upload is overlapped with the obs-space solve when X_host is
     pinned (see ob_priors).  res.ms gains 'upload' (duration of the host-to-device copies) and 'download' (what is
     left of the device-to-host copies after the last sweep).
@@ -895,7 +891,7 @@ def analysis_host(X_host, nlev, lat2d, lon2d, obs: ObsArrays, loc_mode, inflatio
         xdtype = Xh.dtype if dtype is None else dtype
         y0, y1 = band if band is not None else (0, grid.ny)
         ny_loc = y1 - y0
-        banded = (pipeline and fused_sweep_available(xdtype, nens) and Oh.dtype == xdtype and Xh.dtype == xdtype
+        banded = (pipeline and fused_sweep_available(nens) and Oh.dtype == xdtype and Xh.dtype == xdtype
                   and loc_mode == LOC_GC and obs.nobs > 0)
         if banded:
             # Three streams: uploads (band by band, in sweep order), compute, downloads.  With a pinned source and

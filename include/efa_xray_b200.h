@@ -301,8 +301,9 @@ int exb_obs_solve_async_status(void);
  * counters (device uint64[2], may be NULL): [1] += number of (ob, grid point) pairs with non-zero
  * weight = sum_k |F_s(k)| / nlev of SURVEY.md section 8d.
  * Up to 103 members both types run on the two-phase FP64 tensor-core kernel (float32: float32 storage,
- * float64 arithmetic), which synchronises the stream once to size its candidate lists; EXB_SU_IMPL = pipe | mma |
- * vector selects the kernel (DESIGN.md section 4.3). */
+ * float64 arithmetic), which synchronises the stream once to size its candidate lists.  Float64 ensembles of 104 to
+ * 255 members run on the blocked FP64 tensor-core kernel; float32 ensembles of 104 to 256 members and float64
+ * ensembles of 256 run on the vector kernel, whose arithmetic is in the storage type (DESIGN.md section 4.3). */
 int exb_state_update_f64(double *xm, double *Xp, int64_t nlev, int64_t ny, int64_t nx, int nens,
                          const double *grid_u, const double *Yp, const double *rec, const double *obgeo,
                          int64_t nobs, int64_t ob_begin, int64_t ob_end, int loc_mode,

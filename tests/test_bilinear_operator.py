@@ -3,7 +3,6 @@ weights, the numpy reference's known answers and the argument checks of the API 
 needed); on the GPU both stencil kernels against the reference (tests/bilinear_reference.py), and every analysis path
 against the reference analysis built on the unchanged CPU oracle."""
 import dataclasses
-import os
 
 import numpy as np
 import pytest
@@ -374,19 +373,6 @@ def _check_diag(obs, ref_obs):
     assert [o.assimilated for o in obs] == [o.assimilated for o in ref_obs]
 
 
-def _with_env(env, fn):
-    old = {k: os.environ.get(k) for k in env}
-    os.environ.update(env)
-    try:
-        return fn()
-    finally:
-        for k, v in old.items():
-            if v is None:
-                os.environ.pop(k, None)
-            else:
-                os.environ[k] = v
-
-
 def _regrid(case, lat2d, lon2d, seed):
     """The case on another grid of the same shape, with its obs moved into random cells of that grid."""
     ob_lat, ob_lon = _obs_in_cells(lat2d, lon2d, case.nobs, seed)
@@ -406,11 +392,12 @@ _C50 = dict(ny=25, nx=48, nmem=50, nvars=2, ntimes=2, nobs=70, cutoff_km=2500.0,
             frac_skip=0.05)
 
 
+# env: attributes of engine patched for the case; FUSED_MAX_NENS = 0 takes the three-call form
 @pytest.mark.gpu
 @pytest.mark.parametrize('kw,loc,inflation,env', [
     (_MULTI, 'GC', None, {}),
     (_C50, 'GC', None, {}),
-    (_C50, 'GC', None, {'EXB_FUSED': '0'}),
+    (_C50, 'GC', None, {'FUSED_MAX_NENS': 0}),
     (_C50, False, None, {}),
     (_C50, 'GC', 1.15, {}),
     (dict(ny=25, nx=48, nmem=7, nvars=1, ntimes=2, nobs=60, cutoff_km=1500.0, seed=307, offtime=True), 'GC', None, {}),
@@ -419,13 +406,14 @@ _C50 = dict(ny=25, nx=48, nmem=50, nvars=2, ntimes=2, nobs=70, cutoff_km=2500.0,
      {}),
     ('curv', 'GC', None, {}),
 ])
-def test_update_bilinear_matches_reference(kw, loc, inflation, env):
+def test_update_bilinear_matches_reference(kw, loc, inflation, env, monkeypatch):
     EnsembleState, Observation, EnSRF = _api()
     case = _curv_case() if kw == 'curv' else make_case(**kw)
     ref_post, ref_obs, prior = B.ensrf_update(case, loc=loc, inflation=inflation)
     state, obs = build_objects(case, EnsembleState, Observation)
-    post, _ = _with_env(env, lambda: EnSRF(state, obs, verbose=False, loc=loc, inflation=inflation,
-                                           forward_operator='bilinear').update())
+    for name, value in env.items():
+        monkeypatch.setattr(engine, name, value)
+    post, _ = EnSRF(state, obs, verbose=False, loc=loc, inflation=inflation, forward_operator='bilinear').update()
     _check_post(post.to_vect(), ref_post, prior)
     _check_diag(obs, ref_obs)
     assert sum(o.assimilated for o in obs) > 0.8 * len(obs)

@@ -135,6 +135,11 @@ def _oracle_run(case, loc, inflation=None):
     (dict(ny=19, nx=36, nmem=16, nvars=11, ntimes=1, nobs=40, cutoff_km=4000.0, seed=17), 'GC'),
     (dict(ny=25, nx=48, nmem=20, nvars=2, ntimes=1, nobs=80, seed=18), False),
     (dict(ny=46, nx=90, nmem=50, nvars=1, ntimes=1, nobs=200, cutoff_km=1000.0, seed=19), 'GC'),
+    # the largest ensembles of the blocked tensor-core kernel (32 tiles) and of the vector kernel
+    (dict(ny=19, nx=36, nmem=255, nvars=1, ntimes=1, nobs=40, cutoff_km=4000.0, seed=20,
+         avoid_mirror_ties=True), 'GC'),
+    (dict(ny=19, nx=36, nmem=256, nvars=1, ntimes=1, nobs=40, cutoff_km=4000.0, seed=22,
+         avoid_mirror_ties=True), 'GC'),
 ])
 def test_update_matches_oracle(kw, loc):
     """Seeded cases against the oracle: ensemble sizes that exercise every kernel variant, many levels,
@@ -183,17 +188,19 @@ def test_config1_full_size_against_oracle():
 
 def test_fp32_tolerance():
     """fp32 device arithmetic (scalars stay fp64): mean within 1e-5 of the field magnitude, perturbations
-    within 1e-3 of the ensemble spread."""
+    within 1e-3 of the ensemble spread.  At 50 members the state update is the two-phase sweep (float64 arithmetic
+    in registers); at 130 it is the vector kernel, whose row arithmetic is float32 as well."""
     EnsembleState, Observation, EnSRF = _api()
-    case = make_case(ny=46, nx=90, nmem=50, nvars=2, ntimes=1, nobs=300, cutoff_km=2500.0, seed=23)
-    state, obs = build_objects(case, EnsembleState, Observation)
-    post32, _ = EnSRF(state, obs, verbose=False, loc='GC', dtype='f32').update()
-    ref_post, _ = _oracle_run(case, 'GC')
-    p32 = post32.to_vect()
-    m32, mref = p32.mean(axis=1), ref_post.mean(axis=1)
-    assert np.abs(m32 - mref).max() <= 1e-5 * np.abs(mref).max()
-    spread = (ref_post - mref[:, None]).std()
-    assert np.abs((p32 - m32[:, None]) - (ref_post - mref[:, None])).max() <= 1e-3 * spread
+    for nmem in (50, 130):
+        case = make_case(ny=46, nx=90, nmem=nmem, nvars=2, ntimes=1, nobs=300, cutoff_km=2500.0, seed=23)
+        state, obs = build_objects(case, EnsembleState, Observation)
+        post32, _ = EnSRF(state, obs, verbose=False, loc='GC', dtype='f32').update()
+        ref_post, _ = _oracle_run(case, 'GC')
+        p32 = post32.to_vect()
+        m32, mref = p32.mean(axis=1), ref_post.mean(axis=1)
+        assert np.abs(m32 - mref).max() <= 1e-5 * np.abs(mref).max(), nmem
+        spread = (ref_post - mref[:, None]).std()
+        assert np.abs((p32 - m32[:, None]) - (ref_post - mref[:, None])).max() <= 1e-3 * spread, nmem
 
 
 @pytest.mark.parametrize('pinned', [False, True])
@@ -410,36 +417,16 @@ def test_obs_solve_dag_fp32():
     np.testing.assert_allclose(rec[:4], ref[2][:4], rtol=2e-3, equal_nan=True)
 
 
-def _analysis_with_env(case, env, bands=None):
-    """engine.analysis_device on a fresh device copy of the case's state under the given environment; with
-    `bands` the fused sweep is issued band by band (row ranges of the same shard)."""
-    import os
+def _analysis(case, bands=None):
+    """engine.analysis_device on a fresh device copy of the case's state; with `bands` the fused sweep is issued band
+    by band (row ranges of the same shard)."""
     import torch
-    from efa_xray_b200 import engine, _lib
+    from efa_xray_b200 import engine
     dev = torch.device('cuda', 0)
     X = torch.as_tensor(case.to_vect()).to(dev).contiguous()
-    ny, nx = case.lat2d.shape
-    nt = len(case.times)
-    nlev = nt * len(case.varnames)
-    tlo, thi, wlo, whi, _ = engine.time_weights(case.times, case.ob_time)
-    obs = engine.ObsArrays(value=case.ob_value, error=case.ob_error, lat=case.ob_lat, lon=case.ob_lon,
-                           halfwidth=case.ob_halfwidth, assimilate=case.ob_assimilate.astype(np.uint8),
-                           row0=(case.ob_var * nt + tlo) * (ny * nx), row1=(case.ob_var * nt + thi) * (ny * nx),
-                           tw0=wlo, tw1=whi)
+    nlev = len(case.times) * len(case.varnames)
     grid = engine.GridTables(case.lat2d, case.lon2d, dev)
-    old = {k: os.environ.get(k) for k in env}
-    os.environ.update(env)
-    try:
-        if bands is None:
-            res = engine.analysis_device(X, nlev, grid, obs, engine.LOC_GC)
-        else:
-            res = engine.analysis_device(X, nlev, grid, obs, engine.LOC_GC, sweep_bands=bands)
-    finally:
-        for k, v in old.items():
-            if v is None:
-                os.environ.pop(k, None)
-            else:
-                os.environ[k] = v
+    res = engine.analysis_device(X, nlev, grid, _engine_obs(case), engine.LOC_GC, sweep_bands=bands)
     return X.cpu().numpy(), res
 
 
@@ -452,29 +439,42 @@ def _analysis_with_env(case, env, bands=None):
     # beyond the range of the branch-free weight function
     dict(ny=31, nx=60, nmem=16, nvars=2, ntimes=1, nobs=7000, cutoff_km=9000.0, seed=45, frac_skip=0.02),
 ])
-def test_sweep_variants_agree(kw):
-    """The two-phase fused sweep (default), the same kernel without a sweep plan or without candidate lists,
-    band-by-band calls, and the three-call forms (split / sweep / recombine) on the same kernel, on the earlier
-    tensor-core kernel and on the vector kernel all apply the same obs in the same order to every state row."""
+def test_sweep_variants_agree(kw, monkeypatch):
+    """The two-phase sweep, fused with and without a sweep plan, in band-by-band calls and in the three-call form
+    (split / exb_state_update / recombine, the same kernel in split mode), applies the same obs in the same order to
+    every state row as the fused sweep after the persistent obs-space solve.  A numpy replay of sampled rows from the
+    obs-space records checks the default run independently of the sweep kernel."""
+    import torch
+    from efa_xray_b200 import engine
     case = make_case(**kw)
     prior = case.to_vect()
-    ref, res0 = _analysis_with_env(case, {'EXB_SU_IMPL': 'mma', 'EXB_OBS_IMPL': 'persistent'})
+    with monkeypatch.context() as m:
+        m.setenv('EXB_OBS_IMPL', 'persistent')
+        ref, res0 = _analysis(case)
     inc = np.abs(ref - prior).max()
-    ny = case.lat2d.shape[0]
-    runs = {
-        'pipe_fused': _analysis_with_env(case, {}),
-        'pipe_noplan': _analysis_with_env(case, {'EXB_SWEEP_PLAN': '0'}),
-        'pipe_nolist': _analysis_with_env(case, {'EXB_SWEEP_NOLIST': '1'}),
-        'pipe_split': _analysis_with_env(case, {'EXB_FUSED': '0'}),
-        'vector': _analysis_with_env(case, {'EXB_SU_IMPL': 'vector'}),
-        'pipe_bands': _analysis_with_env(case, {}, bands=[(0, 7), (7, 30), (30, ny - 1), (ny - 1, ny)]),
-    }
+    ny, nx = case.lat2d.shape
+    runs = {'fused': _analysis(case)}
+    with monkeypatch.context() as m:
+        m.setattr(engine, 'SweepPlan', lambda *args, **kwargs: None)
+        runs['fused_noplan'] = _analysis(case)
+    with monkeypatch.context() as m:
+        m.setattr(engine, 'FUSED_MAX_NENS', 0)
+        runs['split'] = _analysis(case)
+    runs['bands'] = _analysis(case, bands=[(0, 7), (7, 30), (30, ny - 1), (ny - 1, ny)])
     for name, (X, res) in runs.items():
         # pairs with a non-zero weight: identical up to the handful of pairs within rounding of the edge of a
         # support (the branch-free weight function and the libm one may round a 1e-16 weight to 0 differently)
         assert abs(res.state_pairs - res0.state_pairs) <= 1e-4 * res0.state_pairs, name
         np.testing.assert_allclose(X, ref, rtol=1e-11, err_msg=name)
         assert np.abs(X - ref).max() <= 1e-9 * inc, name
+    obs, Ym, Yp = _obs_block(case)
+    _, ye, rec, _ = _run_obs_solve(obs, Ym, Yp, 1, 'dag')
+    dev = torch.device('cuda', 0)
+    _, geo = engine.upload_obs(obs, dev, 1)
+    grid_u = engine.GridTables(case.lat2d, case.lon2d, dev).u.cpu().numpy()
+    pts, rows = _sample_rows(np.random.default_rng(4), ny, nx, len(case.times) * len(case.varnames))
+    want = _replay_rows(prior[rows], pts, grid_u, ye, rec, geo.cpu().numpy(), 1)
+    assert np.abs(runs['fused'][0][rows] - want).max() <= 1e-9 * inc
 
 
 def test_postprocess_statistics_match_oracle():

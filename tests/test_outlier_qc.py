@@ -202,17 +202,15 @@ def test_engine_rejects_thresholds_of_the_wrong_length(threshold):
 # ---------------------------------------------------------------------------------------------------------------
 # GPU: the public API against the reference
 # ---------------------------------------------------------------------------------------------------------------
-def _with_env(env, fn):
-    old = {k: os.environ.get(k) for k in env}
-    os.environ.update(env)
-    try:
-        return fn()
-    finally:
-        for k, v in old.items():
-            if v is None:
-                os.environ.pop(k, None)
-            else:
-                os.environ[k] = v
+def _patch(monkeypatch, env):
+    """The settings a case runs under: EXB_* environment variables, and attributes of engine (FUSED_MAX_NENS = 0 takes
+    the three-call form: split, exb_state_update, recombine)."""
+    from efa_xray_b200 import engine
+    for name, value in env.items():
+        if name.startswith('EXB_'):
+            monkeypatch.setenv(name, value)
+        else:
+            monkeypatch.setattr(engine, name, value)
 
 
 def _diag(obs, attr):
@@ -238,12 +236,12 @@ _C = dict(ny=25, nx=48, nvars=2, ntimes=1, nobs=120, frac_skip=0.05)
     (dict(_C, nmem=32, cutoff_km=3000.0, seed=304), 'GC', 3.0, {}),
     (dict(_C, nmem=100, cutoff_km=3000.0, seed=305), 'GC', 3.0, {}),
     (dict(ny=19, nx=36, nvars=1, ntimes=1, nobs=80, nmem=130, cutoff_km=4000.0, seed=306), 'GC', 3.0, {}),
-    (dict(_C, nmem=50, cutoff_km=2500.0, seed=307), 'GC', 3.0, {'EXB_SU_IMPL': 'vector'}),
+    (dict(_C, nmem=50, cutoff_km=2500.0, seed=307), 'GC', 3.0, {'FUSED_MAX_NENS': 0}),
     (dict(_C, nmem=50, cutoff_km=2500.0, seed=308, frac_skip=0.2), 'GC', {'var1': 2.5}, {}),
     (dict(_C, nmem=50, cutoff_km=2500.0, seed=308, frac_skip=0.2), 'GC', {'var0': 3.0, 'var1': 2.0},
      {'EXB_OBS_IMPL': 'persistent'}),
 ])
-def test_update_with_qc_matches_reference(kw, loc, threshold, env):
+def test_update_with_qc_matches_reference(kw, loc, threshold, env, monkeypatch):
     """EnSRF(..., outlier_threshold=...) against the reference: the rejected set exactly, the state at
     test_gpu_parity's tolerances, the per-ob diagnostics, and the caller's assimilate_this left alone."""
     EnsembleState, Observation, EnSRF = _api()
@@ -251,7 +249,8 @@ def test_update_with_qc_matches_reference(kw, loc, threshold, env):
     rej, _, ref_post, ref_obs = reference_analysis(case, threshold, loc=loc)
     assert rej.sum() >= 3
     state, obs = build_objects(case, EnsembleState, Observation)
-    post, _ = _with_env(env, lambda: EnSRF(state, obs, verbose=False, loc=loc, outlier_threshold=threshold).update())
+    _patch(monkeypatch, env)
+    post, _ = EnSRF(state, obs, verbose=False, loc=loc, outlier_threshold=threshold).update()
     flags = np.array([o.assimilate_this for o in obs])
     np.testing.assert_array_equal(flags, case.ob_assimilate)
     got_rej = flags & ~np.array([o.assimilated for o in obs])
@@ -264,24 +263,26 @@ def test_update_with_qc_matches_reference(kw, loc, threshold, env):
 
 @pytest.mark.gpu
 def test_fp32_with_qc():
-    """float32 storage: the rejected set exactly, the state at test_fp32_tolerance's tolerance."""
+    """float32 storage: the rejected set exactly, the state at test_fp32_tolerance's tolerance.  At 130 members the
+    state update is the vector kernel, with float32 arithmetic."""
     EnsembleState, Observation, EnSRF = _api()
-    case = _with_gross_errors(make_case(ny=46, nx=90, nmem=50, nvars=2, ntimes=1, nobs=300, cutoff_km=2500.0, seed=23),
-                              seed=23)
-    rej, _, ref_post, _ = reference_analysis(case, 3.0, margin=1e-3)
-    assert rej.sum() >= 5
-    state, obs = build_objects(case, EnsembleState, Observation)
-    post32, _ = EnSRF(state, obs, verbose=False, loc='GC', dtype='f32', outlier_threshold=3.0).update()
-    np.testing.assert_array_equal(~np.array([o.assimilated for o in obs]) & case.ob_assimilate, rej)
-    p32 = post32.to_vect()
-    m32, mref = p32.mean(axis=1), ref_post.mean(axis=1)
-    assert np.abs(m32 - mref).max() <= 1e-5 * np.abs(mref).max()
-    spread = (ref_post - mref[:, None]).std()
-    assert np.abs((p32 - m32[:, None]) - (ref_post - mref[:, None])).max() <= 1e-3 * spread
+    for nmem in (50, 130):
+        case = _with_gross_errors(make_case(ny=46, nx=90, nmem=nmem, nvars=2, ntimes=1, nobs=300, cutoff_km=2500.0,
+                                            seed=23), seed=23)
+        rej, _, ref_post, _ = reference_analysis(case, 3.0, margin=1e-3)
+        assert rej.sum() >= 5
+        state, obs = build_objects(case, EnsembleState, Observation)
+        post32, _ = EnSRF(state, obs, verbose=False, loc='GC', dtype='f32', outlier_threshold=3.0).update()
+        np.testing.assert_array_equal(~np.array([o.assimilated for o in obs]) & case.ob_assimilate, rej)
+        p32 = post32.to_vect()
+        m32, mref = p32.mean(axis=1), ref_post.mean(axis=1)
+        assert np.abs(m32 - mref).max() <= 1e-5 * np.abs(mref).max(), nmem
+        spread = (ref_post - mref[:, None]).std()
+        assert np.abs((p32 - m32[:, None]) - (ref_post - mref[:, None])).max() <= 1e-3 * spread, nmem
 
 
 @pytest.mark.gpu
-def test_unreachable_threshold_is_bit_identical():
+def test_unreachable_threshold_is_bit_identical(monkeypatch):
     """A threshold no ob reaches gives, bit for bit, the analysis and diagnostics of outlier_threshold=None."""
     EnsembleState, Observation, EnSRF = _api()
     case = _with_gross_errors(make_case(ny=46, nx=90, nmem=50, nvars=2, ntimes=1, nobs=300, cutoff_km=2500.0, seed=311,
@@ -290,7 +291,9 @@ def test_unreachable_threshold_is_bit_identical():
     for env in ({}, {'EXB_OBS_IMPL': 'persistent'}):
         for t in (None, 1e6, {'var0': 1e6, 'var1': 1e6}):
             state, obs = build_objects(case, EnsembleState, Observation)
-            post, _ = _with_env(env, lambda: EnSRF(state, obs, verbose=False, loc='GC', outlier_threshold=t).update())
+            with monkeypatch.context() as m:
+                _patch(m, env)
+                post, _ = EnSRF(state, obs, verbose=False, loc='GC', outlier_threshold=t).update()
             outs[(str(env), str(t))] = (post.to_vect(), {a: _diag(obs, a) for a in ('prior_mean', 'prior_var', 'post_mean',
                                                                                       'post_var', 'assimilated')})
     for env in ({}, {'EXB_OBS_IMPL': 'persistent'}):
@@ -320,12 +323,12 @@ def _engine_inputs(case, threshold=np.zeros(0)):
     return dev, nt * len(case.varnames), engine.GridTables(case.lat2d, case.lon2d, dev), obs
 
 
-def _device_analysis(case, obs, env=None, **kw):
+def _device_analysis(case, obs, **kw):
     import torch
     from efa_xray_b200 import engine
     dev, nlev, grid, _ = _engine_inputs(case)
     X = torch.as_tensor(case.to_vect()).to(dev)
-    res = _with_env(env or {}, lambda: engine.analysis_device(X, nlev, grid, obs, engine.LOC_GC, **kw))
+    res = engine.analysis_device(X, nlev, grid, obs, engine.LOC_GC, **kw)
     return X.cpu().numpy(), res
 
 
@@ -334,18 +337,19 @@ def _rejected(obs, res):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize('env', [{}, {'EXB_OBS_IMPL': 'persistent'}, {'EXB_FUSED': '0'}])
-def test_qc_equals_run_with_rejected_obs_flagged_off(env):
+@pytest.mark.parametrize('env', [{}, {'EXB_OBS_IMPL': 'persistent'}, {'FUSED_MAX_NENS': 0}])
+def test_qc_equals_run_with_rejected_obs_flagged_off(env, monkeypatch):
     """The QC analysis against the analysis without QC and with exactly its rejected obs flagged off: obs-space
     diagnostics bit for bit, the state within the parity tolerance (the sweep batches its obs differently)."""
     case = _with_gross_errors(make_case(ny=46, nx=90, nmem=50, nvars=2, ntimes=1, nobs=600, cutoff_km=2500.0, seed=321,
                                         frac_skip=0.05), seed=321)
     _, _, _, obs = _engine_inputs(case, threshold=np.full(case.nobs, 3.0))
-    X, res = _device_analysis(case, obs, env)
+    _patch(monkeypatch, env)
+    X, res = _device_analysis(case, obs)
     rej = _rejected(obs, res)
     assert rej.sum() >= 20
     off = dataclasses.replace(obs, assimilate=(obs.assimilate.astype(bool) & ~rej).astype(np.uint8), threshold=np.zeros(0))
-    X0, res0 = _device_analysis(case, off, env)
+    X0, res0 = _device_analysis(case, off)
     for a in ('prior_mean', 'prior_var', 'post_mean', 'post_var', 'assimilated'):
         np.testing.assert_array_equal(getattr(res, a), getattr(res0, a), err_msg=a)
     _check_post(X, X0, case.to_vect())

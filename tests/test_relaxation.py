@@ -2,7 +2,6 @@
 the Python API and of the C entry points (no device needed), and on the GPU the kernels, every analysis path
 (fused sweep, three-call path, host-buffer band pipeline, latitude-band shards) and BASELINE config 3 against the
 reference (tests/relax_reference.py, built on the CPU oracle)."""
-import os
 
 import numpy as np
 import pytest
@@ -199,23 +198,11 @@ def _check_post(post, ref_post, prior, tol_scale=1.0):
     assert np.abs((post - prior) - inc_ref).max() <= F64_INC_TOL * tol_scale * scale
 
 
-def _with_env(env, fn):
-    old = {k: os.environ.get(k) for k in env}
-    os.environ.update(env)
-    try:
-        return fn()
-    finally:
-        for k, v in old.items():
-            if v is None:
-                os.environ.pop(k, None)
-            else:
-                os.environ[k] = v
-
-
 _C50 = dict(ny=25, nx=48, nmem=50, nvars=2, ntimes=1, nobs=70, cutoff_km=2500.0, seed=201, frac_skip=0.05)
 _INFL_X = ('linspace', 1.0, 1.3, 48)
 
 
+# env: attributes of engine patched for the case; FUSED_MAX_NENS = 0 takes the three-call form
 @pytest.mark.gpu
 @pytest.mark.parametrize('kw,loc,relaxation,inflation,env', [
     (_C50, 'GC', ('rtps', 0.6), None, {}),
@@ -229,8 +216,8 @@ _INFL_X = ('linspace', 1.0, 1.3, 48)
     (dict(ny=25, nx=48, nmem=100, nvars=2, ntimes=1, nobs=60, cutoff_km=3000.0, seed=203), 'GC', ('rtpp', 0.8), None, {}),
     (dict(ny=19, nx=36, nmem=130, nvars=1, ntimes=1, nobs=40, cutoff_km=4000.0, seed=204), 'GC', ('rtps', 0.7), None, {}),
     (dict(ny=19, nx=36, nmem=130, nvars=1, ntimes=1, nobs=40, cutoff_km=4000.0, seed=204), 'GC', ('rtpp', 0.7), None, {}),
-    (_C50, 'GC', ('rtps', 0.6), None, {'EXB_FUSED': '0'}),
-    (_C50, 'GC', ('rtpp', 0.4), 1.1, {'EXB_FUSED': '0'}),
+    (_C50, 'GC', ('rtps', 0.6), None, {'FUSED_MAX_NENS': 0}),
+    (_C50, 'GC', ('rtpp', 0.4), 1.1, {'FUSED_MAX_NENS': 0}),
     (dict(ny=31, nx=60, nmem=24, nvars=2, ntimes=3, nobs=80, cutoff_km=2000.0, seed=205, offtime=True, frac_skip=0.05),
      'GC', ('rtps', {'var1': 0.5}), None, {}),
     (dict(ny=25, nx=48, nmem=20, nvars=2, ntimes=1, nobs=60, seed=206), False, ('rtps', 0.75), None, {}),
@@ -240,9 +227,10 @@ _INFL_X = ('linspace', 1.0, 1.3, 48)
     (dict(one_d=True, npts=24, nmem=8, nvars=2, ntimes=1, nobs=30, cutoff_km=4000.0, seed=207), 'GC', ('rtpp', 0.8),
      None, {}),
 ])
-def test_update_with_relaxation_matches_reference(kw, loc, relaxation, inflation, env):
+def test_update_with_relaxation_matches_reference(kw, loc, relaxation, inflation, env, monkeypatch):
     from conftest import decode_inflation
     from oracle import ensrf_oracle as O
+    from efa_xray_b200 import engine
     EnsembleState, Observation, EnSRF = _api()
     kw = dict(kw)
     case = make_case_1d(**{k: v for k, v in kw.items() if k != 'one_d'}) if kw.pop('one_d', False) else make_case(**kw)
@@ -254,8 +242,9 @@ def test_update_with_relaxation_matches_reference(kw, loc, relaxation, inflation
     unrelaxed, _ = O.ensrf_update(O.State.from_case(case), O.obs_from_case(case), loc=loc, inflation=inflation)
     assert np.abs(ref_post.to_vect() - unrelaxed.to_vect()).max() > 1e-6       # the relaxation does something
     state, obs = build_objects(case, EnsembleState, Observation)
-    post_state, _ = _with_env(env, lambda: EnSRF(state, obs, verbose=False, loc=loc, inflation=inflation,
-                                                  relaxation=relaxation).update())
+    for name, value in env.items():
+        monkeypatch.setattr(engine, name, value)
+    post_state, _ = EnSRF(state, obs, verbose=False, loc=loc, inflation=inflation, relaxation=relaxation).update()
     _check_post(post_state.to_vect(), ref_post.to_vect(), prior)
     # the per-ob diagnostics are those of the serial loop
     for attr in ('prior_mean', 'prior_var', 'post_mean', 'post_var'):

@@ -6,8 +6,6 @@ skips its odd k-step) or 5..7 (member order, mean masked).  Each case below is r
 instantiation of the kernel (16, 40, 64 and 104 columns), and rows no ob can reach are checked to come back
 bit-identical to the prior.
 """
-import os
-
 import numpy as np
 import pytest
 
@@ -20,22 +18,13 @@ F64_INC_TOL = 1e-9        # on the analysis increment, relative to the largest i
 R_EARTH_KM = 6371.0
 
 
-def _run(case, env):
+def _run(case):
     from efa_xray_b200.state.ensemble import EnsembleState
     from efa_xray_b200.observation.observation import Observation
     from efa_xray_b200.assimilation.ensrf import EnSRF
-    old = {k: os.environ.get(k) for k in env}
-    os.environ.update(env)
-    try:
-        state, obs = build_objects(case, EnsembleState, Observation)
-        post, _ = EnSRF(state, obs, verbose=False, loc='GC').update()
-        return post.to_vect()
-    finally:
-        for k, v in old.items():
-            if v is None:
-                os.environ.pop(k, None)
-            else:
-                os.environ[k] = v
+    state, obs = build_objects(case, EnsembleState, Observation)
+    post, _ = EnSRF(state, obs, verbose=False, loc='GC').update()
+    return post.to_vect()
 
 
 def _far_rows(case, margin_km):
@@ -56,17 +45,22 @@ def _far_rows(case, margin_km):
 #   96 (104, 0)  99 (104, 3)  101 (104, 5)  103 (104, 7: the largest fused size)
 # (13 members use seed 415 rather than 313: that case has an ob at 172.76 E whose prior from the forward operator
 # differs from the oracle's, which is not what this test is about)
+# env: attributes of engine patched for the case; FUSED_MAX_NENS = 0 takes the three-call form (split,
+# exb_state_update, recombine), which runs the same kernel in split mode
 @pytest.mark.parametrize('nmem,seed,env', [
     (11, 311, {}), (13, 415, {}), (27, 327, {}), (30, 330, {}), (53, 353, {}), (74, 374, {}), (79, 379, {}),
     (96, 396, {}), (99, 399, {}), (101, 401, {}), (103, 403, {}),
-    (99, 399, {'EXB_FUSED': '0'}), (101, 401, {'EXB_FUSED': '0'}),
+    (99, 399, {'FUSED_MAX_NENS': 0}), (101, 401, {'FUSED_MAX_NENS': 0}),
 ])
-def test_last_tile_layouts_match_oracle(nmem, seed, env):
+def test_last_tile_layouts_match_oracle(nmem, seed, env, monkeypatch):
     from oracle import ensrf_oracle as O
+    from efa_xray_b200 import engine
+    for name, value in env.items():
+        monkeypatch.setattr(engine, name, value)
     # few obs with a short support over a 7.5 degree grid: many rows are out of reach of every ob
     case = make_case(ny=25, nx=48, nmem=nmem, nvars=2, ntimes=1, nobs=16, cutoff_km=1500.0, seed=seed, frac_skip=0.05)
     prior = case.to_vect()
-    post = _run(case, env)
+    post = _run(case)
     ref, _ = O.ensrf_update(O.State.from_case(case), O.obs_from_case(case), loc='GC')
     ref = ref.to_vect()
     np.testing.assert_allclose(post, ref, rtol=F64_RTOL)
